@@ -9,8 +9,13 @@ Workloads (BASELINE.json configs):
           1/2/4/8-GPU sweep is quoted on; B per GPU fixed => weak scaling)
     uci   13-50-1 relu, N=10000, M=5, 4096 chains (configs[1])
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload wide|uci|...] [--batch B]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload wide|uci|...] [--batch B] [--dump-outputs DIR]
   python bench.py --impl reference ...      # the CPU restatement of the reference's path
+
+--dump-outputs DIR writes what the last timed step computed, as the caller receives it, to DIR/<name>.npy: lp (samples,)
+float64 for the density workloads, z_trace (M, chains, steps) float32 and lp_trace (chains, steps) float64 for the MH / MALA
+workloads (every rank's chains when N > 1).  The inputs are seeded, so two builds run with the same arguments can be
+compared output for output.
 
 Synthetic inputs come from workloads.py (NumPy); oracle/ is touched only as the checker after the timed region and by the
 CPU-baseline / --impl reference legs.
@@ -371,6 +376,32 @@ def multi_ctx_section(ssi, torch, prob, world, B, sigma_m, zs, steps):
         eng.close()
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def mh_traces(z_flat, lp_flat, world, chains, steps, M):
+    """Flat device traces gathered rank after rank (each rank's block an (M, chains, steps) / (chains, steps) column-major
+    buffer) in the shapes mh_run returns, over all world * chains chains: z (M, world*chains, steps), lp (world*chains, steps)."""
+    z = z_flat.reshape(world, steps, chains, M).transpose(3, 0, 2, 1).reshape(M, world * chains, steps)
+    lp = lp_flat.reshape(world, steps, chains).transpose(0, 2, 1).reshape(world * chains, steps)
+    return z, lp
+
+
+def dump_outputs(out_dir, arrays: dict):
+    """Write every {name: (array, sample axis)} as out_dir/<name>.npy.  Above DUMP_LIMIT bytes in all, every array keeps the
+    same fixed sample of its samples / chains (sorted ids drawn with default_rng(0)), so two dumps still compare entry for entry."""
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    total = sum(a.nbytes for a, _ in arrays.values())
+    a0, ax0 = next(iter(arrays.values()))
+    n = a0.shape[ax0]
+    keep = None
+    if total > DUMP_LIMIT:
+        keep = np.sort(np.random.default_rng(0).choice(n, max(1, n * DUMP_LIMIT // total), replace=False))
+    for name, (a, axis) in arrays.items():
+        np.save(out_dir / f"{name}.npy", a if keep is None else np.take(a, keep, axis=axis))
+
+
 _REAL_STDOUT = None
 
 
@@ -403,7 +434,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the streams / mh_c5 / multi_device_ctx sections")
     ap.add_argument("--opt", action="append", default=[], help="library A/B switch, key=value (ssi_set_option); repeatable")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy (at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.batch <= 0:
         args.batch = int(os.environ.get("SSI_BENCH_BATCH", WORKLOADS[args.workload][1]))
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
@@ -540,6 +574,13 @@ def main():
     with ClockSampler(local_rank) as clk:
         ms_dev = timed(lambda: step_device(record=True), args.steps)
     eng.sync()
+    if args.dump_outputs and rank == 0:
+        if mh:
+            z, lp = d_tr_all if world > 1 else (d_z_tr, d_lp_tr)
+            z, lp = mh_traces(z.cpu().numpy(), lp.cpu().numpy(), world, B, MH_STEPS, prob.M)
+            dump_outputs(args.dump_outputs, {"z_trace": (z, 1), "lp_trace": (lp, 0)})
+        else:
+            dump_outputs(args.dump_outputs, {"lp": ((d_lp_all if world > 1 else d_lp).cpu().numpy(), 0)})
     st = eng.stats()
     dom_ms, dom_n = st.dominant_ms, st.dominant_launches
     eng.set_option("time_dominant", 0)
