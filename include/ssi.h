@@ -121,12 +121,12 @@ int  ssi_sync(ssi_ctx* ctx);
  * path: 1 = FP16 planes with power-of-two scales, the default; 0 = BF16x3), "mala_rule" (0 = the documented Metropolis-adjusted
  * Langevin ratio, the default; 1 = both proposal densities evaluated with the negated gradient, see ssi_mala_run),
  * "grad_group_gb" (scratch budget of the generic gradient path per group of samples; default a third of the free memory),
- * and A/B switches used by the tests: "tc_nobasis", "tc_nofuse", "tc_noorder", "tc_simt_basis", "tc_nokrev", "tc_alast",
- * "tc_k32", "tc_pair" (1 = CTA pairs with cta_group::2, the default), "b1_simt", "bm_nopack", "bm_variant", "gram_fp64",
- * "gram_chunk", "eig_cluster" (1 = dataflow cluster solver, default; 2 = cluster solver with a barrier per round; 0 = one
- * CTA), "formp_simt", "gemm_simt" (1 = gradient / training GEMMs on the SIMT kernel), "gemm_prec" (tensor-core GEMM planes:
- * 1 = FP16 with per-sample scales, default; 0 = BF16), "gemm_split_acc", "gemm_fwd_chunk", "gemm_chunk", "gemm_tc_mask" (see DESIGN.md); "time_dominant" (0/1)
- * brackets every launch of the path's dominant kernel with CUDA events (ssi_stats_t.dominant_ms) */
+ * and switches used by the tests to force a path the library also selects on its own for some shapes, or a reference
+ * kernel: "tc_nobasis", "tc_nofuse", "tc_noorder", "tc_simt_basis", "tc_pair" (1 = CTA pairs with cta_group::2, the
+ * default), "b1_simt", "gram_fp64" (1 = FP64 SIMT Gram; 0 = tensor-core Gram guarded by a conditioning check, the default;
+ * -1 = tensor-core Gram without the check), "gemm_simt" (1 = gradient / training GEMMs on the SIMT kernel); "time_dominant"
+ * (0/1) brackets every launch of the path's dominant kernel with CUDA events (ssi_stats_t.dominant_ms).  Any other key
+ * returns SSI_ERR_ARG. */
 int  ssi_set_option(ssi_ctx* ctx, const char* key, int64_t value);
 int  ssi_stats(const ssi_ctx* ctx, ssi_stats_t* out);
 

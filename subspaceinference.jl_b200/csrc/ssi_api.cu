@@ -257,34 +257,21 @@ int ssi_set_option(ssi_ctx* ctx, const char* key, int64_t value) {
     // gram_fp64: 1 = always the FP64 SIMT Gram, 0 = tensor-core Gram guarded by the conditioning check (default),
     // -1 = tensor-core Gram without the check (measurement only)
     if (!strcmp(key, "gram_fp64")) { ctx->opt_gram_fp64 = (int)value; return SSI_OK; }
-    if (!strcmp(key, "gram_chunk")) { ctx->opt_gram_chunk = (int)value; return SSI_OK; }
-    if (!strcmp(key, "eig_cluster")) { ctx->opt_eig_cluster = (int)value; return SSI_OK; }
-    if (!strcmp(key, "formp_simt")) { ctx->opt_formp_simt = value != 0; return SSI_OK; }
     if (!strcmp(key, "tc_nobasis")) { ctx->opt_tc_nobasis = value != 0; ssi_tc_invalidate(ctx); ssi_b1_invalidate(ctx); ssi_bm_invalidate(ctx); return SSI_OK; }
     if (!strcmp(key, "time_dominant")) {
         ctx->opt_time_dominant = value != 0;
         ctx->stats.dominant_ms = 0; ctx->stats.dominant_launches = 0; ctx->kt_used = 0;
         return SSI_OK;
     }
-    if (!strcmp(key, "tc_k32")) { ctx->opt_tc_k32 = value != 0; ssi_tc_invalidate(ctx); return SSI_OK; }
-    if (!strcmp(key, "tc_alast")) { ctx->opt_tc_alast = value != 0; return SSI_OK; }
-    if (!strcmp(key, "tc_nokrev")) { ctx->opt_tc_nokrev = value != 0; return SSI_OK; }
+    if (!strcmp(key, "grad_group_gb")) { ctx->opt_grad_group_gb = (int)value; return SSI_OK; }
+    if (!strcmp(key, "gemm_simt")) { ctx->opt_gemm_simt = value != 0; return SSI_OK; }
     // MALA acceptance rule: 0 (default) = the Metropolis-adjusted Langevin ratio as documented; 1 = both proposal densities
     // evaluated with the NEGATED gradient, q(a | b) = N(a - b; -(sigma^2/2) grad(a), sigma^2) -- how AdvancedMH's MALA step is
     // remembered to be written (`spl.proposal(-t_cond.gradient)`); the pinned 0.6.2 source is not available to decide
-    if (!strcmp(key, "grad_group_gb")) { ctx->opt_grad_group_gb = (int)value; return SSI_OK; }
-    if (!strcmp(key, "gemm_tc_mask")) { ctx->opt_gemm_tc_mask = (int)value; return SSI_OK; }
-    if (!strcmp(key, "gemm_prec")) { ctx->opt_gemm_prec = (int)value; return SSI_OK; }
-    if (!strcmp(key, "gemm_split_acc")) { ctx->opt_gemm_split_acc = (int)value; return SSI_OK; }
-    if (!strcmp(key, "gemm_fwd_chunk")) { ctx->opt_gemm_fwd_chunk = (int)value; return SSI_OK; }
-    if (!strcmp(key, "gemm_simt")) { ctx->opt_gemm_simt = value != 0; return SSI_OK; }
-    if (!strcmp(key, "gemm_chunk")) { ctx->opt_gemm_chunk = (int)value; return SSI_OK; }
     if (!strcmp(key, "mala_rule")) { if (value != 0 && value != 1) return ssi_fail(ctx, SSI_ERR_ARG, "mala_rule must be 0 or 1"); ctx->opt_mala_rule = (int)value; return SSI_OK; }
     if (!strcmp(key, "tc_pair")) { ctx->opt_tc_pair = value != 0; return SSI_OK; }
     if (!strcmp(key, "tc_precision")) { ctx->opt_tc_prec = value != 0; ssi_tc_invalidate(ctx); return SSI_OK; }
     if (!strcmp(key, "b1_simt")) { ctx->opt_b1_simt = value != 0; return SSI_OK; }
-    if (!strcmp(key, "bm_nopack")) { ctx->opt_bm_nopack = value != 0; ssi_bm_invalidate(ctx); return SSI_OK; }
-    if (!strcmp(key, "bm_variant")) { ctx->opt_bm_variant = (int)value; return SSI_OK; }
     if (!strcmp(key, "tc_simt_basis")) { ctx->opt_tc_simt_basis = value != 0; ssi_tc_invalidate(ctx); return SSI_OK; }
     if (!strcmp(key, "tc_noorder")) { ctx->opt_tc_noorder = value != 0; return SSI_OK; }
     return ssi_fail(ctx, SSI_ERR_ARG, "unknown option '%s'", key);

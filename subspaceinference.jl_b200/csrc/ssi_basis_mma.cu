@@ -67,25 +67,18 @@ __device__ __forceinline__ void bm_tmem_ld(uint32_t taddr, uint32_t* v) {
 }
 
 // fold SZ hidden units (TMEM columns in v, second-layer weights in wh) into the partial dot products.
-// ReLU variants (MODE): 0 every pair as (w/2) x + (w/2) |x| (FFMA2 + two FFMA with the |.| operand modifier: FMA pipes only);
-// 1 (default) every pair clamped with FMNMX (ALU pipe) then one FFMA2.  Measured on the UCI config: 373 us against 333 us, and
-// a mix of the two (one pair in four as in 0, which would balance the ALU and FMA pipes on paper) 377 us: what counts is
-// register-file traffic, six operand reads per hidden unit for 0 against four for 1.
-// Chunks start at multiples of 8 pairs, so the local pair index decides like the global one (bm_pair_half).
-__host__ __device__ constexpr bool bm_pair_half(int mode, int pair) { return mode == 0 || (mode == 2 && (pair & 3) == 3); }
-template <int ACT, int MODE, int NL, int SZ>
-__device__ __forceinline__ void bm_fold(const uint32_t* v, const float2* wh, float2* lin, float* ab4) {
+// ReLU clamps every pair with FMNMX (ALU pipe), then one FFMA2.  Writing every pair as (w/2) x + (w/2) |x| instead (FFMA2 +
+// two FFMA with the |.| operand modifier: FMA pipes only) measured 373 us against 333 us on the UCI config, and a mix of the
+// two (one pair in four as |x|, which would balance the ALU and FMA pipes on paper) 377 us: what counts is register-file
+// traffic, six operand reads per hidden unit for the |x| form against four.
+template <int ACT, int NL, int SZ>
+__device__ __forceinline__ void bm_fold(const uint32_t* v, const float2* wh, float2* lin) {
 #pragma unroll
     for (int j = 0; j < SZ; j += 2) {
         float2 x = make_float2(__uint_as_float(v[j]), __uint_as_float(v[j + 1]));
         const float2 w2 = wh[j >> 1];
-        if (ACT == SSI_ACT_RELU && bm_pair_half(MODE, j >> 1)) {
-            ab4[j & 3] = fmaf(fabsf(x.x), w2.x, ab4[j & 3]);
-            ab4[(j + 1) & 3] = fmaf(fabsf(x.y), w2.y, ab4[(j + 1) & 3]);
-        } else {
-            x.x = bm_act<ACT>(x.x);
-            x.y = bm_act<ACT>(x.y);
-        }
+        x.x = bm_act<ACT>(x.x);
+        x.y = bm_act<ACT>(x.y);
         lin[(j >> 1) & (NL - 1)] = __ffma2_rn(x, w2, lin[(j >> 1) & (NL - 1)]);
     }
 }
@@ -102,7 +95,7 @@ __device__ __forceinline__ uint64_t bm_desc(uint32_t smem_addr) {
     return d;
 }
 
-template <int ACT, int KB, int HP, bool PACKED, bool OUT_ID, int VAR>
+template <int ACT, int KB, int HP, bool PACKED, bool OUT_ID>
 __global__ void __launch_bounds__(BM_THREADS, 1)
 k_b1_mma(const __grid_constant__ CUtensorMap tmZ, const __grid_constant__ CUtensorMap tmT, const bm_params p) {
     constexpr uint32_t ROW = KB * 2;                       // bytes per operand row
@@ -209,10 +202,7 @@ k_b1_mma(const __grid_constant__ CUtensorMap tmZ, const __grid_constant__ CUtens
         const int q = warp & 3, g = (warp - 2) >> 2;      // warps 2-9; a warp may only touch TMEM lanes [32 (warp % 4), +32)
         const long long srow = (long long)block * 256 + g * 128 + q * 32 + lane;      // this thread's sample
         const bool valid = srow < p.S;
-        // second-layer weights and bias of this sample, in registers for the whole kernel (zero for padded hidden units).
-        // ReLU, VAR 0: relu(x) w = (w/2) x + (w/2) |x| -- a packed FFMA2 for two hidden units' linear parts and an FFMA with the
-        // free |.| operand modifier each, all on the FMA pipes.  VAR 1: clamp with FMNMX (ALU pipe), then one FFMA2 per pair.
-        constexpr bool HALF = ACT == SSI_ACT_RELU && VAR != 1;          // some pairs use the |x| form: their weights are halved
+        // second-layer weights and bias of this sample, in registers for the whole kernel (zero for padded hidden units)
         constexpr int DPT = BM_N / HP;                     // datapoints per tile
         float2 wh[HP / 2];
         {
@@ -220,10 +210,8 @@ k_b1_mma(const __grid_constant__ CUtensorMap tmZ, const __grid_constant__ CUtens
 #pragma unroll
             for (int j = 0; j < HP / 4; ++j) {
                 const float4 w4 = valid ? __ldg(wrow + j) : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
-                const float s0 = (ACT == SSI_ACT_RELU && bm_pair_half(VAR, 2 * j)) ? 0.5f : 1.0f;
-                const float s1 = (ACT == SSI_ACT_RELU && bm_pair_half(VAR, 2 * j + 1)) ? 0.5f : 1.0f;
-                wh[2 * j] = make_float2(s0 * w4.x, s0 * w4.y);
-                wh[2 * j + 1] = make_float2(s1 * w4.z, s1 * w4.w);
+                wh[2 * j] = make_float2(w4.x, w4.y);
+                wh[2 * j + 1] = make_float2(w4.z, w4.w);
             }
         }
         const float b2 = valid ? __ldg(p.B2 + srow) : 0.0f;
@@ -251,11 +239,10 @@ k_b1_mma(const __grid_constant__ CUtensorMap tmZ, const __grid_constant__ CUtens
 #pragma unroll
             for (int d = 0; d < DPT; ++d) yv[d] = (i_base + d < N) ? __ldg(p.Y + i_base + d) : 0.0f;
             float sse_t = 0.0f;
-            constexpr int NL = (ACT == SSI_ACT_RELU && VAR == 0) ? 2 : 4;      // independent FFMA2 chains
+            constexpr int NL = 4;                           // independent FFMA2 chains
             float2 lin[NL];
 #pragma unroll
             for (int i = 0; i < NL; ++i) lin[i] = make_float2(0.0f, 0.0f);
-            float ab4[4] = {0.0f, 0.0f, 0.0f, 0.0f};
             mbar_wait(bar_f + 8 * ab, (it >> 1) & 1);
             tc_fence_after();
             const uint32_t ta = taddr0 + ab * 128;
@@ -281,20 +268,18 @@ k_b1_mma(const __grid_constant__ CUtensorMap tmZ, const __grid_constant__ CUtens
                         tc_fence_before();
                         mbar_arrive(bar_e + 8 * ab);         // the whole accumulator is in registers
                     }
-                    if (sz == 32) bm_fold<ACT, VAR, NL, 32>(v + boff, wh + (off >> 1), lin, ab4);
-                    else if (sz == 16) bm_fold<ACT, VAR, NL, 16>(v + boff, wh + (off >> 1), lin, ab4);
-                    else bm_fold<ACT, VAR, NL, 8>(v + boff, wh + (off >> 1), lin, ab4);
+                    if (sz == 32) bm_fold<ACT, NL, 32>(v + boff, wh + (off >> 1), lin);
+                    else if (sz == 16) bm_fold<ACT, NL, 16>(v + boff, wh + (off >> 1), lin);
+                    else bm_fold<ACT, NL, 8>(v + boff, wh + (off >> 1), lin);
                     if (i == NC - 1) {                       // a datapoint is complete
                         float pre = (lin[0].x + lin[0].y) + (lin[1].x + lin[1].y);
-                        if (NL == 4) pre += (lin[NL - 2].x + lin[NL - 2].y) + (lin[NL - 1].x + lin[NL - 1].y);
-                        if (HALF) pre += (ab4[0] + ab4[1]) + (ab4[2] + ab4[3]);
+                        pre += (lin[2].x + lin[2].y) + (lin[3].x + lin[3].y);
                         pre += b2;
                         if (!OUT_ID) pre = ssi_act(pre, p.act_out);
                         const float df = (i_base + d < N) ? pre - yv[d] : 0.0f;
                         sse_t = fmaf(df, df, sse_t);
 #pragma unroll
                         for (int k = 0; k < NL; ++k) lin[k] = make_float2(0.0f, 0.0f);
-                        ab4[0] = ab4[1] = ab4[2] = ab4[3] = 0.0f;
                     }
                 }
             }
@@ -482,7 +467,7 @@ static int bm_prepare(ssi_ctx* ctx) {
     const long long N = ctx->N;
     s->KB = M1 <= 16 ? 16 : 32;
     s->Hp = H <= 32 ? 32 : (H <= 40 ? 40 : (H <= 48 ? 48 : (H <= 56 ? 56 : 64)));
-    s->packed_ns = (M1 <= 8 && !ctx->opt_bm_nopack) ? (6 * M1 + 15) / 16 : 0;
+    s->packed_ns = M1 <= 8 ? (6 * M1 + 15) / 16 : 0;
     const int slabs = s->packed_ns ? s->packed_ns : 3;
     const long long NW = N * s->Hp;
     const int NT = bm_nt(s->Hp);
@@ -504,17 +489,17 @@ static int bm_prepare(ssi_ctx* ctx) {
 
 typedef void (*bm_kernel_t)(const CUtensorMap, const CUtensorMap, const bm_params);
 template <int KB, int HP, bool PACKED, bool OUT_ID>
-static bm_kernel_t bm_pick_act(int act, int var) {
+static bm_kernel_t bm_pick_act(int act) {
     switch (act) {
-        case SSI_ACT_RELU:    return var == 1 ? k_b1_mma<SSI_ACT_RELU, KB, HP, PACKED, OUT_ID, 1> : k_b1_mma<SSI_ACT_RELU, KB, HP, PACKED, OUT_ID, 0>;
-        case SSI_ACT_TANH:    return k_b1_mma<SSI_ACT_TANH, KB, HP, PACKED, OUT_ID, 0>;
-        case SSI_ACT_SIGMOID: return k_b1_mma<SSI_ACT_SIGMOID, KB, HP, PACKED, OUT_ID, 0>;
-        default:              return k_b1_mma<SSI_ACT_IDENTITY, KB, HP, PACKED, OUT_ID, 0>;
+        case SSI_ACT_RELU:    return k_b1_mma<SSI_ACT_RELU, KB, HP, PACKED, OUT_ID>;
+        case SSI_ACT_TANH:    return k_b1_mma<SSI_ACT_TANH, KB, HP, PACKED, OUT_ID>;
+        case SSI_ACT_SIGMOID: return k_b1_mma<SSI_ACT_SIGMOID, KB, HP, PACKED, OUT_ID>;
+        default:              return k_b1_mma<SSI_ACT_IDENTITY, KB, HP, PACKED, OUT_ID>;
     }
 }
 template <int KB, int HP, bool PACKED>
-static bm_kernel_t bm_pick(int act, int act_out, int var) {
-    return act_out == SSI_ACT_IDENTITY ? bm_pick_act<KB, HP, PACKED, true>(act, var) : bm_pick_act<KB, HP, PACKED, false>(act, var);
+static bm_kernel_t bm_pick(int act, int act_out) {
+    return act_out == SSI_ACT_IDENTITY ? bm_pick_act<KB, HP, PACKED, true>(act) : bm_pick_act<KB, HP, PACKED, false>(act);
 }
 
 int ssi_reduce_partials(ssi_ctx* ctx, const double* partials, int64_t B, int parts, double* d_out);
@@ -525,12 +510,12 @@ int ssi_bm_sse(ssi_ctx* ctx, const float* dZ, int64_t B, double* d_sse) {
     const ssi_model_t& m = ctx->model;
     const int M = ctx->M, H = m.dims[1], KB = s->KB, Hp = s->Hp;
     const int slabs = s->packed_ns ? s->packed_ns : 3;
-    const int a0 = m.act[0], a1 = m.act[1], var = ctx->opt_bm_variant;
+    const int a0 = m.act[0], a1 = m.act[1];
     bm_kernel_t kern = nullptr;
 #define BM_PICK_HP(HPV)                                                                                      \
     if (Hp == HPV)                                                                                           \
-        kern = s->packed_ns ? bm_pick<16, HPV, true>(a0, a1, var)                                            \
-                            : (KB == 16 ? bm_pick<16, HPV, false>(a0, a1, var) : bm_pick<32, HPV, false>(a0, a1, var));
+        kern = s->packed_ns ? bm_pick<16, HPV, true>(a0, a1)                                                 \
+                            : (KB == 16 ? bm_pick<16, HPV, false>(a0, a1) : bm_pick<32, HPV, false>(a0, a1));
     BM_PICK_HP(32) BM_PICK_HP(40) BM_PICK_HP(48) BM_PICK_HP(56) BM_PICK_HP(64)
 #undef BM_PICK_HP
     if (!kern) return ssi_fail(ctx, SSI_ERR_UNSUPPORTED, "basis mma path: no kernel for padded hidden width %d", Hp);

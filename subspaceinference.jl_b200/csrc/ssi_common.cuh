@@ -58,28 +58,16 @@ struct ssi_ctx {
     int opt_path = SSI_PATH_AUTO;
     int opt_group = 0;
     int opt_tc_nofuse = 0;    // debugging / A-B: compute the output layer as its own GEMM
-    int opt_tc_noorder = 0;
-    int opt_tc_k32 = 0;       // A-B: K-major bases always 32 columns wide
-    int opt_tc_alast = 1;     // evict-first hint on the last read of a row block's activations (A-B: 0)
-    int opt_tc_nokrev = 0;    // A-B: every feature tile reads the k-blocks in ascending order
+    int opt_tc_noorder = 0;   // debugging / A-B: sample-major work order on the first layer
     int opt_grad_group_gb = 0; // scratch budget (GB) of the generic gradient path per group of samples (default 6)
-    int opt_gemm_tc_mask = 0; // 0 all; else which GEMM orientations may use the tensor cores (see ssi_gemm_tc.cu)
-    int opt_gemm_prec = 1;    // tensor-core GEMM planes: 1 FP16 with a per-operand scale (FP32-grade), 0 BF16 (no pre-pass)
-    int opt_gemm_split_acc = 2; // tensor-core GEMM: separate accumulator for the small terms: 2 forward layers only (default), 1 all, 0 none
-    int opt_gemm_fwd_chunk = 0; // accumulation chunk (k-blocks) of the forward layers when their accumulators are split
     int opt_gemm_simt = 0;    // 1: keep the gradient / training GEMMs on the SIMT kernel (A-B against ssi_gemm_tc.cu)
-    int opt_gemm_chunk = 0;   // k-blocks (32 k) per FP32 accumulation chunk of the tensor-core GEMM (default 32)
     int opt_mala_rule = 0;    // 0 textbook MALA ratio, 1 negated-gradient proposal densities (see ssi_api.cu)
     int opt_tc_pair = 1;      // GEMM layers with per-sample activations as CTA pairs (cta_group::2); 0: one CTA per tile (A-B)
     int opt_tc_prec = 1;      // operand planes of the tensor path: 1 mixed BF16/FP16 (default), 0 BF16x3 (round 1)
-    int opt_bm_nopack = 0, opt_bm_variant = 1;     // A-B inside k_b1_mma: unpacked operands; ReLU epilogue variant
     int opt_b1_simt = 0;       // A-B: BASIS path on CUDA cores (k_logpost_basis1h) instead of the tensor-core kernel (k_b1_mma)
     int opt_tc_simt_basis = 0; // A-B: first layer as the FP32 SIMT basis combination instead of the tensor-core one
     int opt_gram_fp64 = 0;    // force the FP64 SIMT Gram (default: tensor-core TF32x2 Gram for large n, K <= 128)
-    int opt_formp_simt = 0;   // A-B: P = A V_M with loads from global memory (k_form_p) instead of the TMA-staged stream
-    int opt_eig_cluster = 1;  // eigen-solve (K <= 160) on a cluster of eight CTAs (2: its first version); 0: one CTA (A-B)
-    int opt_gram_chunk = 0;   // tiles (64 rows) per FP32 accumulation chunk of the tensor-core Gram (default 16)
-    int opt_tc_nobasis = 0;   // debugging / A-B: run the first layer as a GEMM instead of the affine-in-z basis combination   // debugging / A-B: sample-major work order on the first layer
+    int opt_tc_nobasis = 0;   // debugging / A-B: run the first layer as a GEMM instead of the affine-in-z basis combination
 
     // model / data / subspace
     ssi_model_t model;

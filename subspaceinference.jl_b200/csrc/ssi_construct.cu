@@ -200,9 +200,9 @@ int ssi_subspace_gram(ssi_ctx* ctx) {
 //      Newton step in FP64; c = rsqrt(1 + t^2), s = t c are orthogonal to working precision by construction, so
 //      accuracy does not depend on t -- only the convergence rate does.
 //   3. With the columns mutually orthogonal,  L V = U S:  lambda_i = |column i|^2 and Pi' u_i is the eigenvector.
-//   K <= 160: one CTA, the matrix lives in shared memory.  Larger K (README's batchsize-1 loader gives K = 1000, SURVEY
-//   Q3): a cooperative grid with the matrix in global memory (L2-resident) and a grid barrier per round; no pair tables,
-//   so K is limited by memory only (ssi_swa_* accept K <= 16384).
+//   K <= 160: a cluster of 8 CTAs, the columns live in shared memory (k_osj_cluster2).  Larger K (README's batchsize-1
+//   loader gives K = 1000, SURVEY Q3): a cooperative grid with the matrix in global memory (L2-resident) and a grid barrier
+//   per round (k_osj); no pair tables, so K is limited by memory only (ssi_swa_* accept K <= 16384).
 // ======================================================================================
 #define OSJ_THREADS 1024
 #define OSJ_SMEM_KMAX 160
@@ -290,11 +290,9 @@ __device__ void osj_pivoted_cholesky(double* __restrict__ G, int K, int ld, int*
 }
 
 __global__ void __launch_bounds__(OSJ_THREADS)
-k_osj(double* __restrict__ Gg /* K x K column-major Gram; on exit the orthogonalised columns of its Cholesky factor */, int K, int max_sweeps,
+k_osj(double* __restrict__ G /* K x K column-major Gram; on exit the orthogonalised columns of its Cholesky factor */, int K, int max_sweeps,
       unsigned* __restrict__ sync_counter /* zeroed */, unsigned* __restrict__ rot_count /* [3], zeroed */,
-      int* __restrict__ perm /* K: row r of the result is original index perm[r] */, int* __restrict__ sweeps_out, int use_smem) {
-    extern __shared__ double osj_smem[];
-    double* G = use_smem ? osj_smem : Gg;
+      int* __restrict__ perm /* K: row r of the result is original index perm[r] */, int* __restrict__ sweeps_out) {
     __shared__ double red[32];
     __shared__ double s_tr;
     const int tid = threadIdx.x, nt = blockDim.x;
@@ -302,11 +300,9 @@ k_osj(double* __restrict__ Gg /* K x K column-major Gram; on exit the orthogonal
     unsigned target = 0;
     if (blockIdx.x == 0) {
         double tr = 0.0;
-        for (int i = tid; i < K; i += nt) tr += fabs(Gg[i + (long long)i * K]);
+        for (int i = tid; i < K; i += nt) tr += fabs(G[i + (long long)i * K]);
         tr = ssi_block_sum(tr, red);
         if (tid == 0) s_tr = tr;
-        if (use_smem)
-            for (long long e = tid; e < (long long)K * K; e += nt) G[e] = Gg[e];
         __syncthreads();
         osj_pivoted_cholesky(G, K, K, perm, (double)K * 2.220446049250313e-16 * s_tr);
     }
@@ -368,172 +364,32 @@ k_osj(double* __restrict__ Gg /* K x K column-major Gram; on exit the orthogonal
         // every rotation of this sweep has been counted before the last barrier of the sweep
         if (*reinterpret_cast<volatile unsigned*>(cnt) == 0u) { ++sweep; converged = true; break; }
     }
-    if (use_smem)
-        for (long long e = tid; e < (long long)K * K; e += nt) Gg[e] = G[e];
     // sweeps executed (the last one without a rotation), or max_sweeps + 1 when the last sweep still rotated
     if (blockIdx.x == 0 && tid == 0) *sweeps_out = converged ? sweep : max_sweeps + 1;
 }
 
 // The same solver for K <= 160 on a CLUSTER of 8 CTAs (distributed shared memory): on one SM the ~K^2 / 2 column updates of a
-// round are issue-bound (2.7 us per round at K = 100, measured); spread over eight SMs a round costs one pair's
-// latency chain plus a hardware cluster barrier.  Every CTA starts from its own copy of the Cholesky factor (computed
-// redundantly, bit-identically).  In every round a CTA orthogonalises the pairs that fall to its half warps, reading
-// its LOCAL shared memory, and writes each of the two columns -- rotated or not -- into the shared memory of the ONE CTA
-// that will own it in the next round (st.shared::cluster; the round-robin schedule is a closed formula, so the next
-// owner is computed, not communicated).  A column is thus valid exactly where it is needed: 2 column transfers per pair
-// and round (80 KB per round over the whole cluster at K = 100) instead of a broadcast.
+// round are issue-bound (2.7 us per round at K = 100, measured; one CTA took 2.8 ms for the whole solve); spread over eight
+// SMs a round costs one pair's latency chain.  Every CTA starts from its own copy of the Cholesky factor (computed
+// redundantly, bit-identically).  In every round a CTA orthogonalises the pairs that fall to its warps, reading its LOCAL
+// shared memory, and writes each of the two columns -- rotated or not -- into the shared memory of the ONE CTA that will
+// own it in the next round (the round-robin schedule is a closed formula, so the next owner is computed, not
+// communicated).  A column is thus valid exactly where it is needed: 2 column transfers per pair and round (80 KB per
+// round over the whole cluster at K = 100) instead of a broadcast.
 #define OSJC_CTAS 8
 #define OSJC_THREADS 512
 #define OSJC_HW (OSJC_THREADS / 32)        // warps (pairs) per CTA and pass: one warp per pair
-#define OSJC_IT ((OSJ_SMEM_KMAX + 31) / 32)   // elements of a column per lane
+static_assert((OSJ_SMEM_KMAX + 1) / 2 <= OSJC_CTAS * OSJC_HW, "k_osj_cluster2 needs a warp for every column pair");
 __device__ __forceinline__ uint32_t osjc_mapa(uint32_t local_addr, uint32_t rank) {
     uint32_t r;
     asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(local_addr), "r"(rank));
     return r;
 }
-__device__ __forceinline__ void osjc_st_f64(uint32_t cluster_addr, double v) {
-    asm volatile("st.shared::cluster.f64 [%0], %1;" ::"r"(cluster_addr), "d"(v) : "memory");
-}
 __device__ __forceinline__ void osjc_st_u32(uint32_t cluster_addr, unsigned v) {
     asm volatile("st.shared::cluster.u32 [%0], %1;" ::"r"(cluster_addr), "r"(v) : "memory");
 }
-// pairs of round r: slot 0 = (m - 1, r), slot i = ((r + i) mod (m - 1), (r - i) mod (m - 1)); slot i belongs to half warp
-// i mod (8 * 16), i.e. to CTA (i mod 128) / 16
-__device__ __forceinline__ int osjc_owner(int x, int r, int m) {
-    int i;
-    if (x == m - 1 || x == r) i = 0;
-    else {
-        i = x - r; if (i < 0) i += m - 1;                  // x = (r + i) mod (m - 1)
-        if (i >= m / 2) i = (m - 1) - i;                   // else x = (r - i) mod (m - 1)
-    }
-    return (i % (OSJC_CTAS * OSJC_HW)) / OSJC_HW;
-}
-__global__ void __cluster_dims__(OSJC_CTAS, 1, 1) __launch_bounds__(OSJC_THREADS)
-k_osj_cluster(double* __restrict__ Gg, int K, int max_sweeps, int* __restrict__ perm_out, int* __restrict__ sweeps_out) {
-    extern __shared__ double osj_smem[];
-    double* G = osj_smem;                                     // K x K
-    int* s_perm = reinterpret_cast<int*>(G + (size_t)K * K);  // K
-    __shared__ double red[32];
-    __shared__ double s_tr;
-    __shared__ unsigned s_cnt, s_slot[OSJC_CTAS], s_mx, s_mxslot[OSJC_CTAS];
-    const int tid = threadIdx.x, nt = blockDim.x;
-    const uint32_t rank = cluster_ctarank();
-    {
-        double tr = 0.0;
-        for (int i = tid; i < K; i += nt) tr += fabs(Gg[i + (long long)i * K]);
-        tr = ssi_block_sum(tr, red);
-        if (tid == 0) { s_tr = tr; s_cnt = 0; s_mx = 0; }
-        for (long long e = tid; e < (long long)K * K; e += nt) G[e] = Gg[e];
-        __syncthreads();
-        osj_pivoted_cholesky(G, K, K, s_perm, (double)K * 2.220446049250313e-16 * s_tr);
-    }
-    cluster_sync_all();
-    const double tol = (double)K * 2.220446049250313e-16, tol2 = tol * tol;
-    const int m = (K + 1) & ~1, np = m / 2;
-    const int hw = (int)rank * OSJC_HW + (tid >> 5), n_hw = OSJC_CTAS * OSJC_HW;
-    const int hl = tid & 31;
-    const uint32_t g_local = smem_u32(G);
-    int sweep = 0;
-    bool converged = false;
-    for (; sweep < max_sweeps; ++sweep) {
-        for (int r = 0; r < m - 1; ++r) {
-            const int rn = (r + 1 == m - 1) ? 0 : r + 1;                  // the schedule is cyclic across sweeps
-            for (int i = hw; i < np; i += n_hw) {
-                int p, q;
-                if (i == 0) { p = m - 1; q = r; }
-                else { p = r + i; if (p >= m - 1) p -= m - 1; q = r - i; if (q < 0) q += m - 1; }
-                if (p > q) { const int t = p; p = q; q = t; }
-                const double* gp = G + (long long)p * K;
-                const uint32_t dst_p = osjc_mapa(g_local, (uint32_t)osjc_owner(p, rn, m)) + (uint32_t)(p * K) * 8u;
-                if (q >= K) {                                               // bye: the column only moves on
-                    for (int k = hl; k < K; k += 32) osjc_st_f64(dst_p + (uint32_t)k * 8u, gp[k]);
-                    continue;
-                }
-                const double* gq = G + (long long)q * K;
-                const uint32_t dst_q = osjc_mapa(g_local, (uint32_t)osjc_owner(q, rn, m)) + (uint32_t)(q * K) * 8u;
-                // the lane's elements of both columns stay in registers: all loads leave before the first use
-                double x[OSJC_IT], y[OSJC_IT];
-#pragma unroll
-                for (int it = 0; it < OSJC_IT; ++it) {
-                    const int k = hl + 32 * it;
-                    x[it] = k < K ? gp[k] : 0.0;
-                    y[it] = k < K ? gq[k] : 0.0;
-                }
-                double a = 0.0, b = 0.0, c = 0.0;
-#pragma unroll
-                for (int it = 0; it < OSJC_IT; ++it) { a = fma(x[it], x[it], a); b = fma(y[it], y[it], b); c = fma(x[it], y[it], c); }
-#pragma unroll
-                for (int o = 16; o > 0; o >>= 1) {
-                    a += __shfl_xor_sync(0xffffffffu, a, o);
-                    b += __shfl_xor_sync(0xffffffffu, b, o);
-                    c += __shfl_xor_sync(0xffffffffu, c, o);
-                }
-                const double c2 = c * c, ab = a * b;
-                double cs = 1.0, sn = 0.0;
-                if (c2 > tol2 * ab) {
-                    const double d = b - a, h = 2.0 * c;
-                    const int ex = max(__double2hiint(fabs(d)), __double2hiint(fabs(h))) >> 20;
-                    const double sc = __hiloint2double((2046 - ex) << 20, 0);
-                    const float df = (float)(d * sc), hf = (float)(h * sc);
-                    const float rf = sqrtf(fmaf(df, df, hf * hf));
-                    double t = (double)(hf / (df + copysignf(rf, df)));
-                    const double f = fma(h * t, t, fma(2.0 * d, t, -h));
-                    t -= f * (double)(1.0f / (float)((2.0 * (h * t + d)) * sc)) * sc;
-                    cs = rsqrt(fma(t, t, 1.0));
-                    sn = t * cs;
-                    if (hl == 0) {
-                        // largest cos^2 rotated away in this sweep (single precision is plenty: it is compared with 1e-15)
-                        const int e2 = __double2hiint(ab) >> 20;
-                        const double s2 = __hiloint2double((2046 - e2) << 20, 0);
-                        atomicAdd(&s_cnt, 1u);
-                        atomicMax(&s_mx, __float_as_uint(fminf((float)(c2 * s2) / (float)(ab * s2), 1.0f)));
-                    }
-                }
-#pragma unroll
-                for (int it = 0; it < OSJC_IT; ++it) {
-                    const int k = hl + 32 * it;
-                    if (k < K) {
-                        osjc_st_f64(dst_p + (uint32_t)k * 8u, cs * x[it] - sn * y[it]);
-                        osjc_st_f64(dst_q + (uint32_t)k * 8u, sn * x[it] + cs * y[it]);
-                    }
-                }
-            }
-            if (r == m - 2) {       // last round of the sweep: publish this CTA's rotation count before the barrier
-                __syncthreads();
-                if (tid < OSJC_CTAS) {
-                    osjc_st_u32(osjc_mapa(smem_u32(&s_slot[rank]), (uint32_t)tid), s_cnt);
-                    osjc_st_u32(osjc_mapa(smem_u32(&s_mxslot[rank]), (uint32_t)tid), s_mx);
-                }
-            }
-            cluster_sync_all();
-        }
-        unsigned total = 0, mx = 0;
-#pragma unroll
-        for (int c = 0; c < OSJC_CTAS; ++c) { total += s_slot[c]; mx = max(mx, s_mxslot[c]); }
-        __syncthreads();
-        if (tid == 0) { s_cnt = 0; s_mx = 0; }
-        __syncthreads();
-        // converged when nothing was rotated, or when every rotation of the sweep was so small (cos < 3e-8) that what it
-        // leaves behind is of second order, cos^2 < 1e-15 (quadratic convergence of the Jacobi method)
-        if (total == 0u || __uint_as_float(mx) < 1e-15f) { ++sweep; converged = true; break; }
-    }
-    // every column is valid in the CTA that owns it in round 0 (the round after the last one): that CTA writes it out
-    for (int i = hw; i < np; i += n_hw) {
-        int p = (i == 0) ? m - 1 : i, q = (i == 0) ? 0 : m - 1 - i;        // round 0: (r + i, r - i) mod (m - 1) with r = 0
-        for (int k = hl; k < K; k += 32) {
-            if (p < K) Gg[k + (long long)p * K] = G[k + (long long)p * K];
-            if (q < K) Gg[k + (long long)q * K] = G[k + (long long)q * K];
-        }
-    }
-    cluster_sync_all();           // no CTA leaves while a peer may still write into its shared memory
-    if (rank == 0) {
-        for (int i = tid; i < K; i += nt) perm_out[i] = s_perm[i];
-        if (tid == 0) *sweeps_out = converged ? sweep : max_sweeps + 1;
-    }
-}
-
-// Second version of the cluster solver (default; the one above stays as option eig_cluster = 2 for A-B).  Same schedule,
-// no barrier: the solver's time is 891 rounds of one rotation each at K = 100, so what counts is the latency of a round.
+// This is the second version of the cluster solver; the first one (a cluster barrier per round) took 1.62 ms at K = 100
+// against 0.77 ms.  The solver's time is 891 rounds of one rotation each at K = 100, so what counts is the latency of a round.
 //   * DATAFLOW instead of a cluster barrier per round.  A rotated column goes to the shared memory of its next owner with
 //     st.async, which completes transaction bytes on an mbarrier of the warp that will consume it (one mbarrier per pair slot
 //     and round parity); that warp posts arrive.expect_tx for its two columns and waits on its own barrier only.  The first
@@ -609,7 +465,7 @@ k_osj_cluster2(double* __restrict__ Gg, int K, int max_sweeps, int* __restrict__
     cluster_sync_all();
     const double tol = (double)K * 2.220446049250313e-16, tol2 = tol * tol;
     const int m = (K + 1) & ~1, np = m / 2;
-    const int spc = (np + OSJC_CTAS - 1) / OSJC_CTAS;         // pair slots per CTA (<= OSJC_HW, checked by the host)
+    const int spc = (np + OSJC_CTAS - 1) / OSJC_CTAS;         // pair slots per CTA (<= OSJC_HW for K <= OSJ_SMEM_KMAX)
     const int slot = (int)rank * spc + wid;                   // this warp's pair slot in every round
     const bool has_pair = wid < spc && slot < np;
     const uint32_t g_local = smem_u32(G), bar_local = smem_u32(&s_bar[0][0]);
@@ -737,99 +593,6 @@ k_osj_cluster2(double* __restrict__ Gg, int K, int max_sweeps, int* __restrict__
         for (int i = tid; i < K; i += nt) perm_out[i] = s_perm[i];
         if (tid == 0) *sweeps_out = converged ? sweep : max_sweeps + 1;
     }
-}
-
-// One CTA, one warp per pair, the matrix in shared memory, one __syncthreads per round (option eig_cluster = 0, A-B).  The
-// cluster kernel above pays ~1 us per round for its cluster barrier (release of the remote stores + arrive + wait; ncu: 46 %
-// of its samples), but this one is bound by the FP64 pipe of its single SM -- ~70 FP64 warp instructions per pair, 3.5 us per
-// round at K = 100: 3.2 ms against 2.05 ms on the cluster.
-#define OSJS_THREADS 1024
-__global__ void __launch_bounds__(OSJS_THREADS)
-k_osj_smem(double* __restrict__ Gg, int K, int max_sweeps, int* __restrict__ perm_out, int* __restrict__ sweeps_out) {
-    extern __shared__ double osj_smem[];
-    double* G = osj_smem;                                     // K x K
-    int* s_perm = reinterpret_cast<int*>(G + (size_t)K * K);  // K
-    __shared__ double red[32];
-    __shared__ double s_tr;
-    __shared__ unsigned s_cnt, s_mx;
-    const int tid = threadIdx.x, nt = blockDim.x;
-    {
-        double tr = 0.0;
-        for (int i = tid; i < K; i += nt) tr += fabs(Gg[i + (long long)i * K]);
-        tr = ssi_block_sum(tr, red);
-        if (tid == 0) { s_tr = tr; s_cnt = 0; s_mx = 0; }
-        for (long long e = tid; e < (long long)K * K; e += nt) G[e] = Gg[e];
-        __syncthreads();
-        osj_pivoted_cholesky(G, K, K, s_perm, (double)K * 2.220446049250313e-16 * s_tr);
-    }
-    const double tol = (double)K * 2.220446049250313e-16, tol2 = tol * tol;
-    const int m = (K + 1) & ~1, np = m / 2;
-    const int wid = tid >> 5, n_w = nt >> 5, hl = tid & 31;
-    int sweep = 0;
-    bool converged = false;
-    for (; sweep < max_sweeps; ++sweep) {
-        for (int r = 0; r < m - 1; ++r) {
-            for (int i = wid; i < np; i += n_w) {
-                int p, q;
-                if (i == 0) { p = m - 1; q = r; }
-                else { p = r + i; if (p >= m - 1) p -= m - 1; q = r - i; if (q < 0) q += m - 1; }
-                if (p > q) { const int t = p; p = q; q = t; }
-                if (q >= K) continue;                                       // bye
-                double* gp = G + (long long)p * K;
-                double* gq = G + (long long)q * K;
-                double x[OSJC_IT], y[OSJC_IT];
-#pragma unroll
-                for (int it = 0; it < OSJC_IT; ++it) {
-                    const int k = hl + 32 * it;
-                    x[it] = k < K ? gp[k] : 0.0;
-                    y[it] = k < K ? gq[k] : 0.0;
-                }
-                double a = 0.0, b = 0.0, c = 0.0;
-#pragma unroll
-                for (int it = 0; it < OSJC_IT; ++it) { a = fma(x[it], x[it], a); b = fma(y[it], y[it], b); c = fma(x[it], y[it], c); }
-#pragma unroll
-                for (int o = 16; o > 0; o >>= 1) {
-                    a += __shfl_xor_sync(0xffffffffu, a, o);
-                    b += __shfl_xor_sync(0xffffffffu, b, o);
-                    c += __shfl_xor_sync(0xffffffffu, c, o);
-                }
-                const double c2 = c * c, ab = a * b;
-                if (c2 <= tol2 * ab) continue;
-                const double d = b - a, h = 2.0 * c;
-                const int ex = max(__double2hiint(fabs(d)), __double2hiint(fabs(h))) >> 20;
-                const double sc = __hiloint2double((2046 - ex) << 20, 0);
-                const float df = (float)(d * sc), hf = (float)(h * sc);
-                const float rf = sqrtf(fmaf(df, df, hf * hf));
-                double t = (double)(hf / (df + copysignf(rf, df)));
-                const double f = fma(h * t, t, fma(2.0 * d, t, -h));
-                t -= f * (double)(1.0f / (float)((2.0 * (h * t + d)) * sc)) * sc;
-                const double cs = rsqrt(fma(t, t, 1.0)), sn = t * cs;
-                if (hl == 0) {
-                    const int e2 = __double2hiint(ab) >> 20;
-                    const double s2 = __hiloint2double((2046 - e2) << 20, 0);
-                    atomicAdd(&s_cnt, 1u);
-                    atomicMax(&s_mx, __float_as_uint(fminf((float)(c2 * s2) / (float)(ab * s2), 1.0f)));
-                }
-#pragma unroll
-                for (int it = 0; it < OSJC_IT; ++it) {
-                    const int k = hl + 32 * it;
-                    if (k < K) {
-                        gp[k] = cs * x[it] - sn * y[it];
-                        gq[k] = sn * x[it] + cs * y[it];
-                    }
-                }
-            }
-            __syncthreads();
-        }
-        const unsigned total = s_cnt, mx = s_mx;
-        __syncthreads();
-        if (tid == 0) { s_cnt = 0; s_mx = 0; }
-        __syncthreads();
-        if (total == 0u || __uint_as_float(mx) < 1e-15f) { ++sweep; converged = true; break; }
-    }
-    for (long long e = tid; e < (long long)K * K; e += nt) Gg[e] = G[e];
-    for (int i = tid; i < K; i += nt) perm_out[i] = s_perm[i];
-    if (tid == 0) *sweeps_out = converged ? sweep : max_sweeps + 1;
 }
 
 // eigenvalues = squared norms of the orthogonalised columns, rank-sorted descending (ties by index); eigenvectors = the
@@ -1023,8 +786,7 @@ static int launch_form_p(ssi_ctx* ctx, const float* dA, int64_t n, int64_t ld, i
     const int Kpad = (K + FP_KC - 1) / FP_KC * FP_KC;
     const size_t v_bytes = sizeof(float) * (size_t)Kpad * MP;
     const size_t smem_tma = (size_t)FP_STAGES * FP_STAGE_BYTES + v_bytes + 2 * FP_STAGES * 8;
-    if (MP <= 32 && smem_tma <= ctx->smem_optin && (ld % 4) == 0 && ((reinterpret_cast<uintptr_t>(dA) & 15) == 0) && n < (1ll << 31) &&
-        !ctx->opt_formp_simt) {
+    if (MP <= 32 && smem_tma <= ctx->smem_optin && (ld % 4) == 0 && ((reinterpret_cast<uintptr_t>(dA) & 15) == 0) && n < (1ll << 31)) {
         PFN_ssi_encodeTiled encode = nullptr;
         SSI_TRY(ssi_tensormap_encoder(ctx, &encode));
         CUtensorMap map;
@@ -1134,19 +896,12 @@ int ssi_swa_eigen_stage(ssi_ctx* ctx, int M, const double* dG_src, bool check, b
     SSI_TRY(swa_eig_layout(ctx, K, e));
     if (dG_src != e.dG)
         SSI_CUDA(ctx, cudaMemcpyAsync(e.dG, dG_src, sizeof(double) * (size_t)K * K, cudaMemcpyDeviceToDevice, ctx->stream));
-    // one-sided Jacobi: in shared memory on one CTA for small K, else a cooperative grid on the matrix in global memory
+    // one-sided Jacobi: on a cluster of 8 CTAs with the columns in shared memory for small K, else a cooperative grid on the
+    // matrix in global memory
     unsigned* d_sync = reinterpret_cast<unsigned*>(e.dSweeps + 1);       // [sync counter | 3 rotation counters]
     SSI_CUDA(ctx, cudaMemsetAsync(d_sync, 0, 4 * sizeof(unsigned), ctx->stream));
-    const int use_smem = K <= OSJ_SMEM_KMAX;
-    const size_t jsm = use_smem ? sizeof(double) * (size_t)K * K : 0;
-    if (jsm > 48 * 1024) SSI_CUDA(ctx, cudaFuncSetAttribute(k_osj, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)jsm));
-    int grid = 1;
-    if (!use_smem) {
-        const int np = (K + 1) / 2;
-        grid = std::max(1, std::min(ctx->sm_count, (np * 16 + OSJ_THREADS - 1) / OSJ_THREADS));
-    }
-    if (use_smem && ctx->opt_eig_cluster == 1 && (K + 1) / 2 <= OSJC_CTAS * OSJC_HW) {
-        // a cluster of 8 CTAs, one warp per column pair, each column in the shared memory of the CTA that needs it next
+    if (K <= OSJ_SMEM_KMAX) {
+        // one warp per column pair, each column in the shared memory of the CTA that needs it next
         const int it = (K + 31) / 32;
         const size_t csm = sizeof(double) * (size_t)K * it * 32 + sizeof(int) * (size_t)K;
 #define OSJC2_LAUNCH(IT_)                                                                                                       \
@@ -1162,24 +917,18 @@ int ssi_swa_eigen_stage(ssi_ctx* ctx, int M, const double* dG_src, bool check, b
             default: OSJC2_LAUNCH(5); break;
         }
 #undef OSJC2_LAUNCH
-    } else if (use_smem && ctx->opt_eig_cluster) {
-        const size_t csm = jsm + sizeof(int) * (size_t)K;
-        SSI_CUDA(ctx, cudaFuncSetAttribute(k_osj_cluster, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)csm));
-        k_osj_cluster<<<OSJC_CTAS, OSJC_THREADS, csm, ctx->stream>>>(e.dG, K, 60, e.dPerm, e.dSweeps);
-    } else if (use_smem) {
-        const size_t csm = jsm + sizeof(int) * (size_t)K;
-        SSI_CUDA(ctx, cudaFuncSetAttribute(k_osj_smem, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)csm));
-        k_osj_smem<<<1, OSJS_THREADS, csm, ctx->stream>>>(e.dG, K, 60, e.dPerm, e.dSweeps);
     } else {
+        const int np = (K + 1) / 2;
+        const int grid = std::max(1, std::min(ctx->sm_count, (np * 16 + OSJ_THREADS - 1) / OSJ_THREADS));
         double* Gp = e.dG;
-        int Kv = K, ms = 60, us = use_smem;
+        int Kv = K, ms = 60;
         unsigned* sc = d_sync;
         unsigned* rc = d_sync + 1;
         int* so = e.dSweeps;
         int* pm = e.dPerm;
-        void* args[] = {&Gp, &Kv, &ms, &sc, &rc, &pm, &so, &us};
-        if (grid > 1) SSI_CUDA(ctx, cudaLaunchCooperativeKernel((const void*)k_osj, dim3(grid), dim3(OSJ_THREADS), args, jsm, ctx->stream));
-        else SSI_CUDA(ctx, cudaLaunchKernel((const void*)k_osj, dim3(1), dim3(OSJ_THREADS), args, jsm, ctx->stream));
+        void* args[] = {&Gp, &Kv, &ms, &sc, &rc, &pm, &so};
+        if (grid > 1) SSI_CUDA(ctx, cudaLaunchCooperativeKernel((const void*)k_osj, dim3(grid), dim3(OSJ_THREADS), args, 0, ctx->stream));
+        else SSI_CUDA(ctx, cudaLaunchKernel((const void*)k_osj, dim3(1), dim3(OSJ_THREADS), args, 0, ctx->stream));
     }
     SSI_LAUNCH_CHECK(ctx);
     k_osj_norms<<<(K * 32 + 255) / 256, 256, 0, ctx->stream>>>(e.dG, K, e.dNorms);

@@ -10,20 +10,18 @@
 //   * warp 0 lands raw FP32 tiles with TMA: A 128 (o) x 32 (k), B 256 (j) x 32 (k), either orientation (k-fast tiles
 //     arrive as [rows][32 k] with 128-byte swizzle, o- / j-fast tiles as [32 k][rows]); edges are zero-filled by TMA;
 //   * eight converter warps split every raw tile into two 16-bit planes in the K-major SWIZZLE_64B operand layout
-//     (transposing the o- / j-fast tiles on the way; both access patterns are conflict-free).  Default: FP16 planes
+//     (transposing the o- / j-fast tiles on the way; both access patterns are conflict-free): FP16 planes
 //     hi = fp16(s x), lo = fp16(s x - hi) with one power-of-two scale s per operand AND BATCH that puts that batch's
 //     largest magnitude at 2^14 (a strided absmax pre-pass, k_gemm_absmax; per batch so that a sample's result cannot
-//     depend on what else is in the launch): 11 + 11 bits for everything within 2^-17 of the largest element.  Option
-//     gemm_prec = 0: BF16 planes without scale or pre-pass (8 + 8 bits: the forward pass then carries 2^-17 per operand,
-//     5e-5 of the gradient norm on the test shapes).  Orientation and plane format are template parameters;
+//     depend on what else is in the launch): 11 + 11 bits for everything within 2^-17 of the largest element (BF16 planes,
+//     8 + 8 bits, left 5e-5 of the gradient norm on the test shapes: DESIGN.md 4.5).  The orientation is a template parameter;
 //   * one thread issues  D += Al Bh' + Ah Bl' + Ah Bh'  (tcgen05.mma kind::f16, M = 128, N = 256, FP32 accumulators in
 //     TMEM, two accumulator buffers).  The forward layers (bias + activation epilogue) keep the two small terms in an
 //     accumulator of their own: they are 2^-11 of the large term, and added into the same truncating accumulator they
 //     lose the bits below the running sum's ulp -- most of what the lo planes carry.  That, not the length of the
 //     accumulation, was the 3.7e-5 of the gradient norm the first version of this kernel showed on the wide network
 //     (FP32 FMA chains: 1.8e-5; with the split: 1.35e-5).  It costs the double buffering of those launches (+7 % on the
-//     whole gradient), so the backward GEMMs, whose results are sums the error averages out of, do without
-//     (option gemm_split_acc: 2 forward only, 1 all, 0 none);
+//     whole gradient), so the backward GEMMs, whose results are sums the error averages out of, do without;
 //   * four epilogue warps drain an accumulator every `chunk` k-blocks (1024 k): the tensor core's FP32 accumulation
 //     truncates, so a long contraction (the weight gradient runs over all N datapoints) is summed in FP32 through the
 //     output tile itself (each tile has one owner: plain read-add-write), and the last chunk applies the epilogue
@@ -39,7 +37,6 @@
 #include "ssi_ptx.cuh"
 #include "ssi_gemm.cuh"
 
-#include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include <algorithm>
 
@@ -62,7 +59,7 @@
 #define GX_EPW 16                                    // output columns per epilogue pass (= one tcgen05.ld of 16 columns)
 
 struct gemm_tc_params {
-    const float* amaxA;          // device: largest |A| per batch (one entry when A is shared), NULL with BF16 planes.  Per batch, not per
+    const float* amaxA;          // device: largest |A| per batch (one entry when A is shared).  Per batch, not per
     const float* amaxB;          // launch: a sample's result must not depend on which other samples share its launch
     float* C; long long c_sj, c_sb;
     int O, J;
@@ -90,37 +87,23 @@ __device__ __forceinline__ int gx_scale_exp(float mx) {
     return (mx > 0.0f && mx < 3.0e38f) ? max(-100, min(100, 14 - ilogbf(mx))) : 0;
 }
 // eight consecutive k of one row -> one 16-byte chunk of each plane
-template <bool F16>
 __device__ __forceinline__ void gx_split8(const float v[8], uint4& hi, uint4& lo, float sc) {
     uint32_t h[4], l[4];
-    if (F16) {
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            const float a = v[2 * i] * sc, b = v[2 * i + 1] * sc;
-            const __half2 hh = __floats2half2_rn(a, b);
-            h[i] = *reinterpret_cast<const uint32_t*>(&hh);
-            const float2 f = __half22float2(hh);
-            const __half2 lh = __floats2half2_rn(a - f.x, b - f.y);
-            l[i] = *reinterpret_cast<const uint32_t*>(&lh);
-        }
-        hi = make_uint4(h[0], h[1], h[2], h[3]);
-        lo = make_uint4(l[0], l[1], l[2], l[3]);
-        return;
-    }
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
-        const __nv_bfloat162 hb = __floats2bfloat162_rn(v[2 * i], v[2 * i + 1]);
-        h[i] = *reinterpret_cast<const uint32_t*>(&hb);
-        const float f0 = __uint_as_float(h[i] << 16), f1 = __uint_as_float(h[i] & 0xffff0000u);
-        const __nv_bfloat162 lb = __floats2bfloat162_rn(v[2 * i] - f0, v[2 * i + 1] - f1);
-        l[i] = *reinterpret_cast<const uint32_t*>(&lb);
+        const float a = v[2 * i] * sc, b = v[2 * i + 1] * sc;
+        const __half2 hh = __floats2half2_rn(a, b);
+        h[i] = *reinterpret_cast<const uint32_t*>(&hh);
+        const float2 f = __half22float2(hh);
+        const __half2 lh = __floats2half2_rn(a - f.x, b - f.y);
+        l[i] = *reinterpret_cast<const uint32_t*>(&lh);
     }
     hi = make_uint4(h[0], h[1], h[2], h[3]);
     lo = make_uint4(l[0], l[1], l[2], l[3]);
 }
 
-// raw FP32 tile (ROWS x 32 k) -> planes H, L ([ROWS][32] BF16, 64-byte rows, SWIZZLE_64B); ct = converter thread 0..255
-template <int ROWS, bool KFAST, bool F16>
+// raw FP32 tile (ROWS x 32 k) -> planes H, L ([ROWS][32] FP16, 64-byte rows, SWIZZLE_64B); ct = converter thread 0..255
+template <int ROWS, bool KFAST>
 __device__ __forceinline__ void gx_convert(const uint8_t* __restrict__ raw, uint8_t* __restrict__ H, uint8_t* __restrict__ L, int ct, float sc) {
 #pragma unroll 2
     for (int i = ct; i < ROWS * 4; i += GX_CONV * 32) {
@@ -140,15 +123,15 @@ __device__ __forceinline__ void gx_convert(const uint8_t* __restrict__ raw, uint
             for (int e = 0; e < 8; ++e) v[e] = src[e * ROWS];
         }
         uint4 hi, lo;
-        gx_split8<F16>(v, hi, lo, sc);
+        gx_split8(v, hi, lo, sc);
         const uint32_t off = (uint32_t)r * 64u + (uint32_t)((q ^ ((r >> 1) & 3)) << 4);      // SWIZZLE_64B: chunk ^ bits [7, 9) of the address
         *reinterpret_cast<uint4*>(H + off) = hi;
         *reinterpret_cast<uint4*>(L + off) = lo;
     }
 }
 
-// AK / BK: the raw tiles of A / B are k-fast; F16: FP16 planes with per-batch scales (else BF16 planes)
-template <bool AK, bool BK, bool F16>
+// AK / BK: the raw tiles of A / B are k-fast
+template <bool AK, bool BK>
 __global__ void __launch_bounds__(GX_THREADS, 1)
 k_gemm_tc(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const gemm_tc_params p) {
     extern __shared__ __align__(1024) uint8_t smem[];
@@ -205,8 +188,7 @@ k_gemm_tc(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
     } else if (warp == 1) {
         // ================= MMA issuer =================
         if (lane == 0) {
-            const uint32_t fmt = F16 ? UMMA_FMT_F16 : UMMA_FMT_BF16;
-            const uint32_t idesc = umma_idesc_f16(GX_BN, fmt, fmt);
+            const uint32_t idesc = umma_idesc_f16(GX_BN, UMMA_FMT_F16, UMMA_FMT_F16);
             int stage = 0;
             uint32_t phase = 0;
             unsigned cidx = 0;
@@ -229,7 +211,7 @@ k_gemm_tc(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
                         const uint64_t dBh = umma_desc_sw64(op + 2 * GX_OP_A), dBl = umma_desc_sw64(op + 2 * GX_OP_A + GX_OP_B);
 #pragma unroll
                         for (int ks = 0; ks < GX_BK / 16; ++ks) {
-                            const uint64_t ko = (uint64_t)(ks * 32 >> 4);      // 16 BF16 = 32 bytes per k-step inside the 64-byte row
+                            const uint64_t ko = (uint64_t)(ks * 32 >> 4);      // 16 FP16 = 32 bytes per k-step inside the 64-byte row
                             umma_bf16(d_small, dAl + ko, dBh + ko, idesc, first ? 0u : 1u);
                             umma_bf16(d_small, dAh + ko, dBl + ko, idesc, 1u);
                             umma_bf16(d_acc, dAh + ko, dBh + ko, idesc, (first && p.split_acc) ? 0u : 1u);
@@ -249,15 +231,15 @@ k_gemm_tc(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
         uint32_t phase = 0;
         for (long long w = blockIdx.x; w < p.n_work; w += gridDim.x) {
             const int b = (int)(w / tiles_per_batch);
-            const float scA = F16 ? scalbnf(1.0f, gx_scale_exp(p.amaxA[p.a_batched ? b : 0])) : 1.0f;
-            const float scB = F16 ? scalbnf(1.0f, gx_scale_exp(p.amaxB[p.b_batched ? b : 0])) : 1.0f;
+            const float scA = scalbnf(1.0f, gx_scale_exp(p.amaxA[p.a_batched ? b : 0]));
+            const float scB = scalbnf(1.0f, gx_scale_exp(p.amaxB[p.b_batched ? b : 0]));
             for (int kb = 0; kb < p.n_kb; ++kb) {
                 mbar_wait(bar_rfull + 8 * stage, phase);
                 mbar_wait(bar_oempty + 8 * stage, phase ^ 1);          // the MMAs that read this operand slot have retired
                 const uint8_t* raw = smem + stage * GX_RAW_STAGE;
                 uint8_t* op = smem + GX_OFF_OP + stage * GX_OP_STAGE;
-                gx_convert<GX_BM, AK, F16>(raw, op, op + GX_OP_A, ct, scA);
-                gx_convert<GX_BN, BK, F16>(raw + GX_RAW_A, op + 2 * GX_OP_A, op + 2 * GX_OP_A + GX_OP_B, ct, scB);
+                gx_convert<GX_BM, AK>(raw, op, op + GX_OP_A, ct, scA);
+                gx_convert<GX_BN, BK>(raw + GX_RAW_A, op + 2 * GX_OP_A, op + 2 * GX_OP_A + GX_OP_B, ct, scB);
                 fence_proxy_async();                   // generic-proxy writes -> visible to the tensor core (async proxy)
                 __syncwarp();
                 if (lane == 0) {
@@ -278,7 +260,7 @@ k_gemm_tc(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
             const int o = to * GX_BM + q * 32 + lane;
             float* crow = p.C + (long long)b * p.c_sb + o;
             const float bias = (p.epi == 1 && o < p.O) ? p.bias[(long long)b * p.bias_sb + o] : 0.0f;
-            const float unscale = F16 ? scalbnf(1.0f, -(gx_scale_exp(p.amaxA[p.a_batched ? b : 0]) + gx_scale_exp(p.amaxB[p.b_batched ? b : 0]))) : 1.0f;
+            const float unscale = scalbnf(1.0f, -(gx_scale_exp(p.amaxA[p.a_batched ? b : 0]) + gx_scale_exp(p.amaxB[p.b_batched ? b : 0])));
             for (int c = 0; c < n_chunks; ++c, ++cidx) {
                 const uint32_t ab = p.split_acc ? 0u : (cidx & 1u), aphase = p.split_acc ? (cidx & 1u) : ((cidx >> 1) & 1u);
                 mbar_wait(bar_tfull + 8 * ab, aphase);
@@ -393,10 +375,6 @@ static bool gx_aligned(const void* p, long long stride_elems) {
 int ssi_gemm_tc_try(ssi_ctx* ctx, const gemm_t& g, int batches, bool a_kfast, bool b_jfast, bool* used) {
     *used = false;
     if (ctx->opt_gemm_simt || g.split > 0 || g.c_so != 1 || batches < 1) return SSI_OK;
-    // A-B switch per operand orientation: bit 0 forward (A o-fast, B k-fast), bit 1 weight gradient (A o-fast, B j-fast),
-    // bit 2 back-propagated delta (A k-fast, B k-fast), bit 3 the rest
-    const int kind = (!a_kfast && !b_jfast) ? 1 : (!a_kfast && b_jfast) ? 2 : (a_kfast && !b_jfast) ? 4 : 8;
-    if (ctx->opt_gemm_tc_mask && !(ctx->opt_gemm_tc_mask & kind)) return SSI_OK;
     if (g.O < 1 || g.J < 64 || g.K < 8 || g.K >= (1ll << 31)) return SSI_OK;
     // small problems: launch + pipeline fill would dominate.  Per batch, NOT per launch: which kernel evaluates a sample must
     // not depend on how many other samples share the call (results are compared bitwise across batch compositions)
@@ -433,40 +411,35 @@ int ssi_gemm_tc_try(ssi_ctx* ctx, const gemm_t& g, int batches, bool a_kfast, bo
                                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) return SSI_OK;
     }
+    // one scale per operand and batch: the largest magnitude over what that batch reads (stream-ordered scratch of the context)
+    const int nbA = a_b ? batches : 1, nbB = b_b ? batches : 1;
+    SSI_TRY(ssi_reserve(ctx, ctx->bGemmAmax, (size_t)(nbA + nbB) * sizeof(float)));
+    float* am = (float*)ctx->bGemmAmax.p;
+    SSI_CUDA(ctx, cudaMemsetAsync(am, 0, (size_t)(nbA + nbB) * sizeof(float), ctx->stream));
+    const long long rowsA = a_kfast ? g.O : g.K, fastA = a_kfast ? g.K : g.O, ldA = a_kfast ? g.a_so : g.a_sk;
+    const long long rowsB = b_jfast ? g.K : g.J, fastB = b_jfast ? g.J : g.K, ldB = b_jfast ? g.b_sk : g.b_sj;
+    const int blocks = 16 * ctx->sm_count;
+    k_gemm_absmax<<<(unsigned)std::min<long long>(blocks, (rowsA * nbA + 7) / 8), 256, 0, ctx->stream>>>(g.A, fastA, ldA, rowsA, g.a_sb, rowsA * nbA, am);
+    SSI_LAUNCH_CHECK(ctx);
+    k_gemm_absmax<<<(unsigned)std::min<long long>(blocks, (rowsB * nbB + 7) / 8), 256, 0, ctx->stream>>>(g.B, fastB, ldB, rowsB, g.b_sb, rowsB * nbB, am + nbA);
+    SSI_LAUNCH_CHECK(ctx);
     gemm_tc_params p{};
-    if (ctx->opt_gemm_prec != 0) {
-        // one scale per operand and batch: the largest magnitude over what that batch reads (stream-ordered scratch of the context)
-        const int nbA = a_b ? batches : 1, nbB = b_b ? batches : 1;
-        SSI_TRY(ssi_reserve(ctx, ctx->bGemmAmax, (size_t)(nbA + nbB) * sizeof(float)));
-        float* am = (float*)ctx->bGemmAmax.p;
-        SSI_CUDA(ctx, cudaMemsetAsync(am, 0, (size_t)(nbA + nbB) * sizeof(float), ctx->stream));
-        const long long rowsA = a_kfast ? g.O : g.K, fastA = a_kfast ? g.K : g.O, ldA = a_kfast ? g.a_so : g.a_sk;
-        const long long rowsB = b_jfast ? g.K : g.J, fastB = b_jfast ? g.J : g.K, ldB = b_jfast ? g.b_sk : g.b_sj;
-        const int blocks = 16 * ctx->sm_count;
-        k_gemm_absmax<<<(unsigned)std::min<long long>(blocks, (rowsA * nbA + 7) / 8), 256, 0, ctx->stream>>>(g.A, fastA, ldA, rowsA, g.a_sb, rowsA * nbA, am);
-        SSI_LAUNCH_CHECK(ctx);
-        k_gemm_absmax<<<(unsigned)std::min<long long>(blocks, (rowsB * nbB + 7) / 8), 256, 0, ctx->stream>>>(g.B, fastB, ldB, rowsB, g.b_sb, rowsB * nbB, am + nbA);
-        SSI_LAUNCH_CHECK(ctx);
-        p.amaxA = am;
-        p.amaxB = am + nbA;
-    }
+    p.amaxA = am;
+    p.amaxB = am + nbA;
     p.C = g.C; p.c_sj = g.c_sj; p.c_sb = g.c_sb;
     p.O = g.O; p.J = g.J;
     p.n_to = (g.O + GX_BM - 1) / GX_BM;
     p.n_tj = (g.J + GX_BN - 1) / GX_BN;
     p.n_work = (long long)p.n_to * p.n_tj * batches;
     p.n_kb = (int)((g.K + GX_BK - 1) / GX_BK);
-    p.chunk = ctx->opt_gemm_chunk > 0 ? ctx->opt_gemm_chunk : 32;
+    p.chunk = 32;
     p.a_kfast = a_kfast ? 1 : 0; p.b_kfast = b_jfast ? 0 : 1;
     p.a_batched = a_b ? 1 : 0; p.b_batched = b_b ? 1 : 0;
-    p.split_acc = (ctx->opt_gemm_split_acc == 1 || (ctx->opt_gemm_split_acc == 2 && g.epi == 1)) ? 1 : 0;
-    if (p.split_acc && g.epi == 1 && ctx->opt_gemm_fwd_chunk > 0) p.chunk = ctx->opt_gemm_fwd_chunk;
+    p.split_acc = g.epi == 1 ? 1 : 0;
     p.epi = g.epi; p.act = g.act; p.bias = g.bias; p.bias_sb = g.bias_sb; p.Hprev = g.Hprev; p.h_sb = g.h_sb;
     typedef void (*gx_kernel_t)(const CUtensorMap, const CUtensorMap, const gemm_tc_params);
-    static const gx_kernel_t kernels[8] = {k_gemm_tc<false, false, false>, k_gemm_tc<false, false, true>, k_gemm_tc<false, true, false>,
-                                           k_gemm_tc<false, true, true>,   k_gemm_tc<true, false, false>, k_gemm_tc<true, false, true>,
-                                           k_gemm_tc<true, true, false>,   k_gemm_tc<true, true, true>};
-    const gx_kernel_t kern = kernels[(p.a_kfast ? 4 : 0) + (p.b_kfast ? 2 : 0) + (p.amaxA ? 1 : 0)];
+    static const gx_kernel_t kernels[4] = {k_gemm_tc<false, false>, k_gemm_tc<false, true>, k_gemm_tc<true, false>, k_gemm_tc<true, true>};
+    const gx_kernel_t kern = kernels[(p.a_kfast ? 2 : 0) + (p.b_kfast ? 1 : 0)];
     SSI_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, GX_SMEM));
     const int grid = (int)std::min<long long>(ctx->sm_count, p.n_work);
     kern<<<grid, GX_THREADS, GX_SMEM, ctx->stream>>>(mapA, mapB, p);

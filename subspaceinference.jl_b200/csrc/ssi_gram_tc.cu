@@ -291,7 +291,7 @@ int ssi_gram_tc_device(ssi_ctx* ctx, const float* dA, int64_t n, int64_t ld, int
     p.tiles_total = (n + GT_ROWS - 1) / GT_ROWS;
     const int grid = (int)std::min<long long>(ctx->sm_count, p.tiles_total);
     p.tiles_per_cta = (p.tiles_total + grid - 1) / grid;
-    p.chunk = ctx->opt_gram_chunk > 0 ? ctx->opt_gram_chunk : 16;       // 1024 rows per FP32 chunk
+    p.chunk = 16;                                                       // 1024 rows per FP32 chunk
     const int elems = 2 * p.NP * 128;
     SSI_TRY(ssi_reserve(ctx, ctx->bGram, sizeof(double) * (size_t)(grid + 1) * elems));
     p.partial = (double*)ctx->bGram.p;

@@ -55,7 +55,6 @@ typedef __nv_bfloat16 bf16;
 // ---------------------------------------------------------------------------------------
 struct tc_params {
     int N, G, m_tiles, n_tiles, k_blocks, BN, width, a_shared, act;
-    int a_last_first;       // A loads of the last feature tile carry the evict-first hint
     int k_rev;              // odd feature tiles read the k-blocks in descending order (L2 reuse of the A row block)
     int a_il;               // A operand planes interleaved per k-block: row = [kb][hi 64 | lo 64] (the basis layer's output)
     int stages, stage_bytes;
@@ -233,7 +232,7 @@ k_tc_layer(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__ CUt
                         const int kbe = (p.k_rev && (nt & 1)) ? p.k_blocks - 1 - kb : kb;
                         const int ka = p.a_il ? 2 * kbe * TC_BK : kbe * TC_BK;
                         // the last feature tile is the last reader of this row block's activations: let them go first
-                        const uint64_t pa = (p.a_last_first && !p.a_shared && nt == p.n_tiles - 1) ? TC_EVICT_FIRST : pol_a;
+                        const uint64_t pa = (!p.a_shared && nt == p.n_tiles - 1) ? TC_EVICT_FIRST : pol_a;
                         if (PAIR) {
                             const int brow = nt * BN + (int)crank * (BN / 2);          // this CTA's half of the weight tile (the maps' box is BN/2 rows)
                             tma_load_3d_pair_hint(sA, &tmAh, full, ka, mt * TC_BM, g, pa);
@@ -1326,7 +1325,7 @@ int ssi_tc_prepare(ssi_ctx* ctx) {
         const size_t NW = (size_t)N * s->width[0];
         SSI_CUDA(ctx, cudaMalloc(&s->Bh, sizeof(bf16) * 2 * (size_t)G * NW));
         if (s->basis_mma) {
-            s->KT = (ctx->M + 1 <= 24 && !ctx->opt_tc_k32) ? 24 : 32;
+            s->KT = ctx->M + 1 <= 24 ? 24 : 32;
             SSI_CUDA(ctx, cudaMalloc(&s->Th, sizeof(bf16) * NW * s->KT));
             SSI_CUDA(ctx, cudaMalloc(&s->Tl, sizeof(bf16) * NW * s->KT));
             SSI_CUDA(ctx, cudaMalloc(&s->Zh, sizeof(bf16) * 128 * 32));
@@ -1493,8 +1492,7 @@ int ssi_tc_sse(ssi_ctx* ctx, const float* dZ, int64_t B, double* d_sse) {
             p.k_blocks = s->Kp[l] / TC_BK;
             p.a_shared = (l == 0);
             p.a_il = (l == 1 && s->basis) ? 1 : 0;
-            p.k_rev = (!p.a_shared && !ctx->opt_tc_nokrev) ? 1 : 0;
-            p.a_last_first = ctx->opt_tc_alast;
+            p.k_rev = !p.a_shared ? 1 : 0;
             p.act = m.act[l];
             // CTA pairs for the layers with per-sample activations (weight rows split across the pair: BN / 2 must be a whole
             // number of 8-row swizzle atoms and a legal MMA N half)

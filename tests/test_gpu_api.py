@@ -97,3 +97,21 @@ def test_next_rows_golden(ssi, engine):
     mean, std = engine.predict(g["pred_Z"], g["pred_Xg"])
     np.testing.assert_allclose(mean, g["pred_mean"], rtol=1e-5, atol=1e-6)
     np.testing.assert_allclose(std, g["pred_std"], rtol=1e-4, atol=1e-6)
+
+
+# every option key with its default value; setting it leaves the context as it was
+KEPT_OPTIONS = {"path": 0, "group": 0, "grad_group_gb": 0, "time_dominant": 0, "mala_rule": 0, "tc_precision": 1,
+                "gram_fp64": 0, "gemm_simt": 0, "b1_simt": 0, "tc_pair": 1, "tc_nobasis": 0, "tc_nofuse": 0,
+                "tc_simt_basis": 0, "tc_noorder": 0}
+# A-B switches whose losing variants have been removed from the library
+REMOVED_OPTIONS = ("eig_cluster", "formp_simt", "gram_chunk", "gemm_prec", "gemm_split_acc", "gemm_fwd_chunk", "gemm_chunk",
+                   "gemm_tc_mask", "tc_k32", "tc_nokrev", "tc_alast", "bm_variant", "bm_nopack")
+
+
+def test_option_keys(ssi, engine):
+    for key, value in KEPT_OPTIONS.items():
+        engine.set_option(key, value)
+    for key in REMOVED_OPTIONS:
+        with pytest.raises(ssi.SsiError) as e:
+            engine.set_option(key, 0)
+        assert e.value.code == -1 and "unknown option" in str(e.value), key

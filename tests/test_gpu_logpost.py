@@ -222,7 +222,7 @@ def test_gradient_vs_oracle(ssi, engine, dims, acts, N, M, B):
     ((11, 44, 1), (1, 0), 501, 9, 130),        # Hp = 48 (TMEM chunks 32 + 16), M + 1 = 10: three-way split as six MMAs, K = 16
     ((8, 37, 1), (3, 0), 77, 2, 9),            # Hp = 40 (chunks 32 + 8), odd number of datapoints: half-empty last tile
 ])
-def test_basis_path_on_tensor_cores_vs_oracle(ssi, engine, dims, acts, N, M, B):
+def test_basis_path_kernels_vs_oracle(ssi, engine, dims, acts, N, M, B):
     """BASIS path, tensor-core kernel (samples along the MMA M dimension) and CUDA-core kernel: both within 1e-5 of the
     Float64 oracle; the tensor-core result of a sample is bitwise independent of the batch it arrives in."""
     rng = np.random.default_rng(stable_seed(dims, N, M, B, "bm"))
@@ -246,9 +246,3 @@ def test_basis_path_on_tensor_cores_vs_oracle(ssi, engine, dims, acts, N, M, B):
     engine.set_option("b1_simt", 0)
     k = min(B, 3)
     np.testing.assert_array_equal(engine.logpost(Z[:, B - k:], 0.7), out[0][B - k:])
-    # A-B switches of the tensor-core kernel: six MMAs of a three-way split instead of products packed along K; the
-    # ReLU-by-|x| epilogue
-    for key in ("bm_nopack", "bm_variant"):
-        engine.set_option(key, 1 if key == "bm_nopack" else 0)
-        np.testing.assert_allclose(engine.logpost(Z, 0.7), ref, rtol=RTOL, err_msg=key)
-        engine.set_option(key, 0 if key == "bm_nopack" else 1)
