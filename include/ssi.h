@@ -81,8 +81,8 @@ typedef struct ssi_stats_t {
     double last_bytes;         /* algorithmic HBM bytes of that call (construction streams), else 0     */
     double last_units;         /* (sample x datapoint) units of that call                              */
     int64_t kernel_launches;   /* kernels launched by this context since creation                      */
-    int64_t mh_accepts;        /* accepted proposals in the last ssi_mh_run (all chains)               */
-    int64_t mh_proposals;      /* proposals in the last ssi_mh_run                                     */
+    int64_t mh_accepts;        /* accepted proposals in the last ssi_mh_run / ssi_mala_run / ssi_hmc_run */
+    int64_t mh_proposals;      /* proposals (transitions) in that run                                  */
     int32_t last_path;         /* SSI_PATH_* actually used by the last log-posterior evaluation        */
     int32_t sm_count;
     int32_t gram_path;         /* last ssi_swa_finish: 1 FP64 SIMT Gram, 2 tensor-core Gram, 3 tensor-core Gram
@@ -104,7 +104,8 @@ int  ssi_version(void);
 /* ---- lifecycle ------------------------------------------------------------------- */
 int  ssi_ctx_create(int device, ssi_ctx** out);
 /* One context over n_dev devices (SURVEY 8(b)-1): W_swa, P, X, Y are replicated on every device; ssi_logpost_batch,
- * ssi_logpost_grad_batch, ssi_mh_run, ssi_mala_run, ssi_mh_run_from, ssi_mh_get_state and ssi_project split their B samples /
+ * ssi_logpost_grad_batch, ssi_mh_run, ssi_mala_run, ssi_mh_run_from, ssi_hmc_run, ssi_mh_get_state, ssi_hmc_get_adapt and
+ * ssi_project split their B samples /
  * n_chains chains into contiguous ranges, one per device (chains keep their global ids: traces are bit-identical to a
  * one-device run); ssi_predict_batch, ssi_swa_* and ssi_train_* run on devices[0] (an installed subspace is replicated).
  * The *_dev entry points and ssi_set_stream take pointers / streams of ONE device and return SSI_ERR_UNSUPPORTED here.
@@ -217,6 +218,46 @@ int  ssi_mh_run_from(ssi_ctx* ctx, int32_t kind, int64_t n_chains, int64_t n_ste
 int  ssi_mh_run_from_dev(ssi_ctx* ctx, int32_t kind, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset,
                          int64_t step_offset, double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask,
                          const float* d_z_state, float* d_z_trace, double* d_lp_trace, uint8_t* d_accept_trace);
+/* ---- fixed-length HMC with per-chain step-size adaptation (alg = :static_hmc) -------------------------------------------
+ * AdvancedHMC's StaticTrajectory / Turing's HMC(eps, n_leapfrog) with a diagonal inverse metric, on the density of ssi_mh_run
+ * (values and gradients from ssi_logpost_grad_batch_dev, n_leapfrog evaluations per transition).  Same arguments, streams
+ * and trace layouts as ssi_mh_run.  Sample 0 is z_state (or sigma_z*eps(chain,0)) and counts as the first of n_steps.
+ * Transition t >= 1 of a chain:
+ *   p_i = n_i / sqrt(inv_metric_i) (FP64), n = the FP32 normals of stream 0 at (chain, t) -- what ssi_rng_replay returns;
+ *   p += eps/2 g(z); n_leapfrog - 1 times { z_i = float((double)z_i + eps inv_metric_i p_i); g = grad lp(z); p += eps g };
+ *   z_i = float((double)z_i + eps inv_metric_i p_i); g = grad lp(z); p += eps/2 g;
+ *   H = -lp + 1/2 sum inv_metric_i p_i^2 (FP64); accept iff -e(chain,t) < -(H' - H)  (e: the Exp(1) variate of RWMH).
+ * The transition is divergent (rejected; accept_trace 2) when a drift yields a non-finite z or H' - H is non-finite or
+ * > 1000; the chain's position is then held at the trajectory's start, so no NaN or Inf reaches the density.
+ * Step size: dual averaging per chain (Hoffman & Gelman 2014, Alg. 5; gamma 0.05, t0 10, kappa 0.75, mu = log(10 eps0),
+ * delta = target_accept) after each transition m = t <= n_adapts, from (log eps, log eps_bar, H_bar) = (log eps0, 0, 0);
+ * transition t uses exp(log eps) while t <= n_adapts and exp(log eps_bar) afterwards (n_adapts == 0: eps0 throughout).
+ * Adaptation never pools across chains, so traces do not depend on which chains share a call or a device.
+ *   step_size_trace  n_chains x n_steps doubles (or NULL): the eps each transition used; NaN for step 0
+ *   accept_trace     1 accepted, 0 rejected, 2 rejected as divergent
+ *   step_offset > 0  continues chains from z_state (the state after step step_offset - 1, ssi_mh_get_state) and, unless
+ *                    n_adapts == 0, adapt_state (3 x n_chains, ssi_hmc_get_adapt): run(0..S) is bit-identical to run(0..h)
+ *                    followed by run(h..S) for every h, in warm-up or after it
+ * The final (z, lp) is read with ssi_mh_get_state; ssi_hmc_get_adapt returns the 3 x n_chains adaptation state of the last
+ * run (SSI_ERR_STATE if the last run on the context was not HMC).  inv_metric is a host pointer in both variants.       */
+typedef struct ssi_hmc_params_t {
+    double  step_size;        /* initial leapfrog step size eps0 > 0                                    */
+    int32_t n_leapfrog;       /* leapfrog steps per transition, >= 1                                    */
+    int64_t n_adapts;         /* transitions 1..n_adapts adapt eps (dual averaging); 0 = fixed eps0     */
+    double  target_accept;    /* delta in (0, 1); AdvancedHMC's StepSizeAdaptor(0.8, ...)               */
+    const double* inv_metric; /* M doubles (host, copied), diagonal of M^-1; NULL = identity             */
+} ssi_hmc_params_t;
+int  ssi_hmc_run(ssi_ctx* ctx, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset, int64_t step_offset,
+                 const ssi_hmc_params_t* hp, double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask,
+                 const float* z_state, const double* adapt_state,
+                 float* z_trace, double* lp_trace, uint8_t* accept_trace, double* step_size_trace);
+/* same; z_state, adapt_state and the traces are device pointers (hp->inv_metric stays a host pointer); asynchronous */
+int  ssi_hmc_run_dev(ssi_ctx* ctx, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset, int64_t step_offset,
+                     const ssi_hmc_params_t* hp, double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask,
+                     const float* d_z_state, const double* d_adapt_state,
+                     float* d_z_trace, double* d_lp_trace, uint8_t* d_accept_trace, double* d_step_size_trace);
+/* 3 x n_chains doubles (host): log eps, log eps_bar, H_bar of every chain of the last HMC run */
+int  ssi_hmc_get_adapt(ssi_ctx* ctx, double* adapt_out);
 /* host replay of the device stream: eps_out (M floats, N(0,1)) and e_out (Exp(1)) of (chain, step) */
 int  ssi_rng_replay(uint64_t seed, int64_t chain, int64_t step, int32_t M, float* eps_out, double* e_out);
 /* map(z -> W_swa + P*z, chm) (src/space_inference.jl:125): W_out n x B column-major (host) */

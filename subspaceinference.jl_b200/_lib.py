@@ -41,6 +41,12 @@ class Stats(C.Structure):
     ]
 
 
+class HmcParams(C.Structure):
+    """ssi_hmc_params_t."""
+    _fields_ = [("step_size", C.c_double), ("n_leapfrog", C.c_int32), ("n_adapts", C.c_int64), ("target_accept", C.c_double),
+                ("inv_metric", C.c_void_p)]
+
+
 _p, _i64, _i32, _u32, _u64, _dbl = C.c_void_p, C.c_int64, C.c_int32, C.c_uint32, C.c_uint64, C.c_double
 
 # name -> (restype, argtypes); kept in one table so tests can check it against include/ssi.h
@@ -70,6 +76,9 @@ SIGNATURES = {
     "ssi_mh_get_state": (C.c_int, [_p, _p, _p]),
     "ssi_mh_run_from": (C.c_int, [_p, _i32, _i64, _i64, _u64, _i64, _i64, _dbl, _dbl, _dbl, _u32, _p, _p, _p, _p]),
     "ssi_mh_run_from_dev": (C.c_int, [_p, _i32, _i64, _i64, _u64, _i64, _i64, _dbl, _dbl, _dbl, _u32, _p, _p, _p, _p]),
+    "ssi_hmc_run": (C.c_int, [_p, _i64, _i64, _u64, _i64, _i64, C.POINTER(HmcParams), _dbl, _dbl, _dbl, _u32, _p, _p, _p, _p, _p, _p]),
+    "ssi_hmc_run_dev": (C.c_int, [_p, _i64, _i64, _u64, _i64, _i64, C.POINTER(HmcParams), _dbl, _dbl, _dbl, _u32, _p, _p, _p, _p, _p, _p]),
+    "ssi_hmc_get_adapt": (C.c_int, [_p, _p]),
     "ssi_rng_replay": (C.c_int, [_u64, _i64, _i64, _i32, _p, _p]),
     "ssi_project": (C.c_int, [_p, _p, _i64, _p]),
     "ssi_predict_batch": (C.c_int, [_p, _p, _i64, _p, _i64, _p, _p, _p]),

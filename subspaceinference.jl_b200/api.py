@@ -18,10 +18,54 @@ from .engine import Engine
 from .flux import ADAM, Chain, DataLoader, Descent, extract_params, load_params, mse, split_data, train_step
 
 _RWMH_ALIASES = ("rwmh", "mh")
+_DEVICE_ALGS = (*_RWMH_ALIASES, "mala", "static_hmc")
 
 
 def _sym(s) -> str:
     return str(s).lstrip(":")
+
+
+def _check_alg(a: str):
+    if a not in _DEVICE_ALGS:
+        if a in ("advi", "hmc", "nuts"):
+            # the reference's :hmc is NUTS with Stan's windowed adaptation (AdvancedHMC); the device's fixed-length sampler
+            # is a different algorithm and answers to :static_hmc only
+            raise NotImplementedError(f"{a} is not available on the device path (Engine.logpost_grad is its l_pi_grad; "
+                                      "alg=:static_hmc is the device's fixed-length HMC)")
+        raise ValueError(f"{a} is not available")                         # src/space_inference.jl:162, :316
+
+
+def _hmc_options(itr: int, M: int, n_leapfrog, step_size, n_adapts, target_accept, inv_metric) -> dict:
+    """Validated keywords of alg=:static_hmc (ValueError before any context exists)."""
+    if isinstance(n_leapfrog, bool) or int(n_leapfrog) != n_leapfrog or n_leapfrog < 1:
+        raise ValueError(f"n_leapfrog must be an integer >= 1 (got {n_leapfrog!r})")
+    step_size = float(step_size)
+    if not (np.isfinite(step_size) and step_size > 0):
+        raise ValueError(f"step_size must be positive and finite (got {step_size!r})")
+    n_adapts = itr // 2 if n_adapts is None else n_adapts
+    if isinstance(n_adapts, bool) or int(n_adapts) != n_adapts or n_adapts < 0:
+        raise ValueError(f"n_adapts must be an integer >= 0 (got {n_adapts!r})")
+    target_accept = float(target_accept)
+    if not 0.0 < target_accept < 1.0:
+        raise ValueError(f"target_accept must be in (0, 1) (got {target_accept!r})")
+    if inv_metric is not None:
+        inv_metric = np.asarray(inv_metric, dtype=np.float64).reshape(-1)
+        if inv_metric.shape[0] != M or not (np.all(np.isfinite(inv_metric)) and np.all(inv_metric > 0)):
+            raise ValueError(f"inv_metric must hold M={M} positive finite values")
+    return dict(n_leapfrog=int(n_leapfrog), step_size=step_size, n_adapts=int(n_adapts), target_accept=target_accept,
+                inv_metric=inv_metric)
+
+
+def _sample(eng: Engine, a: str, n_chains: int, itr: int, seed: int, σ_z, σ_m, σ_p, prior_mask, chain_offset, hmc):
+    """(z_trace, lp_trace) of the device sampler `a`; warm-up transitions of :static_hmc stay in the trace, as AdvancedHMC's
+    `sample` keeps them by default."""
+    if a == "static_hmc":
+        zt, lt, _, _ = eng.hmc_run(n_chains, itr, seed, sigma_z=σ_z, sigma_m=σ_m, sigma_p=σ_p, mask=prior_mask,
+                                   chain_offset=chain_offset, want_accept=False, want_step_size=False, **hmc)
+        return zt, lt
+    zt, lt, _ = eng.mh_run(n_chains, itr, seed, sigma_z=σ_z, sigma_m=σ_m, sigma_p=σ_p, mask=prior_mask,
+                           chain_offset=chain_offset, want_accept=False, kind="mala" if a == "mala" else "rwmh")
+    return zt, lt
 
 
 def shard_rows(n: int, rank: int, world: int):
@@ -128,17 +172,21 @@ def _train_on_device(eng: Engine, model, cost, data, opt, T: int, c: int, print_
 def sub_inference(in_model, data, W_swa, P, *, σ_z: float = 1.0, σ_m: float = 1.0, σ_p: float = 1.0, itr: int = 100,
                   M: int = 3, alg="rwmh", backend="forwarddiff",
                   n_chains: int = 1, seed: int = 0, chain_offset: int = 0, prior_mask: int = TERM_LL,
-                  engine: Engine | None = None, device: int = 0, return_z: bool = False):
+                  engine: Engine | None = None, device: int = 0, return_z: bool = False,
+                  n_leapfrog: int = 10, step_size: float = 0.1, n_adapts: int | None = None, target_accept: float = 0.8,
+                  inv_metric=None):
     """RWMH in the subspace.  Returns (chn, lp): with n_chains == 1 (the reference) `chn` is a
     list of `itr` weight vectors W_swa + P z and `lp` the `itr` log-probabilities
     (src/space_inference.jl:125).  With n_chains > 1 `chn` is the (M, n_chains, itr) array of
     subspace samples (materialising itr x n_chains weight vectors is what the device path
-    avoids; use Engine.project on the samples you need) and lp is (n_chains, itr)."""
+    avoids; use Engine.project on the samples you need) and lp is (n_chains, itr).
+
+    alg=:static_hmc runs fixed-length HMC on the device (n_leapfrog leapfrog steps per transition, initial step size
+    step_size adapted per chain by dual averaging over the first n_adapts transitions (default itr // 2) towards
+    target_accept, diagonal inverse metric inv_metric (default ones)); the warm-up samples stay in the returned trace."""
     a = _sym(alg)
-    if a not in _RWMH_ALIASES and a != "mala":
-        if a in ("advi", "hmc", "nuts"):
-            raise NotImplementedError(f"{a} is not available on the device path (Engine.logpost_grad is its l_pi_grad)")
-        raise ValueError(f"{a} is not available")                         # src/space_inference.jl:162
+    _check_alg(a)
+    hmc = _hmc_options(itr, M, n_leapfrog, step_size, n_adapts, target_accept, inv_metric) if a == "static_hmc" else None
     if not isinstance(in_model, Chain):
         raise TypeError("Error: density function is not avaliable for this model")   # :103
     P = np.asarray(P)
@@ -151,8 +199,7 @@ def sub_inference(in_model, data, W_swa, P, *, σ_z: float = 1.0, σ_m: float = 
         eng.set_model(in_model.dims, in_model.acts)
         eng.set_data(X, Y)
         eng.set_subspace(W_swa, P)
-        zt, lt, _ = eng.mh_run(n_chains, itr, seed, sigma_z=σ_z, sigma_m=σ_m, sigma_p=σ_p, mask=prior_mask,
-                               chain_offset=chain_offset, want_accept=False, kind="mala" if a == "mala" else "rwmh")
+        zt, lt = _sample(eng, a, n_chains, itr, seed, σ_z, σ_m, σ_p, prior_mask, chain_offset, hmc)
         if n_chains == 1 and not return_z:
             W = eng.project(zt[:, 0, :])                                  # map(z -> W_swa + P*z, chm)
             return [W[:, t].copy() for t in range(itr)], lt[0].copy()
@@ -206,15 +253,16 @@ def auto_encoder_subspace(model, cost, data, opt, encoder, decoder, *, T: int = 
 
 def auto_inference(m, data, decoder, W_swa, *, σ_z: float = 1.0, σ_m: float = 1.0, σ_p: float = 1.0, itr: int = 100, M: int = 3,
                    alg="hmc", backend="forwarddiff", n_chains: int = 1, seed: int = 0, chain_offset: int = 0,
-                   prior_mask: int = TERM_LL, engine: Engine | None = None, device: int = 0, return_z: bool = False):
+                   prior_mask: int = TERM_LL, engine: Engine | None = None, device: int = 0, return_z: bool = False,
+                   n_leapfrog: int = 10, step_size: float = 0.1, n_adapts: int | None = None, target_accept: float = 0.8,
+                   inv_metric=None):
     """Sampling with a decoder in place of P: density(z) evaluates the model at W_swa + decoder(z)
-    (src/space_inference.jl:238-318).  :rwmh and :mala run on the device as in sub_inference; the reference's default
-    here is :hmc, whose host-side sampler is not part of the device path (Engine.logpost_grad is its l_pi_grad)."""
+    (src/space_inference.jl:238-318).  :rwmh, :mala and :static_hmc run on the device as in sub_inference; the reference's
+    default here is :hmc (NUTS with windowed adaptation), whose host-side sampler is not part of the device path
+    (Engine.logpost_grad is its l_pi_grad)."""
     a = _sym(alg)
-    if a not in _RWMH_ALIASES and a != "mala":
-        if a in ("advi", "hmc", "nuts"):
-            raise NotImplementedError(f"{a} is not available on the device path (Engine.logpost_grad is its l_pi_grad)")
-        raise ValueError(f"{a} is not available")                         # src/space_inference.jl:316
+    _check_alg(a)
+    hmc = _hmc_options(itr, M, n_leapfrog, step_size, n_adapts, target_accept, inv_metric) if a == "static_hmc" else None
     if not isinstance(m, Chain) or not isinstance(decoder, Chain):
         raise TypeError("Error: density function is not avaliable for this model")
     if decoder.dims[0] != M:
@@ -226,8 +274,7 @@ def auto_inference(m, data, decoder, W_swa, *, σ_z: float = 1.0, σ_m: float = 
         eng.set_model(m.dims, m.acts)
         eng.set_data(X, Y)
         eng.set_decoder(W_swa, decoder.dims, decoder.acts, extract_params(decoder))
-        zt, lt, _ = eng.mh_run(n_chains, itr, seed, sigma_z=σ_z, sigma_m=σ_m, sigma_p=σ_p, mask=prior_mask,
-                               chain_offset=chain_offset, want_accept=False, kind="mala" if a == "mala" else "rwmh")
+        zt, lt = _sample(eng, a, n_chains, itr, seed, σ_z, σ_m, σ_p, prior_mask, chain_offset, hmc)
         if n_chains == 1 and not return_z:
             W = eng.project(zt[:, 0, :])                                  # map(z -> W_swa + decoder(z.params), chm)  (:277)
             return [W[:, t].copy() for t in range(itr)], lt[0].copy()

@@ -12,7 +12,7 @@ PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 LIBDIR = PKG / "lib"
 LIB = LIBDIR / "libssi.so"
-SOURCES = ["ssi_api.cu", "ssi_multi.cu", "ssi_gemm_tc.cu", "ssi_decoder.cu", "ssi_logpost.cu", "ssi_mh.cu", "ssi_construct.cu", "ssi_gram_tc.cu", "ssi_basis.cu", "ssi_basis_mma.cu", "ssi_grad.cu", "ssi_train.cu", "ssi_tc.cu"]
+SOURCES = ["ssi_api.cu", "ssi_multi.cu", "ssi_gemm_tc.cu", "ssi_decoder.cu", "ssi_logpost.cu", "ssi_mh.cu", "ssi_hmc.cu", "ssi_construct.cu", "ssi_gram_tc.cu", "ssi_basis.cu", "ssi_basis_mma.cu", "ssi_grad.cu", "ssi_train.cu", "ssi_tc.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-Wall", "-Xcompiler", "-Wno-unknown-pragmas",

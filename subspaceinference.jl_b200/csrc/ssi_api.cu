@@ -15,7 +15,7 @@ struct nvtx_range {
 #define SSI_NVTX(name) nvtx_range nvtx_range__(name)
 
 int ssi_mh_device(ssi_ctx*, int, int64_t, int64_t, uint64_t, int64_t, int64_t, double, double, double, uint32_t,
-                  const float*, float*, double*, uint8_t*);
+                  const float*, float*, double*, uint8_t*, const ssi_hmc_params_t*, const double*, double*);
 int ssi_mh_fetch_accepts(ssi_ctx*);
 int ssi_swa_push_device(ssi_ctx*, const float*, double);
 int ssi_swa_factor_device(ssi_ctx*, int, float*, double*, int*);
@@ -182,7 +182,8 @@ int ssi_ctx_destroy(ssi_ctx* ctx) {
     cudaFree(ctx->dX); cudaFree(ctx->dY); cudaFree(ctx->dP); cudaFree(ctx->dSubGram);
     cudaFree(ctx->dSwaMean); cudaFree(ctx->dDev); cudaFree(ctx->dSwaAmax);
     ssi_buf_t* bufs[] = {&ctx->bZ, &ctx->bLp, &ctx->bTerms, &ctx->bPartials, &ctx->bW, &ctx->bH0, &ctx->bH1, &ctx->bGram,
-                         &ctx->bEig, &ctx->bMisc, &ctx->bDecZ, &ctx->bDecT, &ctx->bGradW, &ctx->bGradP, &ctx->bRowsum, &ctx->bSkinny, &ctx->bGemmAmax, &ctx->bMhZ, &ctx->bMhZp, &ctx->bMhLp, &ctx->bMhLpP, &ctx->bMhCnt, &ctx->bMhG, &ctx->bSnap};
+                         &ctx->bEig, &ctx->bMisc, &ctx->bDecZ, &ctx->bDecT, &ctx->bGradW, &ctx->bGradP, &ctx->bRowsum, &ctx->bSkinny, &ctx->bGemmAmax, &ctx->bMhZ, &ctx->bMhZp, &ctx->bMhLp, &ctx->bMhLpP, &ctx->bMhCnt, &ctx->bMhG, &ctx->bSnap,
+                         &ctx->bHmcP, &ctx->bHmcH0, &ctx->bHmcEps, &ctx->bHmcDiv, &ctx->bHmcAd};
     for (ssi_buf_t* b : bufs) free_buf(*b);
     for (cudaEvent_t e : ctx->kt_events) cudaEventDestroy(e);
     cudaEventDestroy(ctx->ev0);
@@ -475,16 +476,22 @@ int ssi_logpost_batch(ssi_ctx* ctx, const float* Z, int64_t B, double sigma_m, d
     return SSI_OK;
 }
 
+static const char* mh_name(int kind, bool dev) {
+    static const char* names[2][3] = {{"ssi_mh_run", "ssi_mala_run", "ssi_hmc_run"}, {"ssi_mh_run_dev", "ssi_mala_run_dev", "ssi_hmc_run_dev"}};
+    return names[dev ? 1 : 0][kind];
+}
+
 static int mh_run_dev(ssi_ctx* ctx, int kind, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset, int64_t step_offset,
                       double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask, const float* d_z0,
-                      float* d_z_trace, double* d_lp_trace, uint8_t* d_accept_trace) {
+                      float* d_z_trace, double* d_lp_trace, uint8_t* d_accept_trace,
+                      const ssi_hmc_params_t* hp = nullptr, const double* d_adapt0 = nullptr, double* d_step_size_trace = nullptr) {
     if (!ctx) return SSI_ERR_ARG;
-    SSI_NVTX(kind == 1 ? "ssi_mala_run_dev" : "ssi_mh_run_dev");
+    SSI_NVTX(mh_name(kind, true));
     SSI_NO_MULTI(ctx, "device-pointer entry points");
     SSI_TRY(ssi_use_device(ctx));
     call_timer t(ctx);
     const int rc = ssi_mh_device(ctx, kind, n_chains, n_steps, seed, chain_offset, step_offset, sigma_z, sigma_m, sigma_p, prior_mask,
-                                 d_z0, d_z_trace, d_lp_trace, d_accept_trace);
+                                 d_z0, d_z_trace, d_lp_trace, d_accept_trace, hp, d_adapt0, d_step_size_trace);
     t.stop(false);
     return rc;
 }
@@ -507,6 +514,13 @@ int ssi_mh_run_from_dev(ssi_ctx* ctx, int32_t kind, int64_t n_chains, int64_t n_
     return mh_run_dev(ctx, kind, n_chains, n_steps, seed, chain_offset, step_offset, sigma_z, sigma_m, sigma_p, prior_mask, d_z_state,
                       d_z_trace, d_lp_trace, d_accept_trace);
 }
+int ssi_hmc_run_dev(ssi_ctx* ctx, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset, int64_t step_offset,
+                    const ssi_hmc_params_t* hp, double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask,
+                    const float* d_z_state, const double* d_adapt_state,
+                    float* d_z_trace, double* d_lp_trace, uint8_t* d_accept_trace, double* d_step_size_trace) {
+    return mh_run_dev(ctx, 2, n_chains, n_steps, seed, chain_offset, step_offset, sigma_z, sigma_m, sigma_p, prior_mask, d_z_state,
+                      d_z_trace, d_lp_trace, d_accept_trace, hp, d_adapt_state, d_step_size_trace);
+}
 
 }  // extern "C"
 
@@ -514,25 +528,35 @@ int ssi_mh_run_from_dev(ssi_ctx* ctx, int32_t kind, int64_t n_chains, int64_t n_
 // and c0 == 0 for a single-device context; a multi-device context hands every device its slice of the same host arrays).
 int ssi_mh_run_host_slice(ssi_ctx* ctx, int kind, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset, int64_t step_offset,
                           double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask, const float* z0,
-                          float* z_trace, double* lp_trace, uint8_t* accept_trace, int64_t ld_chains, int64_t c0) {
-    SSI_NVTX(kind == 1 ? "ssi_mala_run" : "ssi_mh_run");
+                          float* z_trace, double* lp_trace, uint8_t* accept_trace, int64_t ld_chains, int64_t c0,
+                          const ssi_hmc_params_t* hp, const double* adapt0, double* step_size_trace) {
+    SSI_NVTX(mh_name(kind, false));
     if (!ctx->has_model || !ctx->has_data || !ctx->has_sub)
         return ssi_fail(ctx, SSI_ERR_STATE, "model, data and subspace must be set before sampling");
     if (n_chains <= 0 || n_steps <= 0) return ssi_fail(ctx, SSI_ERR_ARG, "n_chains and n_steps must be positive");
     SSI_TRY(ssi_use_device(ctx));
     const size_t cs = (size_t)n_chains * (size_t)n_steps;
     const size_t bz = sizeof(float) * ctx->Mz * cs, bl = sizeof(double) * cs, ba = cs;
-    // one scratch allocation: [z_trace | lp_trace | acc | z0]
+    // one scratch allocation: [z_trace | lp_trace | acc | step sizes | adaptation state | z0]
     const size_t off_l = z_trace ? (bz + 255) / 256 * 256 : 0;
     const size_t off_a = off_l + (lp_trace ? (bl + 255) / 256 * 256 : 0);
-    const size_t off_z0 = off_a + (accept_trace ? (ba + 255) / 256 * 256 : 0);
+    const size_t off_e = off_a + (accept_trace ? (ba + 255) / 256 * 256 : 0);
+    const size_t off_ad = off_e + (step_size_trace ? (bl + 255) / 256 * 256 : 0);
+    const size_t bad = adapt0 ? sizeof(double) * 3 * (size_t)n_chains : 0;
+    const size_t off_z0 = off_ad + (bad + 255) / 256 * 256;
     const size_t bz0 = z0 ? sizeof(float) * (size_t)ctx->Mz * n_chains : 0;
     SSI_TRY(ssi_reserve(ctx, ctx->bSnap, off_z0 + bz0 + 256));
     char* base = (char*)ctx->bSnap.p;
     float* dzt = z_trace ? (float*)base : nullptr;
     double* dlt = lp_trace ? (double*)(base + off_l) : nullptr;
     uint8_t* dat = accept_trace ? (uint8_t*)(base + off_a) : nullptr;
+    double* det = step_size_trace ? (double*)(base + off_e) : nullptr;
+    double* dad = nullptr;
     float* dz0 = nullptr;
+    if (adapt0) {
+        dad = (double*)(base + off_ad);
+        SSI_CUDA(ctx, cudaMemcpyAsync(dad, adapt0 + 3 * (size_t)c0, bad, cudaMemcpyHostToDevice, ctx->stream));
+    }
     if (z0) {
         dz0 = (float*)(base + off_z0);
         SSI_CUDA(ctx, cudaMemcpyAsync(dz0, z0 + (size_t)c0 * ctx->Mz, bz0, cudaMemcpyHostToDevice, ctx->stream));
@@ -540,7 +564,7 @@ int ssi_mh_run_host_slice(ssi_ctx* ctx, int kind, int64_t n_chains, int64_t n_st
     for (int attempt = 0; attempt < 2; ++attempt) {      // repeated only if the tensor path's FP16 planes overflowed
         call_timer t(ctx);
         const int rc = ssi_mh_device(ctx, kind, n_chains, n_steps, seed, chain_offset, step_offset, sigma_z, sigma_m, sigma_p, prior_mask,
-                                     dz0, dzt, dlt, dat);
+                                     dz0, dzt, dlt, dat, hp, dad, det);
         t.stop(false);
         if (rc != SSI_OK) return rc;
         SSI_TRY(ssi_sync_internal(ctx));
@@ -556,6 +580,8 @@ int ssi_mh_run_host_slice(ssi_ctx* ctx, int kind, int64_t n_chains, int64_t n_st
                                                   cudaMemcpyDeviceToHost, ctx->stream));
     if (accept_trace) SSI_CUDA(ctx, cudaMemcpy2DAsync(accept_trace + c0, (size_t)ld_chains, dat, ra, ra, (size_t)n_steps,
                                                       cudaMemcpyDeviceToHost, ctx->stream));
+    if (step_size_trace) SSI_CUDA(ctx, cudaMemcpy2DAsync(step_size_trace + c0, sizeof(double) * (size_t)ld_chains, det, rl, rl, (size_t)n_steps,
+                                                         cudaMemcpyDeviceToHost, ctx->stream));
     SSI_TRY(ssi_sync_internal(ctx));
     return ssi_mh_fetch_accepts(ctx);
 }
@@ -563,13 +589,14 @@ extern "C" {
 
 static int mh_run_host(ssi_ctx* ctx, int kind, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset, int64_t step_offset,
                        double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask, const float* z0,
-                       float* z_trace, double* lp_trace, uint8_t* accept_trace) {
+                       float* z_trace, double* lp_trace, uint8_t* accept_trace,
+                       const ssi_hmc_params_t* hp = nullptr, const double* adapt0 = nullptr, double* step_size_trace = nullptr) {
     if (!ctx) return SSI_ERR_ARG;
     if (ctx->is_multi())
         return ssi_multi_mh_run(ctx, kind, n_chains, n_steps, seed, chain_offset, step_offset, sigma_z, sigma_m, sigma_p, prior_mask, z0,
-                                z_trace, lp_trace, accept_trace);
+                                z_trace, lp_trace, accept_trace, hp, adapt0, step_size_trace);
     return ssi_mh_run_host_slice(ctx, kind, n_chains, n_steps, seed, chain_offset, step_offset, sigma_z, sigma_m, sigma_p, prior_mask, z0,
-                                 z_trace, lp_trace, accept_trace, n_chains, 0);
+                                 z_trace, lp_trace, accept_trace, n_chains, 0, hp, adapt0, step_size_trace);
 }
 int ssi_mh_run(ssi_ctx* ctx, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset,
                double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask, const float* z0,
@@ -591,6 +618,19 @@ int ssi_mh_run_from(ssi_ctx* ctx, int32_t kind, int64_t n_chains, int64_t n_step
     return mh_run_host(ctx, kind, n_chains, n_steps, seed, chain_offset, step_offset, sigma_z, sigma_m, sigma_p, prior_mask, z_state,
                        z_trace, lp_trace, accept_trace);
 }
+int ssi_hmc_run(ssi_ctx* ctx, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset, int64_t step_offset,
+                const ssi_hmc_params_t* hp, double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask,
+                const float* z_state, const double* adapt_state,
+                float* z_trace, double* lp_trace, uint8_t* accept_trace, double* step_size_trace) {
+    if (!ctx) return SSI_ERR_ARG;
+    // checked here as well as per device, so that a multi-device context reports the argument, not a device
+    SSI_TRY(ssi_hmc_check(ctx, hp, ctx->Mz));
+    if (step_offset > 0 && !z_state) return ssi_fail(ctx, SSI_ERR_ARG, "a continued run (step_offset > 0) needs the chain state z");
+    if (step_offset > 0 && hp->n_adapts > 0 && !adapt_state)
+        return ssi_fail(ctx, SSI_ERR_ARG, "a continued HMC run with n_adapts > 0 needs the adaptation state (ssi_hmc_get_adapt)");
+    return mh_run_host(ctx, 2, n_chains, n_steps, seed, chain_offset, step_offset, sigma_z, sigma_m, sigma_p, prior_mask, z_state,
+                       z_trace, lp_trace, accept_trace, hp, adapt_state, step_size_trace);
+}
 
 }  // extern "C"
 
@@ -603,12 +643,28 @@ int ssi_mh_get_state_slice(ssi_ctx* ctx, float* z_out, double* lp_out) {
     SSI_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return SSI_OK;
 }
+// dual-averaging state (3 x n_chains) of the last HMC run's chains on this device
+int ssi_hmc_get_adapt_slice(ssi_ctx* ctx, double* adapt_out) {
+    if (ctx->mh_chains <= 0 || ctx->mh_kind != 2) return ssi_fail(ctx, SSI_ERR_STATE, "the last run on this context was not HMC");
+    SSI_TRY(ssi_use_device(ctx));
+    SSI_CUDA(ctx, cudaMemcpyAsync(adapt_out, ctx->bHmcAd.p, sizeof(double) * 3 * (size_t)ctx->mh_chains, cudaMemcpyDeviceToHost, ctx->stream));
+    SSI_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return SSI_OK;
+}
 extern "C" {
 
 int ssi_mh_get_state(ssi_ctx* ctx, float* z_out, double* lp_out) {
     if (!ctx) return SSI_ERR_ARG;
     if (ctx->is_multi()) return ssi_multi_mh_get_state(ctx, z_out, lp_out);
     return ssi_mh_get_state_slice(ctx, z_out, lp_out);
+}
+
+int ssi_hmc_get_adapt(ssi_ctx* ctx, double* adapt_out) {
+    if (!ctx) return SSI_ERR_ARG;
+    if (!adapt_out) return ssi_fail(ctx, SSI_ERR_ARG, "adapt_out is NULL");
+    if (ctx->mh_chains <= 0 || ctx->mh_kind != 2) return ssi_fail(ctx, SSI_ERR_STATE, "the last run on this context was not HMC");
+    if (ctx->is_multi()) return ssi_multi_hmc_get_adapt(ctx, adapt_out);
+    return ssi_hmc_get_adapt_slice(ctx, adapt_out);
 }
 
 int ssi_rng_replay(uint64_t seed, int64_t chain, int64_t step, int32_t M, float* eps_out, double* e_out) {

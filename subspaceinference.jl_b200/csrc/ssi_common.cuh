@@ -97,6 +97,10 @@ struct ssi_ctx {
     // MH state
     ssi_buf_t bMhZ, bMhZp, bMhLp, bMhLpP, bMhCnt, bMhG;
     int64_t mh_chains = 0;       // chains of the last run (ssi_mh_get_state)
+    int mh_kind = -1;            // sampler of the last run: 0 RWMH, 1 MALA, 2 HMC (ssi_hmc_get_adapt needs 2)
+    // HMC integrator (ssi_hmc.cu): momentum (M x C), start energy, step size of the transition, divergence flag (C each),
+    // dual-averaging state (3 x C: log eps, log eps_bar, H_bar)
+    ssi_buf_t bHmcP, bHmcH0, bHmcEps, bHmcDiv, bHmcAd;
 
     // SWA / construction state
     int64_t swa_n = 0, swa_Kmax = 0, swa_K = 0;
@@ -181,15 +185,27 @@ int ssi_multi_logpost(ssi_ctx* ctx, int grad, const float* Z, int64_t B, double 
                       double* lp_out, double* second_out);
 int ssi_multi_mh_run(ssi_ctx* ctx, int kind, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset, int64_t step_offset,
                      double sigma_z, double sigma_m, double sigma_p, uint32_t mask, const float* z0,
-                     float* z_trace, double* lp_trace, uint8_t* accept_trace);
+                     float* z_trace, double* lp_trace, uint8_t* accept_trace,
+                     const ssi_hmc_params_t* hp, const double* adapt0, double* step_size_trace);
 int ssi_multi_mh_get_state(ssi_ctx* ctx, float* z_out, double* lp_out);
+int ssi_multi_hmc_get_adapt(ssi_ctx* ctx, double* adapt_out);
 int ssi_multi_project(ssi_ctx* ctx, const float* Z, int64_t B, float* W_out);
 int ssi_multi_swa_finish(ssi_ctx* ctx, int32_t M, float* W_swa_out, float* P_out, double* s_out, int32_t install);
 // per-device halves of the host-pointer MH entry points (ssi_api.cu)
+// (kind 2, HMC: hp, the adaptation state adapt0 (3 x n_chains, or NULL) and the step-size trace; NULL for kinds 0 and 1)
 int ssi_mh_run_host_slice(ssi_ctx* ctx, int kind, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset, int64_t step_offset,
                           double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask, const float* z0,
-                          float* z_trace, double* lp_trace, uint8_t* accept_trace, int64_t ld_chains, int64_t c0);
+                          float* z_trace, double* lp_trace, uint8_t* accept_trace, int64_t ld_chains, int64_t c0,
+                          const ssi_hmc_params_t* hp, const double* adapt0, double* step_size_trace);
 int ssi_mh_get_state_slice(ssi_ctx* ctx, float* z_out, double* lp_out);
+int ssi_hmc_get_adapt_slice(ssi_ctx* ctx, double* adapt_out);
+
+// ---- HMC integrator (ssi_hmc.cu) -----------------------------------------------------------
+int ssi_hmc_check(ssi_ctx* ctx, const ssi_hmc_params_t* hp, int M);
+int ssi_hmc_prepare(ssi_ctx* ctx, int64_t C, const ssi_hmc_params_t* hp, const double* d_adapt0);
+int ssi_hmc_transition(ssi_ctx* ctx, int64_t C, uint64_t seed, int64_t chain_off, int64_t t, const ssi_hmc_params_t* hp,
+                       double sigma_z, double sigma_m, double sigma_p, uint32_t mask, float* d_ztr, double* d_lptr,
+                       uint8_t* d_acctr, double* d_etr, double* units, double* flops);
 
 // ---- decoder (ssi_decoder.cu) -------------------------------------------------------------
 void ssi_dec_destroy(ssi_ctx* ctx);

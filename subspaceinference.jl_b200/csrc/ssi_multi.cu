@@ -176,17 +176,19 @@ int ssi_multi_logpost(ssi_ctx* ctx, int grad, const float* Z, int64_t B, double 
 // of each step's row of the host traces
 int ssi_multi_mh_run(ssi_ctx* ctx, int kind, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset, int64_t step_offset,
                      double sigma_z, double sigma_m, double sigma_p, uint32_t mask, const float* z0,
-                     float* z_trace, double* lp_trace, uint8_t* accept_trace) {
+                     float* z_trace, double* lp_trace, uint8_t* accept_trace,
+                     const ssi_hmc_params_t* hp, const double* adapt0, double* step_size_trace) {
     if (n_chains <= 0 || n_steps <= 0) return ssi_fail(ctx, SSI_ERR_ARG, "n_chains and n_steps must be positive");
     const int n_dev = (int)ctx->children.size();
     ctx->mh_chains = n_chains;
+    ctx->mh_kind = kind;
     return for_each_device(ctx, [&](ssi_ctx* c, int d) {
         int64_t c0, c1;
         shard_range(n_chains, n_dev, d, c0, c1);
         c->mh_chains = 0;
         if (c1 <= c0) return (int)SSI_OK;
         return ssi_mh_run_host_slice(c, kind, c1 - c0, n_steps, seed, chain_offset + c0, step_offset, sigma_z, sigma_m, sigma_p, mask, z0,
-                                     z_trace, lp_trace, accept_trace, n_chains, c0);
+                                     z_trace, lp_trace, accept_trace, n_chains, c0, hp, adapt0, step_size_trace);
     });
 }
 
@@ -200,6 +202,17 @@ int ssi_multi_mh_get_state(ssi_ctx* ctx, float* z_out, double* lp_out) {
         shard_range(C, n_dev, d, c0, c1);
         if (c1 <= c0) return (int)SSI_OK;
         return ssi_mh_get_state_slice(c, z_out ? z_out + (size_t)c0 * M : nullptr, lp_out ? lp_out + c0 : nullptr);
+    });
+}
+
+int ssi_multi_hmc_get_adapt(ssi_ctx* ctx, double* adapt_out) {
+    const int n_dev = (int)ctx->children.size();
+    const int64_t C = ctx->mh_chains;
+    return for_each_device(ctx, [&](ssi_ctx* c, int d) {
+        int64_t c0, c1;
+        shard_range(C, n_dev, d, c0, c1);
+        if (c1 <= c0) return (int)SSI_OK;
+        return ssi_hmc_get_adapt_slice(c, adapt_out + 3 * (size_t)c0);
     });
 }
 

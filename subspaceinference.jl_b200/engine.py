@@ -230,6 +230,62 @@ class Engine:
                                              C.c_void_p(d_z0 or None), C.c_void_p(d_z_trace or None),
                                              C.c_void_p(d_lp_trace or None), C.c_void_p(d_accept or None)))
 
+    # ---- fixed-length HMC with per-chain dual averaging (alg = :static_hmc) -------------------------------------
+    def _hmc_params(self, step_size, n_leapfrog, n_adapts, target_accept, inv_metric):
+        minv = None
+        if inv_metric is not None:
+            minv = np.ascontiguousarray(np.asarray(inv_metric, dtype=np.float64).reshape(-1))
+            if minv.shape[0] != self.M:
+                raise ValueError(f"inv_metric must have M={self.M} entries")
+        hp = _lib.HmcParams(float(step_size), int(n_leapfrog), int(n_adapts), float(target_accept), _ptr(minv).value)
+        return hp, minv                      # minv must outlive the call that reads hp
+
+    def hmc_run(self, n_chains: int, n_steps: int, seed: int, step_size: float, n_leapfrog: int, n_adapts: int = 0,
+                target_accept: float = 0.8, inv_metric=None, sigma_z=1.0, sigma_m=1.0, sigma_p=1.0, mask=TERM_LL,
+                chain_offset: int = 0, z0=None, step_offset: int = 0, adapt_state=None,
+                want_z=True, want_lp=True, want_accept=True, want_step_size=True):
+        """Fixed-length HMC (ssi_hmc_run): n_leapfrog leapfrog steps per transition, diagonal inverse metric inv_metric
+        (M values, default ones), step size adapted per chain by dual averaging over transitions 1..n_adapts.
+        Returns (z_trace (M, n_chains, n_steps) f32, lp_trace (n_chains, n_steps) f64, accept (n_chains, n_steps) u8 with
+        1 accepted / 0 rejected / 2 divergent, step_size_trace (n_chains, n_steps) f64, NaN at step 0); entries not
+        requested are None.  step_offset > 0 continues chains from z0 = mh_state()[0] and adapt_state = hmc_adapt()."""
+        zt = np.empty((self.M, n_chains, n_steps), np.float32, order="F") if want_z else None
+        lt = np.empty((n_chains, n_steps), np.float64, order="F") if want_lp else None
+        at = np.empty((n_chains, n_steps), np.uint8, order="F") if want_accept else None
+        et = np.empty((n_chains, n_steps), np.float64, order="F") if want_step_size else None
+        z0a = _f32(z0) if z0 is not None else None
+        if z0a is not None and z0a.shape != (self.M, n_chains):
+            raise ValueError("z0 must be (M, n_chains)")
+        ada = None
+        if adapt_state is not None:
+            ada = np.require(np.asarray(adapt_state, dtype=np.float64), requirements=["ALIGNED", "F_CONTIGUOUS"])
+            if ada.shape != (3, n_chains):
+                raise ValueError("adapt_state must be (3, n_chains)")
+        hp, _minv = self._hmc_params(step_size, n_leapfrog, n_adapts, target_accept, inv_metric)
+        self._check(self._lib.ssi_hmc_run(self._h, n_chains, n_steps, seed, chain_offset, step_offset, C.byref(hp),
+                                          sigma_z, sigma_m, sigma_p, mask, _ptr(z0a), _ptr(ada), _ptr(zt), _ptr(lt), _ptr(at), _ptr(et)))
+        self._last_chains = n_chains
+        return zt, lt, at, et
+
+    def hmc_run_dev(self, n_chains: int, n_steps: int, seed: int, step_size: float, n_leapfrog: int, n_adapts: int = 0,
+                    target_accept: float = 0.8, inv_metric=None, sigma_z=1.0, sigma_m=1.0, sigma_p=1.0, mask=TERM_LL,
+                    chain_offset: int = 0, step_offset: int = 0, d_z0: int | None = None, d_adapt: int | None = None,
+                    d_z_trace: int | None = None, d_lp_trace: int | None = None, d_accept: int | None = None,
+                    d_step_size: int | None = None):
+        """Device-pointer variant of hmc_run (asynchronous on the context stream)."""
+        hp, _minv = self._hmc_params(step_size, n_leapfrog, n_adapts, target_accept, inv_metric)
+        self._check(self._lib.ssi_hmc_run_dev(self._h, n_chains, n_steps, seed, chain_offset, step_offset, C.byref(hp),
+                                              sigma_z, sigma_m, sigma_p, mask, C.c_void_p(d_z0 or None), C.c_void_p(d_adapt or None),
+                                              C.c_void_p(d_z_trace or None), C.c_void_p(d_lp_trace or None),
+                                              C.c_void_p(d_accept or None), C.c_void_p(d_step_size or None)))
+        self._last_chains = n_chains
+
+    def hmc_adapt(self) -> np.ndarray:
+        """(3, n_chains) f64: log eps, log eps_bar, H_bar of every chain of the last HMC run (what hmc_run's adapt_state takes)."""
+        a = np.empty((3, self._last_chains), np.float64, order="F")
+        self._check(self._lib.ssi_hmc_get_adapt(self._h, _ptr(a)))
+        return a
+
     def rng_replay(self, seed: int, chain: int, step: int, M: int | None = None):
         M = self.M if M is None else M
         eps = np.empty(M, np.float32)

@@ -77,6 +77,41 @@ function logpost_batch(ctx::Ctx, Z::AbstractMatrix; σ_m = 1.0, σ_p = 1.0, σ_z
     return lp
 end
 
+# ssi_hmc_params_t (include/ssi.h): passed by reference, inv_metric a host pointer (C_NULL = identity)
+struct HmcParams
+    step_size::Float64
+    n_leapfrog::Int32
+    n_adapts::Int64
+    target_accept::Float64
+    inv_metric::Ptr{Float64}
+end
+
+# alg = :static_hmc: fixed-length HMC (AdvancedHMC's StaticTrajectory, Turing's HMC(ε, n_leapfrog)) with per-chain dual averaging
+# of ε over the first n_adapts transitions; the warm-up samples stay in the trace.  Not :hmc, which in the reference is NUTS with
+# Stan's windowed adaptation and stays host-side.
+function check_hmc(M, n_leapfrog, step_size, n_adapts, target_accept, inv_metric)
+    n_leapfrog >= 1 || throw(ArgumentError("n_leapfrog must be >= 1"))
+    (isfinite(step_size) && step_size > 0) || throw(ArgumentError("step_size must be positive and finite"))
+    n_adapts >= 0 || throw(ArgumentError("n_adapts must be >= 0"))
+    0 < target_accept < 1 || throw(ArgumentError("target_accept must be in (0, 1)"))
+    inv_metric === nothing || (length(inv_metric) == M && all(x -> isfinite(x) && x > 0, inv_metric)) ||
+        throw(ArgumentError("inv_metric must hold M positive finite values"))
+end
+
+function run_static_hmc(ctx::Ctx, M, n_chains, itr, seed, σ_z, σ_m, σ_p, prior_mask, n_leapfrog, step_size, n_adapts,
+                        target_accept, inv_metric)
+    zt = Array{Float32}(undef, M, n_chains, itr); lp = Matrix{Float64}(undef, n_chains, itr)
+    minv = inv_metric === nothing ? nothing : Vector{Float64}(inv_metric)
+    GC.@preserve minv begin
+        hp = Ref(HmcParams(step_size, n_leapfrog, n_adapts, target_accept, minv === nothing ? C_NULL : pointer(minv)))
+        check(ctx, ccall((:ssi_hmc_run, libssi), Cint,
+                         (Ptr{Cvoid}, Int64, Int64, UInt64, Int64, Int64, Ref{HmcParams}, Float64, Float64, Float64, UInt32,
+                          Ptr{Float32}, Ptr{Float64}, Ptr{Float32}, Ptr{Float64}, Ptr{UInt8}, Ptr{Float64}),
+                         ctx.h, n_chains, itr, seed, 0, 0, hp, σ_z, σ_m, σ_p, prior_mask, C_NULL, C_NULL, zt, lp, C_NULL, C_NULL))
+    end
+    return zt, lp
+end
+
 # ---- public API ---------------------------------------------------------------------------------
 # l_pi_grad(theta) = (density(theta), gradient(density, theta))  (src/space_inference.jl:107), batched over the columns of Z:
 # what AdvancedHMC's Hamiltonian(metric, density, l_pi_grad) (:146) needs, one reverse pass instead of ForwardDiff's M forward passes.
@@ -146,17 +181,24 @@ end
 
 function sub_inference(in_model, data, W_swa, P; σ_z = 1.0, σ_m = 1.0, σ_p = 1.0, itr = 100, M = 3,
                        alg = :rwmh, backend = :forwarddiff,
-                       n_chains = 1, seed = rand(UInt64), prior_mask = TERM_LL, ctx::Ctx = Ctx())
-    # :rwmh / :mh (:113-116) and :mala (:117-120) run on the device; :hmc / :nuts / :advi stay in the reference and can take
-    # logpost_grad below as their l_pi_grad (:107)
-    (alg == :rwmh || alg == :mh || alg == :mala) || throw("$alg is not available")            # :162
+                       n_chains = 1, seed = rand(UInt64), prior_mask = TERM_LL, ctx::Ctx = Ctx(),
+                       n_leapfrog = 10, step_size = 0.1, n_adapts = div(itr, 2), target_accept = 0.8, inv_metric = nothing)
+    # :rwmh / :mh (:113-116), :mala (:117-120) and :static_hmc run on the device; :hmc / :nuts / :advi stay in the reference and
+    # can take logpost_grad below as their l_pi_grad (:107)
+    (alg == :rwmh || alg == :mh || alg == :mala || alg == :static_hmc) || throw("$alg is not available")            # :162
+    alg == :static_hmc && check_hmc(M, n_leapfrog, step_size, n_adapts, target_accept, inv_metric)
     size(P, 2) == M || throw(DimensionMismatch("P has $(size(P, 2)) columns but M = $M"))
     set_problem!(ctx, in_model, data, W_swa, P)
-    zt = Array{Float32}(undef, M, n_chains, itr); lp = Matrix{Float64}(undef, n_chains, itr)
-    check(ctx, ccall((alg == :mala ? :ssi_mala_run : :ssi_mh_run, libssi), Cint,
-                     (Ptr{Cvoid}, Int64, Int64, UInt64, Int64, Float64, Float64, Float64, UInt32,
-                      Ptr{Float32}, Ptr{Float32}, Ptr{Float64}, Ptr{UInt8}),
-                     ctx.h, n_chains, itr, seed, 0, σ_z, σ_m, σ_p, prior_mask, C_NULL, zt, lp, C_NULL))
+    if alg == :static_hmc
+        zt, lp = run_static_hmc(ctx, M, n_chains, itr, seed, σ_z, σ_m, σ_p, prior_mask, n_leapfrog, step_size, n_adapts,
+                                target_accept, inv_metric)
+    else
+        zt = Array{Float32}(undef, M, n_chains, itr); lp = Matrix{Float64}(undef, n_chains, itr)
+        check(ctx, ccall((alg == :mala ? :ssi_mala_run : :ssi_mh_run, libssi), Cint,
+                         (Ptr{Cvoid}, Int64, Int64, UInt64, Int64, Float64, Float64, Float64, UInt32,
+                          Ptr{Float32}, Ptr{Float32}, Ptr{Float64}, Ptr{UInt8}),
+                         ctx.h, n_chains, itr, seed, 0, σ_z, σ_m, σ_p, prior_mask, C_NULL, zt, lp, C_NULL))
+    end
     if n_chains == 1
         # map(z -> W_swa + P*z.params, chm), map(z -> z.lp, chm)   (:125)
         Wout = Matrix{Float32}(undef, length(W_swa), itr)
@@ -219,8 +261,11 @@ function auto_encoder_subspace(model, cost, data, opt, encoder, decoder; T = 10,
 end
 
 function auto_inference(m, data, decoder, W_swa; σ_z = 1.0, σ_m = 1.0, σ_p = 1.0, itr = 100, M = 3, alg = :hmc,
-                        backend = :forwarddiff, n_chains = 1, seed = rand(UInt64), prior_mask = TERM_LL, ctx::Ctx = Ctx())
-    (alg == :rwmh || alg == :mh || alg == :mala) || throw("$alg is not available")            # :316; :hmc/:nuts/:advi stay host-side
+                        backend = :forwarddiff, n_chains = 1, seed = rand(UInt64), prior_mask = TERM_LL, ctx::Ctx = Ctx(),
+                        n_leapfrog = 10, step_size = 0.1, n_adapts = div(itr, 2), target_accept = 0.8, inv_metric = nothing)
+    # :316; :hmc/:nuts/:advi stay host-side
+    (alg == :rwmh || alg == :mh || alg == :mala || alg == :static_hmc) || throw("$alg is not available")
+    alg == :static_hmc && check_hmc(M, n_leapfrog, step_size, n_adapts, target_accept, inv_metric)
     dims, acts = describe(m)
     check(ctx, ccall((:ssi_set_model, libssi), Cint, (Ptr{Cvoid}, Cint, Ptr{Int32}, Ptr{Int32}), ctx.h, length(acts), dims, acts))
     X = Matrix{Float32}(data.data[1]); Y = Matrix{Float32}(data.data[2])
@@ -228,11 +273,16 @@ function auto_inference(m, data, decoder, W_swa; σ_z = 1.0, σ_m = 1.0, σ_p = 
     ddims, dacts = describe(decoder)
     check(ctx, ccall((:ssi_set_decoder, libssi), Cint, (Ptr{Cvoid}, Ptr{Float32}, Int32, Ptr{Int32}, Ptr{Int32}, Ptr{Float32}),
                      ctx.h, Float32.(W_swa), length(dacts), ddims, dacts, flat_params(decoder)))
-    zt = Array{Float32}(undef, M, n_chains, itr); lp = Matrix{Float64}(undef, n_chains, itr)
-    check(ctx, ccall((alg == :mala ? :ssi_mala_run : :ssi_mh_run, libssi), Cint,
-                     (Ptr{Cvoid}, Int64, Int64, UInt64, Int64, Float64, Float64, Float64, UInt32,
-                      Ptr{Float32}, Ptr{Float32}, Ptr{Float64}, Ptr{UInt8}),
-                     ctx.h, n_chains, itr, seed, 0, σ_z, σ_m, σ_p, prior_mask, C_NULL, zt, lp, C_NULL))
+    if alg == :static_hmc
+        zt, lp = run_static_hmc(ctx, M, n_chains, itr, seed, σ_z, σ_m, σ_p, prior_mask, n_leapfrog, step_size, n_adapts,
+                                target_accept, inv_metric)
+    else
+        zt = Array{Float32}(undef, M, n_chains, itr); lp = Matrix{Float64}(undef, n_chains, itr)
+        check(ctx, ccall((alg == :mala ? :ssi_mala_run : :ssi_mh_run, libssi), Cint,
+                         (Ptr{Cvoid}, Int64, Int64, UInt64, Int64, Float64, Float64, Float64, UInt32,
+                          Ptr{Float32}, Ptr{Float32}, Ptr{Float64}, Ptr{UInt8}),
+                         ctx.h, n_chains, itr, seed, 0, σ_z, σ_m, σ_p, prior_mask, C_NULL, zt, lp, C_NULL))
+    end
     n_chains == 1 || return zt, lp
     Wout = Matrix{Float32}(undef, length(W_swa), itr)          # map(z -> W_swa + decoder(z.params), chm)  (:277)
     check(ctx, ccall((:ssi_project, libssi), Cint, (Ptr{Cvoid}, Ptr{Float32}, Int64, Ptr{Float32}), ctx.h, Matrix{Float32}(zt[:, 1, :]), itr, Wout))
