@@ -23,9 +23,10 @@
  *   - a context is not re-entrant.  ssi_ctx_create binds it to ONE device; ssi_ctx_create_multi returns a context that
  *     drives several devices from the one calling process (the reference is a single Julia process,
  *     src/space_inference.jl:82-84): set_* calls are replicated, the batched host-pointer calls shard samples / chains
- *     across the devices and every device lands its slice in the caller's host arrays.  Alternatively one process (and
- *     one context) per GPU shards chains by `chain_offset`.  Either way the counter-based RNG is keyed on the GLOBAL
- *     chain id, so results do not depend on the number of GPUs.
+ *     across the devices and every device lands its slice in the caller's host arrays.  A sampler run's arguments are
+ *     checked before it is sharded, so a rejected run fails as on one device and leaves the last run's state readable.
+ *     Alternatively one process (and one context) per GPU shards chains by `chain_offset`.  Either way the counter-based
+ *     RNG is keyed on the GLOBAL chain id, so results do not depend on the number of GPUs.
  *   - distinct contexts are independent (no shared mutable state), also on the same device.
  *   - there is no CPU fallback: every compute entry point fails with SSI_ERR_CUDA when
  *     no sm_100 device is usable.

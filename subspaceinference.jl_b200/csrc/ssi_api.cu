@@ -14,8 +14,6 @@ struct nvtx_range {
 };
 #define SSI_NVTX(name) nvtx_range nvtx_range__(name)
 
-int ssi_mh_device(ssi_ctx*, int, int64_t, int64_t, uint64_t, int64_t, int64_t, double, double, double, uint32_t,
-                  const float*, float*, double*, uint8_t*, const ssi_hmc_params_t*, const double*, double*);
 int ssi_mh_fetch_accepts(ssi_ctx*);
 int ssi_swa_push_device(ssi_ctx*, const float*, double);
 int ssi_swa_factor_device(ssi_ctx*, int, float*, double*, int*);
@@ -481,90 +479,46 @@ static const char* mh_name(int kind, bool dev) {
     return names[dev ? 1 : 0][kind];
 }
 
-static int mh_run_dev(ssi_ctx* ctx, int kind, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset, int64_t step_offset,
-                      double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask, const float* d_z0,
-                      float* d_z_trace, double* d_lp_trace, uint8_t* d_accept_trace,
-                      const ssi_hmc_params_t* hp = nullptr, const double* d_adapt0 = nullptr, double* d_step_size_trace = nullptr) {
-    if (!ctx) return SSI_ERR_ARG;
-    SSI_NVTX(mh_name(kind, true));
-    SSI_NO_MULTI(ctx, "device-pointer entry points");
-    SSI_TRY(ssi_use_device(ctx));
-    call_timer t(ctx);
-    const int rc = ssi_mh_device(ctx, kind, n_chains, n_steps, seed, chain_offset, step_offset, sigma_z, sigma_m, sigma_p, prior_mask,
-                                 d_z0, d_z_trace, d_lp_trace, d_accept_trace, hp, d_adapt0, d_step_size_trace);
-    t.stop(false);
-    return rc;
-}
-int ssi_mh_run_dev(ssi_ctx* ctx, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset,
-                   double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask, const float* d_z0,
-                   float* d_z_trace, double* d_lp_trace, uint8_t* d_accept_trace) {
-    return mh_run_dev(ctx, 0, n_chains, n_steps, seed, chain_offset, 0, sigma_z, sigma_m, sigma_p, prior_mask, d_z0, d_z_trace,
-                      d_lp_trace, d_accept_trace);
-}
-int ssi_mala_run_dev(ssi_ctx* ctx, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset,
-                     double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask, const float* d_z0,
-                     float* d_z_trace, double* d_lp_trace, uint8_t* d_accept_trace) {
-    return mh_run_dev(ctx, 1, n_chains, n_steps, seed, chain_offset, 0, sigma_z, sigma_m, sigma_p, prior_mask, d_z0, d_z_trace,
-                      d_lp_trace, d_accept_trace);
-}
-int ssi_mh_run_from_dev(ssi_ctx* ctx, int32_t kind, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset,
-                        int64_t step_offset, double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask,
-                        const float* d_z_state, float* d_z_trace, double* d_lp_trace, uint8_t* d_accept_trace) {
-    if (ctx && kind != 0 && kind != 1) return ssi_fail(ctx, SSI_ERR_ARG, "kind must be 0 (RWMH) or 1 (MALA)");
-    return mh_run_dev(ctx, kind, n_chains, n_steps, seed, chain_offset, step_offset, sigma_z, sigma_m, sigma_p, prior_mask, d_z_state,
-                      d_z_trace, d_lp_trace, d_accept_trace);
-}
-int ssi_hmc_run_dev(ssi_ctx* ctx, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset, int64_t step_offset,
-                    const ssi_hmc_params_t* hp, double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask,
-                    const float* d_z_state, const double* d_adapt_state,
-                    float* d_z_trace, double* d_lp_trace, uint8_t* d_accept_trace, double* d_step_size_trace) {
-    return mh_run_dev(ctx, 2, n_chains, n_steps, seed, chain_offset, step_offset, sigma_z, sigma_m, sigma_p, prior_mask, d_z_state,
-                      d_z_trace, d_lp_trace, d_accept_trace, hp, d_adapt_state, d_step_size_trace);
-}
-
 }  // extern "C"
 
-// Host-pointer run of the chains [c0, c0 + n_chains) of a trace that holds ld_chains chains per step (ld_chains == n_chains
-// and c0 == 0 for a single-device context; a multi-device context hands every device its slice of the same host arrays).
-int ssi_mh_run_host_slice(ssi_ctx* ctx, int kind, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset, int64_t step_offset,
-                          double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask, const float* z0,
-                          float* z_trace, double* lp_trace, uint8_t* accept_trace, int64_t ld_chains, int64_t c0,
-                          const ssi_hmc_params_t* hp, const double* adapt0, double* step_size_trace) {
-    SSI_NVTX(mh_name(kind, false));
-    if (!ctx->has_model || !ctx->has_data || !ctx->has_sub)
-        return ssi_fail(ctx, SSI_ERR_STATE, "model, data and subspace must be set before sampling");
-    if (n_chains <= 0 || n_steps <= 0) return ssi_fail(ctx, SSI_ERR_ARG, "n_chains and n_steps must be positive");
+// Host-pointer run of the chains [c0, c1) of `run` on this device (c0 == 0 and c1 == run.n_chains for a single-device
+// context; a multi-device context hands every device its slice of the same host arrays).
+int ssi_mh_run_host_slice(ssi_ctx* ctx, const ssi_mh_run_t& run, int64_t c0, int64_t c1) {
+    SSI_NVTX(mh_name(run.kind, false));
     SSI_TRY(ssi_use_device(ctx));
-    const size_t cs = (size_t)n_chains * (size_t)n_steps;
-    const size_t bz = sizeof(float) * ctx->Mz * cs, bl = sizeof(double) * cs, ba = cs;
+    ssi_mh_run_t r = run;          // this device's shard, its pointers into bSnap
+    r.n_chains = c1 - c0;
+    r.chain_offset = run.chain_offset + c0;
+    const int M = ctx->Mz;
+    const size_t cs = (size_t)r.n_chains * (size_t)r.n_steps;
+    const size_t bz = sizeof(float) * M * cs, bl = sizeof(double) * cs, ba = cs;
     // one scratch allocation: [z_trace | lp_trace | acc | step sizes | adaptation state | z0]
-    const size_t off_l = z_trace ? (bz + 255) / 256 * 256 : 0;
-    const size_t off_a = off_l + (lp_trace ? (bl + 255) / 256 * 256 : 0);
-    const size_t off_e = off_a + (accept_trace ? (ba + 255) / 256 * 256 : 0);
-    const size_t off_ad = off_e + (step_size_trace ? (bl + 255) / 256 * 256 : 0);
-    const size_t bad = adapt0 ? sizeof(double) * 3 * (size_t)n_chains : 0;
+    const size_t off_l = run.z_trace ? (bz + 255) / 256 * 256 : 0;
+    const size_t off_a = off_l + (run.lp_trace ? (bl + 255) / 256 * 256 : 0);
+    const size_t off_e = off_a + (run.accept_trace ? (ba + 255) / 256 * 256 : 0);
+    const size_t off_ad = off_e + (run.step_size_trace ? (bl + 255) / 256 * 256 : 0);
+    const size_t bad = run.adapt0 ? sizeof(double) * 3 * (size_t)r.n_chains : 0;
     const size_t off_z0 = off_ad + (bad + 255) / 256 * 256;
-    const size_t bz0 = z0 ? sizeof(float) * (size_t)ctx->Mz * n_chains : 0;
+    const size_t bz0 = run.z0 ? sizeof(float) * (size_t)M * r.n_chains : 0;
     SSI_TRY(ssi_reserve(ctx, ctx->bSnap, off_z0 + bz0 + 256));
     char* base = (char*)ctx->bSnap.p;
-    float* dzt = z_trace ? (float*)base : nullptr;
-    double* dlt = lp_trace ? (double*)(base + off_l) : nullptr;
-    uint8_t* dat = accept_trace ? (uint8_t*)(base + off_a) : nullptr;
-    double* det = step_size_trace ? (double*)(base + off_e) : nullptr;
-    double* dad = nullptr;
-    float* dz0 = nullptr;
-    if (adapt0) {
-        dad = (double*)(base + off_ad);
-        SSI_CUDA(ctx, cudaMemcpyAsync(dad, adapt0 + 3 * (size_t)c0, bad, cudaMemcpyHostToDevice, ctx->stream));
+    r.z_trace = run.z_trace ? (float*)base : nullptr;
+    r.lp_trace = run.lp_trace ? (double*)(base + off_l) : nullptr;
+    r.accept_trace = run.accept_trace ? (uint8_t*)(base + off_a) : nullptr;
+    r.step_size_trace = run.step_size_trace ? (double*)(base + off_e) : nullptr;
+    if (run.adapt0) {
+        double* dad = (double*)(base + off_ad);
+        SSI_CUDA(ctx, cudaMemcpyAsync(dad, run.adapt0 + 3 * (size_t)c0, bad, cudaMemcpyHostToDevice, ctx->stream));
+        r.adapt0 = dad;
     }
-    if (z0) {
-        dz0 = (float*)(base + off_z0);
-        SSI_CUDA(ctx, cudaMemcpyAsync(dz0, z0 + (size_t)c0 * ctx->Mz, bz0, cudaMemcpyHostToDevice, ctx->stream));
+    if (run.z0) {
+        float* dz0 = (float*)(base + off_z0);
+        SSI_CUDA(ctx, cudaMemcpyAsync(dz0, run.z0 + (size_t)c0 * M, bz0, cudaMemcpyHostToDevice, ctx->stream));
+        r.z0 = dz0;
     }
     for (int attempt = 0; attempt < 2; ++attempt) {      // repeated only if the tensor path's FP16 planes overflowed
         call_timer t(ctx);
-        const int rc = ssi_mh_device(ctx, kind, n_chains, n_steps, seed, chain_offset, step_offset, sigma_z, sigma_m, sigma_p, prior_mask,
-                                     dz0, dzt, dlt, dat, hp, dad, det);
+        const int rc = ssi_mh_device(ctx, r);
         t.stop(false);
         if (rc != SSI_OK) return rc;
         SSI_TRY(ssi_sync_internal(ctx));
@@ -572,82 +526,129 @@ int ssi_mh_run_host_slice(ssi_ctx* ctx, int kind, int64_t n_chains, int64_t n_st
         SSI_TRY(ssi_tc_range_exceeded(ctx, &exceeded));
         if (!exceeded) break;
     }
-    // a step's row of the device trace is this device's n_chains chains; in the host trace rows are ld_chains chains apart
-    const size_t rz = sizeof(float) * (size_t)ctx->Mz * n_chains, rl = sizeof(double) * (size_t)n_chains, ra = (size_t)n_chains;
-    if (z_trace) SSI_CUDA(ctx, cudaMemcpy2DAsync(z_trace + (size_t)c0 * ctx->Mz, sizeof(float) * (size_t)ctx->Mz * ld_chains, dzt, rz, rz, (size_t)n_steps,
-                                                 cudaMemcpyDeviceToHost, ctx->stream));
-    if (lp_trace) SSI_CUDA(ctx, cudaMemcpy2DAsync(lp_trace + c0, sizeof(double) * (size_t)ld_chains, dlt, rl, rl, (size_t)n_steps,
-                                                  cudaMemcpyDeviceToHost, ctx->stream));
-    if (accept_trace) SSI_CUDA(ctx, cudaMemcpy2DAsync(accept_trace + c0, (size_t)ld_chains, dat, ra, ra, (size_t)n_steps,
+    // a step's row of the device trace is this device's chains; in the host trace rows are run.n_chains chains apart
+    const int64_t ld = run.n_chains;
+    const size_t rz = sizeof(float) * (size_t)M * r.n_chains, rl = sizeof(double) * (size_t)r.n_chains, ra = (size_t)r.n_chains;
+    if (run.z_trace) SSI_CUDA(ctx, cudaMemcpy2DAsync(run.z_trace + (size_t)c0 * M, sizeof(float) * (size_t)M * ld, r.z_trace, rz, rz,
+                                                     (size_t)r.n_steps, cudaMemcpyDeviceToHost, ctx->stream));
+    if (run.lp_trace) SSI_CUDA(ctx, cudaMemcpy2DAsync(run.lp_trace + c0, sizeof(double) * (size_t)ld, r.lp_trace, rl, rl, (size_t)r.n_steps,
                                                       cudaMemcpyDeviceToHost, ctx->stream));
-    if (step_size_trace) SSI_CUDA(ctx, cudaMemcpy2DAsync(step_size_trace + c0, sizeof(double) * (size_t)ld_chains, det, rl, rl, (size_t)n_steps,
-                                                         cudaMemcpyDeviceToHost, ctx->stream));
+    if (run.accept_trace) SSI_CUDA(ctx, cudaMemcpy2DAsync(run.accept_trace + c0, (size_t)ld, r.accept_trace, ra, ra, (size_t)r.n_steps,
+                                                          cudaMemcpyDeviceToHost, ctx->stream));
+    if (run.step_size_trace) SSI_CUDA(ctx, cudaMemcpy2DAsync(run.step_size_trace + c0, sizeof(double) * (size_t)ld, r.step_size_trace, rl, rl,
+                                                             (size_t)r.n_steps, cudaMemcpyDeviceToHost, ctx->stream));
     SSI_TRY(ssi_sync_internal(ctx));
     return ssi_mh_fetch_accepts(ctx);
 }
+
+// Every sampler entry point: one check of the whole run, before any allocation, copy or device dispatch, then the run on
+// the device (dev: `r` holds device pointers) or sharded over the devices of the context.  kind_arg: the caller chose the
+// kind (ssi_mh_run_from[_dev]).
+static int mh_run(ssi_ctx* ctx, const ssi_mh_run_t& r, bool dev, bool kind_arg = false) {
+    if (!ctx) return SSI_ERR_ARG;
+    if (dev) SSI_NO_MULTI(ctx, "device-pointer entry points");
+    if (kind_arg && r.kind != 0 && r.kind != 1) return ssi_fail(ctx, SSI_ERR_ARG, "kind must be 0 (RWMH) or 1 (MALA)");
+    if (r.n_chains <= 0 || r.n_steps <= 0) return ssi_fail(ctx, SSI_ERR_ARG, "n_chains and n_steps must be positive");
+    if (r.chain_offset < 0 || r.step_offset < 0 || r.chain_offset > 0xffffffffll - r.n_chains || r.step_offset > 0xffffffffll - r.n_steps)
+        return ssi_fail(ctx, SSI_ERR_ARG, "chain ids and steps must fit 32 bits");
+    if (r.step_offset > 0 && !r.z0) return ssi_fail(ctx, SSI_ERR_ARG, "a continued run (step_offset > 0) needs the chain state z");
+    if (r.kind == 2) {
+        SSI_TRY(ssi_hmc_check(ctx, r.hp, ctx->Mz));
+        if (r.step_offset > 0 && r.hp->n_adapts > 0 && !r.adapt0)
+            return ssi_fail(ctx, SSI_ERR_ARG, "a continued HMC run with n_adapts > 0 needs the adaptation state (ssi_hmc_get_adapt)");
+    }
+    if (!ctx->has_model || !ctx->has_data || !ctx->has_sub)
+        return ssi_fail(ctx, SSI_ERR_STATE, "model, data and subspace must be set before sampling");
+    if (!dev) return ctx->is_multi() ? ssi_multi_mh_run(ctx, r) : ssi_mh_run_host_slice(ctx, r, 0, r.n_chains);
+    SSI_NVTX(mh_name(r.kind, true));
+    SSI_TRY(ssi_use_device(ctx));
+    call_timer t(ctx);
+    const int rc = ssi_mh_device(ctx, r);
+    t.stop(false);
+    return rc;
+}
+
 extern "C" {
 
-static int mh_run_host(ssi_ctx* ctx, int kind, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset, int64_t step_offset,
-                       double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask, const float* z0,
-                       float* z_trace, double* lp_trace, uint8_t* accept_trace,
-                       const ssi_hmc_params_t* hp = nullptr, const double* adapt0 = nullptr, double* step_size_trace = nullptr) {
-    if (!ctx) return SSI_ERR_ARG;
-    if (ctx->is_multi())
-        return ssi_multi_mh_run(ctx, kind, n_chains, n_steps, seed, chain_offset, step_offset, sigma_z, sigma_m, sigma_p, prior_mask, z0,
-                                z_trace, lp_trace, accept_trace, hp, adapt0, step_size_trace);
-    return ssi_mh_run_host_slice(ctx, kind, n_chains, n_steps, seed, chain_offset, step_offset, sigma_z, sigma_m, sigma_p, prior_mask, z0,
-                                 z_trace, lp_trace, accept_trace, n_chains, 0, hp, adapt0, step_size_trace);
-}
 int ssi_mh_run(ssi_ctx* ctx, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset,
                double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask, const float* z0,
                float* z_trace, double* lp_trace, uint8_t* accept_trace) {
-    return mh_run_host(ctx, 0, n_chains, n_steps, seed, chain_offset, 0, sigma_z, sigma_m, sigma_p, prior_mask, z0, z_trace, lp_trace,
-                       accept_trace);
+    return mh_run(ctx, {.kind = 0, .n_chains = n_chains, .n_steps = n_steps, .seed = seed, .chain_offset = chain_offset,
+                        .sigma_z = sigma_z, .sigma_m = sigma_m, .sigma_p = sigma_p, .mask = prior_mask, .z0 = z0,
+                        .z_trace = z_trace, .lp_trace = lp_trace, .accept_trace = accept_trace}, false);
+}
+int ssi_mh_run_dev(ssi_ctx* ctx, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset,
+                   double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask, const float* d_z0,
+                   float* d_z_trace, double* d_lp_trace, uint8_t* d_accept_trace) {
+    return mh_run(ctx, {.kind = 0, .n_chains = n_chains, .n_steps = n_steps, .seed = seed, .chain_offset = chain_offset,
+                        .sigma_z = sigma_z, .sigma_m = sigma_m, .sigma_p = sigma_p, .mask = prior_mask, .z0 = d_z0,
+                        .z_trace = d_z_trace, .lp_trace = d_lp_trace, .accept_trace = d_accept_trace}, true);
 }
 int ssi_mala_run(ssi_ctx* ctx, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset,
                  double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask, const float* z0,
                  float* z_trace, double* lp_trace, uint8_t* accept_trace) {
-    return mh_run_host(ctx, 1, n_chains, n_steps, seed, chain_offset, 0, sigma_z, sigma_m, sigma_p, prior_mask, z0, z_trace, lp_trace,
-                       accept_trace);
+    return mh_run(ctx, {.kind = 1, .n_chains = n_chains, .n_steps = n_steps, .seed = seed, .chain_offset = chain_offset,
+                        .sigma_z = sigma_z, .sigma_m = sigma_m, .sigma_p = sigma_p, .mask = prior_mask, .z0 = z0,
+                        .z_trace = z_trace, .lp_trace = lp_trace, .accept_trace = accept_trace}, false);
+}
+int ssi_mala_run_dev(ssi_ctx* ctx, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset,
+                     double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask, const float* d_z0,
+                     float* d_z_trace, double* d_lp_trace, uint8_t* d_accept_trace) {
+    return mh_run(ctx, {.kind = 1, .n_chains = n_chains, .n_steps = n_steps, .seed = seed, .chain_offset = chain_offset,
+                        .sigma_z = sigma_z, .sigma_m = sigma_m, .sigma_p = sigma_p, .mask = prior_mask, .z0 = d_z0,
+                        .z_trace = d_z_trace, .lp_trace = d_lp_trace, .accept_trace = d_accept_trace}, true);
 }
 int ssi_mh_run_from(ssi_ctx* ctx, int32_t kind, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset, int64_t step_offset,
                     double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask, const float* z_state,
                     float* z_trace, double* lp_trace, uint8_t* accept_trace) {
-    if (ctx && kind != 0 && kind != 1) return ssi_fail(ctx, SSI_ERR_ARG, "kind must be 0 (RWMH) or 1 (MALA)");
-    if (ctx && step_offset > 0 && !z_state) return ssi_fail(ctx, SSI_ERR_ARG, "a continued run (step_offset > 0) needs the chain state z");
-    return mh_run_host(ctx, kind, n_chains, n_steps, seed, chain_offset, step_offset, sigma_z, sigma_m, sigma_p, prior_mask, z_state,
-                       z_trace, lp_trace, accept_trace);
+    return mh_run(ctx, {.kind = kind, .n_chains = n_chains, .n_steps = n_steps, .seed = seed, .chain_offset = chain_offset,
+                        .step_offset = step_offset, .sigma_z = sigma_z, .sigma_m = sigma_m, .sigma_p = sigma_p,
+                        .mask = prior_mask, .z0 = z_state, .z_trace = z_trace, .lp_trace = lp_trace,
+                        .accept_trace = accept_trace}, false, true);
+}
+int ssi_mh_run_from_dev(ssi_ctx* ctx, int32_t kind, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset,
+                        int64_t step_offset, double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask,
+                        const float* d_z_state, float* d_z_trace, double* d_lp_trace, uint8_t* d_accept_trace) {
+    return mh_run(ctx, {.kind = kind, .n_chains = n_chains, .n_steps = n_steps, .seed = seed, .chain_offset = chain_offset,
+                        .step_offset = step_offset, .sigma_z = sigma_z, .sigma_m = sigma_m, .sigma_p = sigma_p,
+                        .mask = prior_mask, .z0 = d_z_state, .z_trace = d_z_trace, .lp_trace = d_lp_trace,
+                        .accept_trace = d_accept_trace}, true, true);
 }
 int ssi_hmc_run(ssi_ctx* ctx, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset, int64_t step_offset,
                 const ssi_hmc_params_t* hp, double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask,
                 const float* z_state, const double* adapt_state,
                 float* z_trace, double* lp_trace, uint8_t* accept_trace, double* step_size_trace) {
-    if (!ctx) return SSI_ERR_ARG;
-    // checked here as well as per device, so that a multi-device context reports the argument, not a device
-    SSI_TRY(ssi_hmc_check(ctx, hp, ctx->Mz));
-    if (step_offset > 0 && !z_state) return ssi_fail(ctx, SSI_ERR_ARG, "a continued run (step_offset > 0) needs the chain state z");
-    if (step_offset > 0 && hp->n_adapts > 0 && !adapt_state)
-        return ssi_fail(ctx, SSI_ERR_ARG, "a continued HMC run with n_adapts > 0 needs the adaptation state (ssi_hmc_get_adapt)");
-    return mh_run_host(ctx, 2, n_chains, n_steps, seed, chain_offset, step_offset, sigma_z, sigma_m, sigma_p, prior_mask, z_state,
-                       z_trace, lp_trace, accept_trace, hp, adapt_state, step_size_trace);
+    return mh_run(ctx, {.kind = 2, .n_chains = n_chains, .n_steps = n_steps, .seed = seed, .chain_offset = chain_offset,
+                        .step_offset = step_offset, .sigma_z = sigma_z, .sigma_m = sigma_m, .sigma_p = sigma_p,
+                        .mask = prior_mask, .hp = hp, .z0 = z_state, .adapt0 = adapt_state, .z_trace = z_trace,
+                        .lp_trace = lp_trace, .accept_trace = accept_trace, .step_size_trace = step_size_trace}, false);
+}
+int ssi_hmc_run_dev(ssi_ctx* ctx, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset, int64_t step_offset,
+                    const ssi_hmc_params_t* hp, double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask,
+                    const float* d_z_state, const double* d_adapt_state,
+                    float* d_z_trace, double* d_lp_trace, uint8_t* d_accept_trace, double* d_step_size_trace) {
+    return mh_run(ctx, {.kind = 2, .n_chains = n_chains, .n_steps = n_steps, .seed = seed, .chain_offset = chain_offset,
+                        .step_offset = step_offset, .sigma_z = sigma_z, .sigma_m = sigma_m, .sigma_p = sigma_p,
+                        .mask = prior_mask, .hp = hp, .z0 = d_z_state, .adapt0 = d_adapt_state, .z_trace = d_z_trace,
+                        .lp_trace = d_lp_trace, .accept_trace = d_accept_trace, .step_size_trace = d_step_size_trace}, true);
 }
 
 }  // extern "C"
 
-// final (z, lp) of the chains of the last run on this context: what a caller saves to continue later with ssi_mh_run_from
-int ssi_mh_get_state_slice(ssi_ctx* ctx, float* z_out, double* lp_out) {
-    if (ctx->mh_chains <= 0) return ssi_fail(ctx, SSI_ERR_STATE, "no chains have been run on this context");
+// final (z, lp) of the n chains of the last run on this device: what a caller saves to continue later with ssi_mh_run_from
+int ssi_mh_get_state_slice(ssi_ctx* ctx, int64_t n, float* z_out, double* lp_out) {
+    if (ctx->mh_chains != n) return ssi_fail(ctx, SSI_ERR_STATE, "no chains have been run on this context");
     SSI_TRY(ssi_use_device(ctx));
-    if (z_out) SSI_CUDA(ctx, cudaMemcpyAsync(z_out, ctx->bMhZ.p, sizeof(float) * (size_t)ctx->Mz * ctx->mh_chains, cudaMemcpyDeviceToHost, ctx->stream));
-    if (lp_out) SSI_CUDA(ctx, cudaMemcpyAsync(lp_out, ctx->bMhLp.p, sizeof(double) * (size_t)ctx->mh_chains, cudaMemcpyDeviceToHost, ctx->stream));
+    if (z_out) SSI_CUDA(ctx, cudaMemcpyAsync(z_out, ctx->bMhZ.p, sizeof(float) * (size_t)ctx->Mz * n, cudaMemcpyDeviceToHost, ctx->stream));
+    if (lp_out) SSI_CUDA(ctx, cudaMemcpyAsync(lp_out, ctx->bMhLp.p, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
     SSI_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return SSI_OK;
 }
-// dual-averaging state (3 x n_chains) of the last HMC run's chains on this device
-int ssi_hmc_get_adapt_slice(ssi_ctx* ctx, double* adapt_out) {
-    if (ctx->mh_chains <= 0 || ctx->mh_kind != 2) return ssi_fail(ctx, SSI_ERR_STATE, "the last run on this context was not HMC");
+// dual-averaging state (3 x n) of the n chains of the last HMC run on this device
+int ssi_hmc_get_adapt_slice(ssi_ctx* ctx, int64_t n, double* adapt_out) {
+    if (ctx->mh_chains != n || ctx->mh_kind != 2) return ssi_fail(ctx, SSI_ERR_STATE, "the last run on this context was not HMC");
     SSI_TRY(ssi_use_device(ctx));
-    SSI_CUDA(ctx, cudaMemcpyAsync(adapt_out, ctx->bHmcAd.p, sizeof(double) * 3 * (size_t)ctx->mh_chains, cudaMemcpyDeviceToHost, ctx->stream));
+    SSI_CUDA(ctx, cudaMemcpyAsync(adapt_out, ctx->bHmcAd.p, sizeof(double) * 3 * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
     SSI_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return SSI_OK;
 }
@@ -655,8 +656,9 @@ extern "C" {
 
 int ssi_mh_get_state(ssi_ctx* ctx, float* z_out, double* lp_out) {
     if (!ctx) return SSI_ERR_ARG;
+    if (ctx->mh_chains <= 0) return ssi_fail(ctx, SSI_ERR_STATE, "no chains have been run on this context");
     if (ctx->is_multi()) return ssi_multi_mh_get_state(ctx, z_out, lp_out);
-    return ssi_mh_get_state_slice(ctx, z_out, lp_out);
+    return ssi_mh_get_state_slice(ctx, ctx->mh_chains, z_out, lp_out);
 }
 
 int ssi_hmc_get_adapt(ssi_ctx* ctx, double* adapt_out) {
@@ -664,7 +666,7 @@ int ssi_hmc_get_adapt(ssi_ctx* ctx, double* adapt_out) {
     if (!adapt_out) return ssi_fail(ctx, SSI_ERR_ARG, "adapt_out is NULL");
     if (ctx->mh_chains <= 0 || ctx->mh_kind != 2) return ssi_fail(ctx, SSI_ERR_STATE, "the last run on this context was not HMC");
     if (ctx->is_multi()) return ssi_multi_hmc_get_adapt(ctx, adapt_out);
-    return ssi_hmc_get_adapt_slice(ctx, adapt_out);
+    return ssi_hmc_get_adapt_slice(ctx, ctx->mh_chains, adapt_out);
 }
 
 int ssi_rng_replay(uint64_t seed, int64_t chain, int64_t step, int32_t M, float* eps_out, double* e_out) {

@@ -183,29 +183,44 @@ int ssi_multi_set_data(ssi_ctx* ctx, const float* X, const float* Y, int64_t N);
 int ssi_multi_set_subspace(ssi_ctx* ctx, const float* W_swa, const float* P, int64_t n, int32_t M);
 int ssi_multi_logpost(ssi_ctx* ctx, int grad, const float* Z, int64_t B, double sigma_m, double sigma_p, double sigma_z, uint32_t mask,
                       double* lp_out, double* second_out);
-int ssi_multi_mh_run(ssi_ctx* ctx, int kind, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset, int64_t step_offset,
-                     double sigma_z, double sigma_m, double sigma_p, uint32_t mask, const float* z0,
-                     float* z_trace, double* lp_trace, uint8_t* accept_trace,
-                     const ssi_hmc_params_t* hp, const double* adapt0, double* step_size_trace);
+// One sampler run, as a public sampler entry point (include/ssi.h) received it and checked it.  Host pointers down to
+// ssi_mh_run_host_slice, which hands ssi_mh_device its shard's descriptor with device pointers.
+struct ssi_mh_run_t {
+    int kind = 0;                           // 0 RWMH, 1 MALA, 2 HMC
+    int64_t n_chains = 0, n_steps = 0;
+    uint64_t seed = 0;
+    int64_t chain_offset = 0, step_offset = 0;
+    double sigma_z = 1.0, sigma_m = 1.0, sigma_p = 1.0;
+    uint32_t mask = 0;
+    const ssi_hmc_params_t* hp = nullptr;   // kind 2 only, as are adapt0 and step_size_trace
+    const float* z0 = nullptr;
+    const double* adapt0 = nullptr;
+    float* z_trace = nullptr;
+    double* lp_trace = nullptr;
+    uint8_t* accept_trace = nullptr;
+    double* step_size_trace = nullptr;
+};
+
+int ssi_multi_mh_run(ssi_ctx* ctx, const ssi_mh_run_t& run);
 int ssi_multi_mh_get_state(ssi_ctx* ctx, float* z_out, double* lp_out);
 int ssi_multi_hmc_get_adapt(ssi_ctx* ctx, double* adapt_out);
 int ssi_multi_project(ssi_ctx* ctx, const float* Z, int64_t B, float* W_out);
 int ssi_multi_swa_finish(ssi_ctx* ctx, int32_t M, float* W_swa_out, float* P_out, double* s_out, int32_t install);
-// per-device halves of the host-pointer MH entry points (ssi_api.cu)
-// (kind 2, HMC: hp, the adaptation state adapt0 (3 x n_chains, or NULL) and the step-size trace; NULL for kinds 0 and 1)
-int ssi_mh_run_host_slice(ssi_ctx* ctx, int kind, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset, int64_t step_offset,
-                          double sigma_z, double sigma_m, double sigma_p, uint32_t prior_mask, const float* z0,
-                          float* z_trace, double* lp_trace, uint8_t* accept_trace, int64_t ld_chains, int64_t c0,
-                          const ssi_hmc_params_t* hp, const double* adapt0, double* step_size_trace);
-int ssi_mh_get_state_slice(ssi_ctx* ctx, float* z_out, double* lp_out);
-int ssi_hmc_get_adapt_slice(ssi_ctx* ctx, double* adapt_out);
+// per-device halves of the host-pointer MH entry points (ssi_api.cu): chains [c0, c1) of `run`, and the state of the
+// n chains of the last run on this device
+int ssi_mh_run_host_slice(ssi_ctx* ctx, const ssi_mh_run_t& run, int64_t c0, int64_t c1);
+int ssi_mh_get_state_slice(ssi_ctx* ctx, int64_t n, float* z_out, double* lp_out);
+int ssi_hmc_get_adapt_slice(ssi_ctx* ctx, int64_t n, double* adapt_out);
 
-// ---- HMC integrator (ssi_hmc.cu) -----------------------------------------------------------
+// ---- samplers (ssi_mh.cu, ssi_hmc.cu) --------------------------------------------------------
+// the run on this device; every pointer of `run` is a device pointer
+int ssi_mh_device(ssi_ctx* ctx, const ssi_mh_run_t& run);
+// the samplers' one density call: log-density (kind 0) or log-density and gradient (kinds 1, 2) of the run's n_chains
+// points zp into lpp (and gp), the work added to *units / *flops; the only place the run's sigmas meet the density's order
+int ssi_mh_density(ssi_ctx* ctx, const ssi_mh_run_t& run, const float* zp, double* lpp, double* gp, double* units, double* flops);
 int ssi_hmc_check(ssi_ctx* ctx, const ssi_hmc_params_t* hp, int M);
-int ssi_hmc_prepare(ssi_ctx* ctx, int64_t C, const ssi_hmc_params_t* hp, const double* d_adapt0);
-int ssi_hmc_transition(ssi_ctx* ctx, int64_t C, uint64_t seed, int64_t chain_off, int64_t t, const ssi_hmc_params_t* hp,
-                       double sigma_z, double sigma_m, double sigma_p, uint32_t mask, float* d_ztr, double* d_lptr,
-                       uint8_t* d_acctr, double* d_etr, double* units, double* flops);
+int ssi_hmc_prepare(ssi_ctx* ctx, const ssi_mh_run_t& run);
+int ssi_hmc_transition(ssi_ctx* ctx, const ssi_mh_run_t& run, int64_t i, double* units, double* flops);
 
 // ---- decoder (ssi_decoder.cu) -------------------------------------------------------------
 void ssi_dec_destroy(ssi_ctx* ctx);

@@ -171,30 +171,32 @@ int ssi_hmc_check(ssi_ctx* ctx, const ssi_hmc_params_t* hp, int M) {
     return SSI_OK;
 }
 
-// per-run state: the integrator buffers and the adaptation state, (log eps0, 0, 0) or d_adapt0 (3 x C, device)
-int ssi_hmc_prepare(ssi_ctx* ctx, int64_t C, const ssi_hmc_params_t* hp, const double* d_adapt0) {
+// per-run state: the integrator buffers and the adaptation state, (log eps0, 0, 0) or run.adapt0 (3 x n_chains, device)
+int ssi_hmc_prepare(ssi_ctx* ctx, const ssi_mh_run_t& r) {
     const int M = ctx->Mz;
+    const int64_t C = r.n_chains;
     SSI_TRY(ssi_reserve(ctx, ctx->bHmcP, sizeof(double) * (size_t)M * C));
     SSI_TRY(ssi_reserve(ctx, ctx->bHmcH0, sizeof(double) * (size_t)C));
     SSI_TRY(ssi_reserve(ctx, ctx->bHmcEps, sizeof(double) * (size_t)C));
     SSI_TRY(ssi_reserve(ctx, ctx->bHmcAd, sizeof(double) * 3 * (size_t)C));
     SSI_TRY(ssi_reserve(ctx, ctx->bHmcDiv, (size_t)C));
     double* ad = (double*)ctx->bHmcAd.p;
-    if (d_adapt0) {
-        SSI_CUDA(ctx, cudaMemcpyAsync(ad, d_adapt0, sizeof(double) * 3 * (size_t)C, cudaMemcpyDeviceToDevice, ctx->stream));
+    if (r.adapt0) {
+        SSI_CUDA(ctx, cudaMemcpyAsync(ad, r.adapt0, sizeof(double) * 3 * (size_t)C, cudaMemcpyDeviceToDevice, ctx->stream));
     } else {
-        k_hmc_adapt_init<<<(unsigned)((C + 127) / 128), 128, 0, ctx->stream>>>(C, std::log(hp->step_size), ad);
+        k_hmc_adapt_init<<<(unsigned)((C + 127) / 128), 128, 0, ctx->stream>>>(C, std::log(r.hp->step_size), ad);
         SSI_LAUNCH_CHECK(ctx);
     }
     return SSI_OK;
 }
 
-// one transition t >= 1 of all C chains: (z, lp, g) = (bMhZ, bMhLp, first half of bMhG) is the current state, bMhZp /
-// bMhLpP / the second half of bMhG hold the trajectory; the trace pointers address step t's row (or are NULL)
-int ssi_hmc_transition(ssi_ctx* ctx, int64_t C, uint64_t seed, int64_t chain_off, int64_t t, const ssi_hmc_params_t* hp,
-                       double sigma_z, double sigma_m, double sigma_p, uint32_t mask, float* d_ztr, double* d_lptr,
-                       uint8_t* d_acctr, double* d_etr, double* units, double* flops) {
+// transition t = step_offset + i >= 1 of all chains into trace row i: (z, lp, g) = (bMhZ, bMhLp, first half of bMhG) is
+// the current state, bMhZp / bMhLpP / the second half of bMhG hold the trajectory
+int ssi_hmc_transition(ssi_ctx* ctx, const ssi_mh_run_t& r, int64_t i, double* units, double* flops) {
     const int M = ctx->Mz;
+    const int64_t C = r.n_chains;
+    const unsigned t = (unsigned)(r.step_offset + i);
+    const ssi_hmc_params_t* hp = r.hp;
     hmc_minv_t minv;
     for (int m = 0; m < SSI_MAX_M; ++m) minv.v[m] = (hp->inv_metric && m < M) ? hp->inv_metric[m] : 1.0;
     float* z = (float*)ctx->bMhZ.p;
@@ -211,7 +213,7 @@ int ssi_hmc_transition(ssi_ctx* ctx, int64_t C, uint64_t seed, int64_t chain_off
     unsigned long long* cnt = (unsigned long long*)ctx->bMhCnt.p;
     const unsigned grid = (unsigned)((C + 127) / 128);
 
-    k_hmc_begin<<<grid, 128, 0, ctx->stream>>>(C, M, seed, chain_off, (unsigned)t, minv, hp->step_size, hp->n_adapts, z, lp, g, zp, p,
+    k_hmc_begin<<<grid, 128, 0, ctx->stream>>>(C, M, r.seed, r.chain_offset, t, minv, hp->step_size, hp->n_adapts, z, lp, g, zp, p,
                                                h0, eps, ad, div);
     SSI_LAUNCH_CHECK(ctx);
     for (int l = 0; l < hp->n_leapfrog; ++l) {
@@ -219,12 +221,12 @@ int ssi_hmc_transition(ssi_ctx* ctx, int64_t C, uint64_t seed, int64_t chain_off
             k_hmc_leap<<<grid, 128, 0, ctx->stream>>>(C, M, minv, z, zp, p, gp, eps, div);
             SSI_LAUNCH_CHECK(ctx);
         }
-        SSI_TRY(ssi_logpost_grad_device(ctx, zp, C, sigma_m, sigma_p, sigma_z, mask, lpp, gp));
-        *units += ctx->stats.last_units;
-        *flops += ctx->stats.last_flops;
+        SSI_TRY(ssi_mh_density(ctx, r, zp, lpp, gp, units, flops));
     }
-    k_hmc_end<<<grid, 128, 0, ctx->stream>>>(C, M, seed, chain_off, (unsigned)t, minv, hp->step_size, hp->n_adapts, hp->target_accept,
-                                             z, lp, g, zp, lpp, gp, p, h0, eps, ad, div, d_ztr, d_lptr, d_acctr, d_etr, cnt);
+    k_hmc_end<<<grid, 128, 0, ctx->stream>>>(C, M, r.seed, r.chain_offset, t, minv, hp->step_size, hp->n_adapts, hp->target_accept,
+                                             z, lp, g, zp, lpp, gp, p, h0, eps, ad, div, r.z_trace ? r.z_trace + (size_t)i * C * M : nullptr,
+                                             r.lp_trace ? r.lp_trace + (size_t)i * C : nullptr, r.accept_trace ? r.accept_trace + (size_t)i * C : nullptr,
+                                             r.step_size_trace ? r.step_size_trace + (size_t)i * C : nullptr, cnt);
     SSI_LAUNCH_CHECK(ctx);
     return SSI_OK;
 }

@@ -91,97 +91,86 @@ k_mh_accept(float* __restrict__ z, const float* __restrict__ zp, double* __restr
 //   `MALA(x -> MvNormal((sigma_z^2 / 2) .* x, sigma_z))`, init_params = rand(MvNormal(zeros(M), sigma_z))): the proposal is
 //   z' = z + (sigma_z^2/2) grad lp(z) + sigma_z eps, accepted iff -e < lp' - lp + log q(z|z') - log q(z'|z); value and
 //   gradient of every chain's proposal come from one batched reverse pass (ssi_logpost_grad_device) per step.
-// step0 > 0 continues chains (SURVEY 5, checkpoint / resume): d_z0 is then the state after step step0 - 1, its
+// step_offset > 0 continues chains (SURVEY 5, checkpoint / resume): z0 is then the state after step step_offset - 1, its
 // log-density (and gradient) is re-evaluated -- the evaluation is deterministic and batch-invariant, so the continued run
-// is bit-identical to an uninterrupted one -- and steps step0 .. step0 + S - 1 draw from the Philox counters of those
-// steps; trace row t - step0 receives step t.
-// kind 2: fixed-length HMC with per-chain dual averaging (ssi_hmc.cu, parameters hp): sample 0 and the re-established state
-//   of a continued run are MALA's (value and gradient cached per chain); every later step is one HMC transition.  d_adapt0
-//   (3 x C, device) is the adaptation state after step step0 - 1 (NULL: the initial one, allowed for step0 > 0 only when
-//   hp->n_adapts == 0); d_etr receives the step size of every transition (NaN for step 0).
-int ssi_mh_device(ssi_ctx* ctx, int kind, int64_t C, int64_t S, uint64_t seed, int64_t chain_off, int64_t step0,
-                  double sigma_z, double sigma_m, double sigma_p, uint32_t mask,
-                  const float* d_z0, float* d_ztr, double* d_lptr, uint8_t* d_acctr,
-                  const ssi_hmc_params_t* hp, const double* d_adapt0, double* d_etr) {
-    if (!ctx->has_model || !ctx->has_data || !ctx->has_sub)
-        return ssi_fail(ctx, SSI_ERR_STATE, "model, data and subspace must be set before sampling");
-    if (C <= 0 || S <= 0) return ssi_fail(ctx, SSI_ERR_ARG, "n_chains and n_steps must be positive");
-    if (step0 < 0 || (step0 > 0 && !d_z0)) return ssi_fail(ctx, SSI_ERR_ARG, "a continued run (step_offset > 0) needs the chain state z");
-    if (chain_off < 0 || chain_off + C > 0xffffffffll || step0 + S > 0xffffffffll)
-        return ssi_fail(ctx, SSI_ERR_ARG, "chain ids and steps must fit 32 bits");
+// is bit-identical to an uninterrupted one -- and the following steps draw from the Philox counters of those steps; trace
+// row i receives step step_offset + i.
+// kind 2: fixed-length HMC with per-chain dual averaging (ssi_hmc.cu): sample 0 and the re-established state of a continued
+//   run are MALA's (value and gradient cached per chain); every later step is one HMC transition.  adapt0 is the
+//   adaptation state after step step_offset - 1 (NULL: the initial one); step_size_trace receives the step size of every
+//   transition (NaN for step 0).
+// The arguments have been checked by the public entry point.
+int ssi_mh_device(ssi_ctx* ctx, const ssi_mh_run_t& r) {
     const int M = ctx->Mz;         // the sampler works in the caller's z (a decoder maps it inside the density)
-    if (kind == 2) {
-        SSI_TRY(ssi_hmc_check(ctx, hp, M));
-        if (step0 > 0 && hp->n_adapts > 0 && !d_adapt0)
-            return ssi_fail(ctx, SSI_ERR_ARG, "a continued HMC run with n_adapts > 0 needs the adaptation state (ssi_hmc_get_adapt)");
-    }
+    const int64_t C = r.n_chains;
     SSI_TRY(ssi_reserve(ctx, ctx->bMhZ, sizeof(float) * (size_t)M * C));
     SSI_TRY(ssi_reserve(ctx, ctx->bMhZp, sizeof(float) * (size_t)M * C));
     SSI_TRY(ssi_reserve(ctx, ctx->bMhLp, sizeof(double) * (size_t)C));
     SSI_TRY(ssi_reserve(ctx, ctx->bMhLpP, sizeof(double) * (size_t)C));
     SSI_TRY(ssi_reserve(ctx, ctx->bMhCnt, sizeof(unsigned long long)));
     double *g = nullptr, *gp = nullptr;
-    if (kind != 0) {
+    if (r.kind != 0) {
         SSI_TRY(ssi_reserve(ctx, ctx->bMhG, sizeof(double) * 2 * (size_t)M * C));
         g = (double*)ctx->bMhG.p;
         gp = g + (size_t)M * C;
     }
-    const double half_s2 = 0.5 * sigma_z * sigma_z, inv2s2 = 1.0 / (2.0 * sigma_z * sigma_z);
+    const double half_s2 = 0.5 * r.sigma_z * r.sigma_z, inv2s2 = 1.0 / (2.0 * r.sigma_z * r.sigma_z);
     float* z = (float*)ctx->bMhZ.p;
     float* zp = (float*)ctx->bMhZp.p;
     double* lp = (double*)ctx->bMhLp.p;
     double* lpp = (double*)ctx->bMhLpP.p;
     unsigned long long* cnt = (unsigned long long*)ctx->bMhCnt.p;
     SSI_CUDA(ctx, cudaMemsetAsync(cnt, 0, sizeof(unsigned long long), ctx->stream));
-    if (kind == 2) SSI_TRY(ssi_hmc_prepare(ctx, C, hp, d_adapt0));
+    if (r.kind == 2) SSI_TRY(ssi_hmc_prepare(ctx, r));
 
     const int nblk = (M + 3) / 4;
     const unsigned g_prop = (unsigned)((C * nblk + 255) / 256);
     const unsigned g_acc = (unsigned)((C + 255) / 256);
     double units = 0, flops = 0;
 
-    if (step0 > 0) {
+    if (r.step_offset > 0) {
         // re-establish (z, lp[, grad]) of the saved state: evaluate it as a proposal and force-accept it without a trace row
-        SSI_CUDA(ctx, cudaMemcpyAsync(zp, d_z0, sizeof(float) * (size_t)M * C, cudaMemcpyDeviceToDevice, ctx->stream));
-        if (kind != 0) SSI_TRY(ssi_logpost_grad_device(ctx, zp, C, sigma_m, sigma_p, sigma_z, mask, lpp, gp));
-        else SSI_TRY(ssi_logpost_device(ctx, zp, C, sigma_m, sigma_p, sigma_z, mask, lpp, nullptr));
-        units += ctx->stats.last_units;
-        flops += ctx->stats.last_flops;
-        k_mh_accept<<<g_acc, 256, 0, ctx->stream>>>(z, zp, lp, lpp, C, M, seed, chain_off, 0u, 1, nullptr, nullptr, nullptr, cnt, g, gp,
-                                                  half_s2, inv2s2, ctx->opt_mala_rule);
+        SSI_CUDA(ctx, cudaMemcpyAsync(zp, r.z0, sizeof(float) * (size_t)M * C, cudaMemcpyDeviceToDevice, ctx->stream));
+        SSI_TRY(ssi_mh_density(ctx, r, zp, lpp, gp, &units, &flops));
+        k_mh_accept<<<g_acc, 256, 0, ctx->stream>>>(z, zp, lp, lpp, C, M, r.seed, r.chain_offset, 0u, 1, nullptr, nullptr, nullptr, cnt,
+                                                  g, gp, half_s2, inv2s2, ctx->opt_mala_rule);
         SSI_LAUNCH_CHECK(ctx);
     }
-    for (int64_t i = 0; i < S; ++i) {
-        const int64_t t = step0 + i;
-        if (kind == 2 && t > 0) {
-            SSI_TRY(ssi_hmc_transition(ctx, C, seed, chain_off, t, hp, sigma_z, sigma_m, sigma_p, mask,
-                                       d_ztr ? d_ztr + (size_t)i * C * M : nullptr, d_lptr ? d_lptr + (size_t)i * C : nullptr,
-                                       d_acctr ? d_acctr + (size_t)i * C : nullptr, d_etr ? d_etr + (size_t)i * C : nullptr, &units, &flops));
+    for (int64_t i = 0; i < r.n_steps; ++i) {
+        const int64_t t = r.step_offset + i;
+        if (r.kind == 2 && t > 0) {
+            SSI_TRY(ssi_hmc_transition(ctx, r, i, &units, &flops));
             continue;
         }
-        if (t == 0 && d_z0) {
-            SSI_CUDA(ctx, cudaMemcpyAsync(zp, d_z0, sizeof(float) * (size_t)M * C, cudaMemcpyDeviceToDevice, ctx->stream));
+        if (t == 0 && r.z0) {
+            SSI_CUDA(ctx, cudaMemcpyAsync(zp, r.z0, sizeof(float) * (size_t)M * C, cudaMemcpyDeviceToDevice, ctx->stream));
         } else {
-            k_mh_propose<<<g_prop, 256, 0, ctx->stream>>>(z, zp, C, M, seed, chain_off, (unsigned)t, (float)sigma_z, t == 0, g, half_s2);
+            k_mh_propose<<<g_prop, 256, 0, ctx->stream>>>(z, zp, C, M, r.seed, r.chain_offset, (unsigned)t, (float)r.sigma_z, t == 0, g, half_s2);
             SSI_LAUNCH_CHECK(ctx);
         }
-        if (kind != 0) SSI_TRY(ssi_logpost_grad_device(ctx, zp, C, sigma_m, sigma_p, sigma_z, mask, lpp, gp));
-        else SSI_TRY(ssi_logpost_device(ctx, zp, C, sigma_m, sigma_p, sigma_z, mask, lpp, nullptr));
-        units += ctx->stats.last_units;
-        flops += ctx->stats.last_flops;
+        SSI_TRY(ssi_mh_density(ctx, r, zp, lpp, gp, &units, &flops));
         // trace row i of this call = step t of the chain
-        k_mh_accept<<<g_acc, 256, 0, ctx->stream>>>(z, zp, lp, lpp, C, M, seed, chain_off, (unsigned)t, t == 0,
-                                                  d_ztr ? d_ztr + (size_t)i * C * M : nullptr, d_lptr ? d_lptr + (size_t)i * C : nullptr,
-                                                  d_acctr ? d_acctr + (size_t)i * C : nullptr, cnt, g, gp, half_s2, inv2s2, ctx->opt_mala_rule);
+        k_mh_accept<<<g_acc, 256, 0, ctx->stream>>>(z, zp, lp, lpp, C, M, r.seed, r.chain_offset, (unsigned)t, t == 0,
+                                                  r.z_trace ? r.z_trace + (size_t)i * C * M : nullptr, r.lp_trace ? r.lp_trace + (size_t)i * C : nullptr,
+                                                  r.accept_trace ? r.accept_trace + (size_t)i * C : nullptr, cnt, g, gp, half_s2, inv2s2, ctx->opt_mala_rule);
         SSI_LAUNCH_CHECK(ctx);
         // the initial sample has no step size: all-ones bytes are a NaN double
-        if (kind == 2 && d_etr) SSI_CUDA(ctx, cudaMemsetAsync(d_etr, 0xff, sizeof(double) * (size_t)C, ctx->stream));
+        if (r.kind == 2 && r.step_size_trace)
+            SSI_CUDA(ctx, cudaMemsetAsync(r.step_size_trace, 0xff, sizeof(double) * (size_t)C, ctx->stream));
     }
     ctx->stats.last_units = units;
     ctx->stats.last_flops = flops;
-    ctx->stats.mh_proposals = C * (S - (step0 == 0 ? 1 : 0));
+    ctx->stats.mh_proposals = C * (r.n_steps - (r.step_offset == 0 ? 1 : 0));
     ctx->mh_chains = C;
-    ctx->mh_kind = kind;
+    ctx->mh_kind = r.kind;
+    return SSI_OK;
+}
+
+int ssi_mh_density(ssi_ctx* ctx, const ssi_mh_run_t& r, const float* zp, double* lpp, double* gp, double* units, double* flops) {
+    if (r.kind != 0) SSI_TRY(ssi_logpost_grad_device(ctx, zp, r.n_chains, r.sigma_m, r.sigma_p, r.sigma_z, r.mask, lpp, gp));
+    else SSI_TRY(ssi_logpost_device(ctx, zp, r.n_chains, r.sigma_m, r.sigma_p, r.sigma_z, r.mask, lpp, nullptr));
+    *units += ctx->stats.last_units;
+    *flops += ctx->stats.last_flops;
     return SSI_OK;
 }
 

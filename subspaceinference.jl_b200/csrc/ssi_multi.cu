@@ -43,6 +43,25 @@ int for_each_device(ssi_ctx* ctx, F fn) {
     return SSI_OK;
 }
 
+// run fn(child, begin, end) on every device whose shard [begin, end) of `total` items is not empty.  A device with an empty
+// shard takes no part; when the call does work (`work`), that device's per-call stats are cleared, so that ssi_stats
+// reports this call and not the device's previous one.
+template <typename F>
+int for_each_shard(ssi_ctx* ctx, int64_t total, bool work, F fn) {
+    const int n_dev = (int)ctx->children.size();
+    return for_each_device(ctx, [&](ssi_ctx* c, int d) {
+        int64_t b, e;
+        shard_range(total, n_dev, d, b, e);
+        if (e > b) return fn(c, b, e);
+        if (work) {
+            ssi_stats_t& s = c->stats;
+            s.last_ms = s.last_flops = s.last_bytes = s.last_units = 0.0;
+            s.mh_accepts = s.mh_proposals = 0;
+        }
+        return (int)SSI_OK;
+    });
+}
+
 }  // namespace
 
 extern "C" int ssi_ctx_create(int device, ssi_ctx** out);
@@ -160,12 +179,8 @@ int ssi_multi_logpost(ssi_ctx* ctx, int grad, const float* Z, int64_t B, double 
     if (!ctx->has_model || !ctx->has_data || !ctx->has_sub)
         return ssi_fail(ctx, SSI_ERR_STATE, "model, data and subspace must be set before evaluating the log-posterior");
     if (B == 0) return SSI_OK;
-    const int n_dev = (int)ctx->children.size();
     const int M = ctx->Mz;
-    return for_each_device(ctx, [&](ssi_ctx* c, int d) {
-        int64_t b0, b1;
-        shard_range(B, n_dev, d, b0, b1);
-        if (b1 <= b0) return (int)SSI_OK;
+    return for_each_shard(ctx, B, true, [&](ssi_ctx* c, int64_t b0, int64_t b1) {
         double* second = second_out ? second_out + (size_t)b0 * (grad ? M : 3) : nullptr;
         return grad ? ssi_logpost_grad_batch(c, Z + (size_t)b0 * M, b1 - b0, sigma_m, sigma_p, sigma_z, mask, lp_out + b0, second)
                     : ssi_logpost_batch(c, Z + (size_t)b0 * M, b1 - b0, sigma_m, sigma_p, sigma_z, mask, lp_out + b0, second);
@@ -173,59 +188,33 @@ int ssi_multi_logpost(ssi_ctx* ctx, int grad, const float* Z, int64_t B, double 
 }
 
 // chains [c0_d, c1_d) of the run go to device d with their global ids chain_offset + c; every device writes its columns
-// of each step's row of the host traces
-int ssi_multi_mh_run(ssi_ctx* ctx, int kind, int64_t n_chains, int64_t n_steps, uint64_t seed, int64_t chain_offset, int64_t step_offset,
-                     double sigma_z, double sigma_m, double sigma_p, uint32_t mask, const float* z0,
-                     float* z_trace, double* lp_trace, uint8_t* accept_trace,
-                     const ssi_hmc_params_t* hp, const double* adapt0, double* step_size_trace) {
-    if (n_chains <= 0 || n_steps <= 0) return ssi_fail(ctx, SSI_ERR_ARG, "n_chains and n_steps must be positive");
-    const int n_dev = (int)ctx->children.size();
-    ctx->mh_chains = n_chains;
-    ctx->mh_kind = kind;
-    return for_each_device(ctx, [&](ssi_ctx* c, int d) {
-        int64_t c0, c1;
-        shard_range(n_chains, n_dev, d, c0, c1);
-        c->mh_chains = 0;
-        if (c1 <= c0) return (int)SSI_OK;
-        return ssi_mh_run_host_slice(c, kind, c1 - c0, n_steps, seed, chain_offset + c0, step_offset, sigma_z, sigma_m, sigma_p, mask, z0,
-                                     z_trace, lp_trace, accept_trace, n_chains, c0, hp, adapt0, step_size_trace);
-    });
+// of each step's row of the host traces.  The arguments have been checked for the whole run before any device starts.
+int ssi_multi_mh_run(ssi_ctx* ctx, const ssi_mh_run_t& run) {
+    const int rc = for_each_shard(ctx, run.n_chains, true,
+                                  [&](ssi_ctx* c, int64_t c0, int64_t c1) { return ssi_mh_run_host_slice(c, run, c0, c1); });
+    if (rc == SSI_OK) { ctx->mh_chains = run.n_chains; ctx->mh_kind = run.kind; }
+    return rc;
 }
 
 int ssi_multi_mh_get_state(ssi_ctx* ctx, float* z_out, double* lp_out) {
-    if (ctx->mh_chains <= 0) return ssi_fail(ctx, SSI_ERR_STATE, "no chains have been run on this context");
-    const int n_dev = (int)ctx->children.size();
-    const int64_t C = ctx->mh_chains;
     const int M = ctx->Mz;
-    return for_each_device(ctx, [&](ssi_ctx* c, int d) {
-        int64_t c0, c1;
-        shard_range(C, n_dev, d, c0, c1);
-        if (c1 <= c0) return (int)SSI_OK;
-        return ssi_mh_get_state_slice(c, z_out ? z_out + (size_t)c0 * M : nullptr, lp_out ? lp_out + c0 : nullptr);
+    return for_each_shard(ctx, ctx->mh_chains, false, [&](ssi_ctx* c, int64_t c0, int64_t c1) {
+        return ssi_mh_get_state_slice(c, c1 - c0, z_out ? z_out + (size_t)c0 * M : nullptr, lp_out ? lp_out + c0 : nullptr);
     });
 }
 
 int ssi_multi_hmc_get_adapt(ssi_ctx* ctx, double* adapt_out) {
-    const int n_dev = (int)ctx->children.size();
-    const int64_t C = ctx->mh_chains;
-    return for_each_device(ctx, [&](ssi_ctx* c, int d) {
-        int64_t c0, c1;
-        shard_range(C, n_dev, d, c0, c1);
-        if (c1 <= c0) return (int)SSI_OK;
-        return ssi_hmc_get_adapt_slice(c, adapt_out + 3 * (size_t)c0);
+    return for_each_shard(ctx, ctx->mh_chains, false, [&](ssi_ctx* c, int64_t c0, int64_t c1) {
+        return ssi_hmc_get_adapt_slice(c, c1 - c0, adapt_out + 3 * (size_t)c0);
     });
 }
 
 int ssi_multi_project(ssi_ctx* ctx, const float* Z, int64_t B, float* W_out) {
     if (!ctx->has_model || !ctx->has_sub) return ssi_fail(ctx, SSI_ERR_STATE, "model and subspace must be set");
     if (B == 0) return SSI_OK;
-    const int n_dev = (int)ctx->children.size();
     const int M = ctx->Mz;
     const int64_t n = ctx->model.n;
-    return for_each_device(ctx, [&](ssi_ctx* c, int d) {
-        int64_t b0, b1;
-        shard_range(B, n_dev, d, b0, b1);
-        if (b1 <= b0) return (int)SSI_OK;
+    return for_each_shard(ctx, B, true, [&](ssi_ctx* c, int64_t b0, int64_t b1) {
         return ssi_project(c, Z + (size_t)b0 * M, b1 - b0, W_out + (size_t)b0 * n);
     });
 }

@@ -181,13 +181,17 @@ class Engine:
         return (mean, std, traj) if return_trajectories else (mean, std)
 
     # ---- RWMH ------------------------------------------------------------------------------
+    def _traces(self, n_chains: int, n_steps: int, want_z, want_lp, want_accept, want_step_size=False):
+        """Host traces of a sampler run (None where not wanted): z (M, n_chains, n_steps) f32, lp / accept / step size f64 / u8 / f64."""
+        per_chain = lambda want, dtype: np.empty((n_chains, n_steps), dtype, order="F") if want else None
+        return (np.empty((self.M, n_chains, n_steps), np.float32, order="F") if want_z else None,
+                per_chain(want_lp, np.float64), per_chain(want_accept, np.uint8), per_chain(want_step_size, np.float64))
+
     def mh_run(self, n_chains: int, n_steps: int, seed: int, sigma_z=1.0, sigma_m=1.0, sigma_p=1.0, mask=TERM_LL,
                chain_offset: int = 0, z0=None, want_z=True, want_lp=True, want_accept=True, kind: str = "rwmh"):
         """Returns (z_trace (M, n_chains, n_steps) f32, lp_trace (n_chains, n_steps) f64,
         accept (n_chains, n_steps) u8); entries not requested are None."""
-        zt = np.empty((self.M, n_chains, n_steps), np.float32, order="F") if want_z else None
-        lt = np.empty((n_chains, n_steps), np.float64, order="F") if want_lp else None
-        at = np.empty((n_chains, n_steps), np.uint8, order="F") if want_accept else None
+        zt, lt, at, _ = self._traces(n_chains, n_steps, want_z, want_lp, want_accept)
         z0a = _f32(z0) if z0 is not None else None
         if z0a is not None and z0a.shape != (self.M, n_chains):
             raise ValueError("z0 must be (M, n_chains)")
@@ -210,9 +214,7 @@ class Engine:
         """Continue chains saved with mh_state(): steps step_offset .. step_offset + n_steps - 1 of the same Philox streams."""
         z_state = _f32(z_state)
         n_chains = z_state.shape[1]
-        zt = np.empty((self.M, n_chains, n_steps), np.float32, order="F") if want_z else None
-        lt = np.empty((n_chains, n_steps), np.float64, order="F") if want_lp else None
-        at = np.empty((n_chains, n_steps), np.uint8, order="F") if want_accept else None
+        zt, lt, at, _ = self._traces(n_chains, n_steps, want_z, want_lp, want_accept)
         self._check(self._lib.ssi_mh_run_from(self._h, {"rwmh": 0, "mala": 1}[kind], n_chains, n_steps, seed, chain_offset, step_offset,
                                               sigma_z, sigma_m, sigma_p, mask, _ptr(z_state), _ptr(zt), _ptr(lt), _ptr(at)))
         self._last_chains = n_chains
@@ -249,10 +251,7 @@ class Engine:
         Returns (z_trace (M, n_chains, n_steps) f32, lp_trace (n_chains, n_steps) f64, accept (n_chains, n_steps) u8 with
         1 accepted / 0 rejected / 2 divergent, step_size_trace (n_chains, n_steps) f64, NaN at step 0); entries not
         requested are None.  step_offset > 0 continues chains from z0 = mh_state()[0] and adapt_state = hmc_adapt()."""
-        zt = np.empty((self.M, n_chains, n_steps), np.float32, order="F") if want_z else None
-        lt = np.empty((n_chains, n_steps), np.float64, order="F") if want_lp else None
-        at = np.empty((n_chains, n_steps), np.uint8, order="F") if want_accept else None
-        et = np.empty((n_chains, n_steps), np.float64, order="F") if want_step_size else None
+        zt, lt, at, et = self._traces(n_chains, n_steps, want_z, want_lp, want_accept, want_step_size)
         z0a = _f32(z0) if z0 is not None else None
         if z0a is not None and z0a.shape != (self.M, n_chains):
             raise ValueError("z0 must be (M, n_chains)")
