@@ -184,6 +184,30 @@ def _act_deriv_from_output(h: np.ndarray, act: int) -> np.ndarray:
     return np.ones_like(h)
 
 
+def _forward_all(w: np.ndarray, dims, acts, X: np.ndarray):
+    """(layers, [H_0 = X, H_1, ..., H_L]): the forward pass with every activation kept, Float64."""
+    layers = restructure(np.asarray(w, np.float64), dims)
+    hs = [np.asarray(X, np.float64)]
+    for (W, b), act in zip(layers, acts):
+        hs.append(_activate(W @ hs[-1] + b[:, None], act))
+    return layers, hs
+
+
+def _reverse_gw(layers, hs, dims, acts, delta: np.ndarray) -> np.ndarray:
+    """Reverse pass through the Dense chain from the output delta dL/d(pre_L) (O, N): dL/dw in the flat layout,
+    ``gW_l = delta_l H_{l-1}'``, ``gb_l = rowsum(delta_l)``, ``delta_{l-1} = (W_l' delta_l) * act_{l-1}'(H_{l-1})``."""
+    gw = np.zeros(n_params(dims))
+    offs = layer_offsets(dims)
+    for l in range(len(layers) - 1, -1, -1):
+        W, _ = layers[l]
+        w0, b0, _, dout = offs[l]
+        gw[w0:b0] = (delta @ hs[l].T).reshape(-1, order="F")       # vec(W_l) is column-major (o + i*out)
+        gw[b0:b0 + dout] = delta.sum(axis=1)
+        if l > 0:
+            delta = (W.T @ delta) * _act_deriv_from_output(hs[l], acts[l - 1])
+    return gw
+
+
 def density_and_grad(prob: Problem, z, sigma_m=1.0, sigma_p=1.0, sigma_z=1.0, mask=TERM_LL):
     """``l_pi_grad(theta) = (density(theta), gradient(density, theta))`` (src/space_inference.jl:107), the closure of
     the :mala/:hmc/:nuts branches.  The reference differentiates ``density`` with ForwardDiff/ReverseDiff/Zygote
@@ -191,22 +215,12 @@ def density_and_grad(prob: Problem, z, sigma_m=1.0, sigma_p=1.0, sigma_z=1.0, ma
     ``P' grad_W``) and pinned against torch autograd and central differences in tests/test_oracle.py."""
     z = np.asarray(z, np.float64)
     w = project(prob.W_swa, prob.P, z)
-    layers = restructure(w, prob.dims)
-    hs = [np.asarray(prob.X, np.float64)]
-    for (W, b), act in zip(layers, prob.acts):
-        hs.append(_activate(W @ hs[-1] + b[:, None], act))
+    layers, hs = _forward_all(w, prob.dims, prob.acts, prob.X)
     lp = density(prob, z, sigma_m, sigma_p, sigma_z, mask)
     gw = np.zeros_like(w)
     if mask & TERM_LL:
         delta = -(hs[-1] - np.asarray(prob.Y, np.float64)) / (sigma_m * sigma_m) * _act_deriv_from_output(hs[-1], prob.acts[-1])
-        offs = layer_offsets(prob.dims)
-        for l in range(len(layers) - 1, -1, -1):
-            W, _ = layers[l]
-            w0, b0, _, dout = offs[l]
-            gw[w0:b0] = (delta @ hs[l].T).reshape(-1, order="F")       # vec(W_l) is column-major (o + i*out)
-            gw[b0:b0 + dout] = delta.sum(axis=1)
-            if l > 0:
-                delta = (W.T @ delta) * _act_deriv_from_output(hs[l], prob.acts[l - 1])
+        gw = _reverse_gw(layers, hs, prob.dims, prob.acts, delta)
     P = np.asarray(prob.P, np.float64)
     g = P.T @ gw
     if mask & TERM_PRIOR_W:
@@ -408,6 +422,29 @@ def predictive_sweep(dims, acts, W_swa: np.ndarray, P: np.ndarray, Z: np.ndarray
 def samples_to_weights(prob: Problem, z_trace: np.ndarray) -> np.ndarray:
     """``map(z -> W_swa + P*z.params, chm)`` (src/space_inference.jl:125): (n_steps, n)."""
     return np.stack([project(prob.W_swa, prob.P, z) for z in z_trace])
+
+
+# --------------------------------------------------------------------------------------
+# Mini-batch training step                                (src/subspace_construction.jl:39-43)
+# --------------------------------------------------------------------------------------
+def mse_loss_and_grad(w: np.ndarray, dims, acts, X: np.ndarray, Y: np.ndarray):
+    """``training_loss = Flux.Losses.mse(m(x), y)`` and its gradient for the Dense chain with flat parameters ``w``:
+    loss = mean((pred - Y)^2) over all O*nb entries, gw = dL/dw in the flat layout [vec(W_1); b_1; ...].  Float64."""
+    layers, hs = _forward_all(w, dims, acts, X)
+    r = hs[-1] - np.asarray(Y, np.float64)
+    delta = (2.0 / r.size) * r * _act_deriv_from_output(hs[-1], acts[-1])
+    return float(np.mean(r * r)), _reverse_gw(layers, hs, dims, acts, delta)
+
+
+def adam_step(w, g, m, v, t: int, eta: float, b1: float = 0.9, b2: float = 0.999):
+    """Step t (1-based) of Flux 0.11's ADAM, in Float64: ``m = b1 m + (1-b1) g``, ``v = b2 v + (1-b2) g^2``,
+    ``w -= eta m/(1-b1^t) / (sqrt(v/(1-b2^t)) + 1e-8)`` (Flux keeps b^t as a running product starting at b).
+    Returns (w, m, v)."""
+    g = np.asarray(g, np.float64)
+    m = b1 * np.asarray(m, np.float64) + (1.0 - b1) * g
+    v = b2 * np.asarray(v, np.float64) + (1.0 - b2) * g * g
+    w = np.asarray(w, np.float64) - m / (1.0 - b1 ** t) / (np.sqrt(v / (1.0 - b2 ** t)) + 1e-8) * eta
+    return w, m, v
 
 
 # --------------------------------------------------------------------------------------

@@ -11,6 +11,7 @@ import pytest
 import scipy.stats as st
 
 import ssi_oracle as orc
+from conftest import stable_seed
 
 GOLD = Path(__file__).parent / "golden"
 
@@ -250,6 +251,49 @@ def test_density_gradient_against_torch_autograd_and_central_differences(dims, a
             tot = tot - (zt ** 2).sum() / (2 * sz * sz)
         tot.backward()
         np.testing.assert_allclose(g, zt.grad.numpy(), rtol=1e-10, atol=1e-12)
+
+
+@pytest.mark.parametrize("dims,acts", [((3, 6, 4, 2), (2, 3, 0)), ((5, 9, 7, 3), (1, 0, 2)), ((4, 5, 2), (3, 1))])
+def test_mse_gradient_against_torch_autograd(dims, acts):
+    """The training step's cost, Flux.Losses.mse(m(x), y) (src/subspace_construction.jl:39-43): loss and dL/dw in the flat
+    layout vs torch autograd in Float64, every activation in a hidden and in the output position."""
+    import torch
+    rng = np.random.default_rng(stable_seed(dims, acts))
+    nb = 13
+    w = orc.glorot_flat(rng, dims) + 0.1 * rng.standard_normal(orc.n_params(dims)).astype(np.float32)
+    X = rng.standard_normal((dims[0], nb)).astype(np.float32)
+    Y = rng.standard_normal((dims[-1], nb)).astype(np.float32)
+    loss, gw = orc.mse_loss_and_grad(w, dims, acts, X, Y)
+    wt = torch.tensor(w, dtype=torch.float64, requires_grad=True)
+    h, off = torch.from_numpy(X.astype(np.float64)), 0
+    for l, act in enumerate(acts):
+        i, o = dims[l], dims[l + 1]
+        Wl = wt[off:off + i * o].reshape(i, o).T
+        off += i * o
+        h = [lambda x: x, torch.relu, torch.tanh, torch.sigmoid][act](Wl @ h + wt[off:off + o][:, None])
+        off += o
+    tot = torch.mean((h - torch.from_numpy(Y.astype(np.float64))) ** 2)
+    tot.backward()
+    np.testing.assert_allclose(loss, tot.item(), rtol=1e-12)
+    np.testing.assert_allclose(gw, wt.grad.numpy(), rtol=1e-10, atol=1e-12 * np.abs(gw).max())
+
+
+def test_adam_step_matches_flux_adam(ssi):
+    """Five steps of the Float64 ADAM restatement vs the package's Flux 0.11 ADAM (torch, Float32)."""
+    import torch
+    rng = np.random.default_rng(5)
+    n, eta, beta = 257, 3e-3, (0.8, 0.99)
+    w0 = rng.standard_normal(n).astype(np.float32)
+    p = torch.tensor(w0, requires_grad=True)
+    opt = ssi.ADAM(eta, beta)
+    w, m, v = w0.astype(np.float64), np.zeros(n), np.zeros(n)
+    for t in range(1, 6):
+        g = (rng.standard_normal(n) * 10.0 ** rng.uniform(-4, 1, n)).astype(np.float32)
+        p.grad = torch.from_numpy(g.copy())
+        opt.update([p])
+        w, m, v = orc.adam_step(w, g, m, v, t, eta, *beta)
+        np.testing.assert_allclose(p.detach().numpy(), w, rtol=0, atol=4 * np.spacing(np.float32(np.abs(w).max())) + 1e-6 * eta,
+                                   err_msg=f"step {t}")
 
 
 def test_mala_restatement_satisfies_detailed_balance():
