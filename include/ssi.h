@@ -98,6 +98,7 @@ typedef struct ssi_stats_t {
     int64_t tc_range_fallbacks;/* tensor path: evaluations repeated on BF16 planes because an activation left the   */
                                /* calibrated range of the FP16 planes (see DESIGN.md 4.1); 0 in normal operation   */
     int64_t gemm_tc_launches;  /* gradient / training GEMMs this context ran on the tensor cores (ssi_gemm_tc.cu)     */
+    int64_t gemm_skinny_launches; /* narrow-layer GEMMs of the gradient / training paths that ran on k_gemm_skinny_* */
 } ssi_stats_t;
 
 int  ssi_version(void);

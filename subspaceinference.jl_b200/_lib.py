@@ -37,7 +37,7 @@ class Stats(C.Structure):
         ("gram_path", C.c_int32), ("jacobi_sweeps", C.c_int32), ("gram_risk", C.c_double),
         ("dominant_ms", C.c_double), ("dominant_launches", C.c_int64),
         ("finish_gram_ms", C.c_double), ("finish_eigen_ms", C.c_double), ("finish_p_ms", C.c_double),
-        ("tc_range_fallbacks", C.c_int64), ("gemm_tc_launches", C.c_int64),
+        ("tc_range_fallbacks", C.c_int64), ("gemm_tc_launches", C.c_int64), ("gemm_skinny_launches", C.c_int64),
     ]
 
 

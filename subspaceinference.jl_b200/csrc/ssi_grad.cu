@@ -306,6 +306,7 @@ static int gemm_skinny_try(ssi_ctx* ctx, const gemm_t& g, int batches, bool a_kf
         SSI_LAUNCH_CHECK(ctx);
         *used = true;
     }
+    if (*used) ++ctx->stats.gemm_skinny_launches;
     return SSI_OK;
 }
 

@@ -142,6 +142,7 @@ int ssi_multi_stats(const ssi_ctx* ctx, ssi_stats_t* out) {
             acc.dominant_ms = std::max(acc.dominant_ms, s.dominant_ms);
             acc.dominant_launches += s.dominant_launches;
             acc.gemm_tc_launches += s.gemm_tc_launches;
+            acc.gemm_skinny_launches += s.gemm_skinny_launches;
         }
     }
     *out = acc;

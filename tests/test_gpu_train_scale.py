@@ -1,11 +1,9 @@
 """The on-device training step (src/subspace_construction.jl:39-43) and the long-contraction GEMMs of the gradient path at
 the sizes they run at, against the Float64 oracle.
 
-The library has no gradient readback, and none is needed: a Descent step computes W1 = float((double)W0 - eta * (double)G)
-(ssi_train.cu, k_train_update), so g = (W0 - W1) / eta in Float64 recovers the device's FP32 gradient G to about 2^-24
-relative wherever eta |G| >> |W0| (`probe_grad`).  With that, the step is compared block by block (every W_l and b_l) with
-`ssi_oracle.mse_loss_and_grad`, on the tensor-core kernels and, beside them, with every contraction forced onto the FP32
-SIMT kernel (option gemm_simt).
+The device's FP32 gradient is read through one Descent step (`probe_grad`, tests/train_probe.py) and compared block by
+block (every W_l and b_l) with `ssi_oracle.mse_loss_and_grad`, on the tensor-core kernels and, beside them, with every
+contraction forced onto the FP32 SIMT kernel (option gemm_simt).
 
 What the shapes reach (ssi_grad.cu / ssi_gemm_tc.cu dispatch):
   * C4, 784-2048-2048-2048-10 relu, nb = 512 (the benched step): the three hidden forwards, three hidden weight gradients
@@ -25,55 +23,21 @@ Measured on one B200 at its 1000 W power limit, worst block error relative to th
   Loss within 2.9e-7 (tensor cores) and 1.2e-8 (SIMT) of the oracle.  ADAM: 0.24 of the per-element bar; SWA mean and
   deviations 0.31 of theirs.  logpost_grad on 96-1300-1100-8: 6.8e-7 / 1.3e-6 (mask 1), 4.2e-6 / 3.1e-6 (mask 7).
 The tensor-core error is up to 64 times the SIMT error per block: it is the truncation bias of k_gemm_tc's accumulator
-(TC_TRUNCATION below; with 16-block chunks it halves), so the tensor-core bar is 2.5x the SIMT error plus that budget.
-The relu data sets are built without pre-activations near the kink (`_problem`); before that, one flipped relu
-decision put 2e-4 of the block norm on the first layers' gradient on SIMT and tensor cores alike.
+(TC_TRUNCATION in tests/train_probe.py; with 16-block chunks it halves), so the tensor-core bar is 2.5x the SIMT error
+plus that budget.  The relu data sets are built without pre-activations near the kink (`problem`); before that, one flipped
+relu decision put 2e-4 of the block norm on the first layers' gradient on SIMT and tensor cores alike.
 """
 import numpy as np
 import pytest
 
 import ssi_oracle as orc
 from conftest import stable_seed
+from train_probe import BLOCK_BAR, LOSS_RTOL, TC_OVER_SIMT, TC_TRUNCATION, block_errors, probe_grad, problem
 
 pytestmark = pytest.mark.gpu
 
 C4_DIMS, C4_ACTS = (784, 2048, 2048, 2048, 10), (1, 1, 1, 0)
 RAGGED_DIMS, RAGGED_ACTS = (97, 1300, 1100, 7), (2, 3, 0)
-BLOCK_BAR = 5e-5            # per-block error, relative to the block norm
-TC_OVER_SIMT = 2.5          # tensor-core error no worse than this multiple of the FP32 SIMT error ...
-# ... plus the truncation of k_gemm_tc's FP32 accumulator: every MMA's add rounds toward zero, six adds per 32-wide k-block,
-# and the accumulator is drained every 32 k-blocks.  Measured: the error is linear in the chunk length (halved at 16), and
-# systematic, so the row sums of the bias gradients keep it (SIMT rounds to nearest: 1e-7 to 5e-7 on these shapes).
-TC_TRUNCATION = 32 * 6 * 2.0 ** -24
-RELU_BAND = 3e-5            # no relu pre-activation of the data sets below comes closer than this to 0
-LOSS_RTOL = 1e-5
-
-
-def _problem(dims, acts, N, seed):
-    """Training data as profiles/bench_streams.py builds it for C4: X uniform in [0, 1), Y standard normal.  The weights
-    are Flux's glorot init with biases drawn uniform in [-0.1, 0.1), so that every bias term of the epilogues counts.
-
-    relu is not differentiable at 0: a pre-activation within FP32 rounding of 0 can take the other branch on the device,
-    and one such flip moves a whole block's gradient by ~1e-3 of its norm (one element of delta_l against a sum of nb
-    rank-one terms).  So the bias of every relu unit whose pre-activation comes within RELU_BAND of 0 on any datapoint is
-    drawn again, layer by layer in Float64, until none does."""
-    rng = np.random.default_rng(seed)
-    W0 = orc.glorot_flat(rng, dims)
-    X = rng.random((dims[0], N), dtype=np.float32)
-    Y = rng.standard_normal((dims[-1], N)).astype(np.float32)
-    h = X.astype(np.float64)
-    for (w_off, b_off, din, dout), act in zip(orc.layer_offsets(dims), acts):
-        W = W0[w_off:b_off].reshape(din, dout).T.astype(np.float64)
-        b = W0[b_off:b_off + dout]
-        b[:] = rng.uniform(-0.1, 0.1, dout)
-        pre = W @ h + b.astype(np.float64)[:, None]
-        redo = np.flatnonzero(np.abs(pre).min(axis=1) < RELU_BAND) if act == orc.ACT_RELU else []
-        while len(redo):
-            b[redo] = rng.uniform(-0.1, 0.1, len(redo))
-            pre[redo] = W[redo] @ h + b[redo].astype(np.float64)[:, None]
-            redo = redo[np.abs(pre[redo]).min(axis=1) < RELU_BAND]
-        h = orc._activate(pre, act)
-    return W0, X, Y
 
 
 def _setup(engine, dims, acts, X, Y):
@@ -87,34 +51,6 @@ def _columns(batch):
     return np.asarray(batch)
 
 
-def probe_grad(engine, W0, batch, want_loss=True):
-    """(loss, g, W1): the FP32 gradient the device's training step computes at W0 on `batch`, read through one Descent step.
-
-    A first step at eta = 1 gives max |G| to FP32 precision; the probe step is then the power of two that puts
-    eta max|G| near 2^40, so that (W0 - W1) / eta is exact in Float64 apart from the one FP32 rounding of W1, and nothing
-    overflows.  W1 (the probe's raw output) is returned for bitwise comparisons.  The training state is left at W0 again,
-    so the caller may probe once more or begin its own run."""
-    W0 = np.asarray(W0, np.float32)
-    engine.train_begin(W0, "descent", 1.0)
-    engine.train_step(batch)
-    gmax = np.abs(W0.astype(np.float64) - engine.train_weights()).max()
-    eta = 2.0 ** (40 - int(np.ceil(np.log2(gmax))))
-    engine.train_begin(W0, "descent", eta)
-    loss = engine.train_step(batch, want_loss=want_loss)
-    W1 = engine.train_weights()
-    engine.train_begin(W0, "descent", eta)
-    return loss, (W0.astype(np.float64) - W1.astype(np.float64)) / eta, W1
-
-
-def _block_errors(g, g_ref, dims):
-    """[(name, |g - g_ref| / |g_ref|)] for every W_l and b_l."""
-    out = []
-    for l, (w_off, b_off, din, dout) in enumerate(orc.layer_offsets(dims)):
-        for name, lo, hi in ((f"W{l + 1}", w_off, b_off), (f"b{l + 1}", b_off, b_off + dout)):
-            out.append((name, np.linalg.norm(g[lo:hi] - g_ref[lo:hi]) / np.linalg.norm(g_ref[lo:hi])))
-    return out
-
-
 def _check_step(engine, label, dims, acts, W0, X, Y, batch, tc_launches):
     """Probe the step on the tensor-core kernels and on SIMT; check loss and every block against the oracle."""
     cols = _columns(batch)
@@ -125,7 +61,7 @@ def _check_step(engine, label, dims, acts, W0, X, Y, batch, tc_launches):
         before = engine.stats().gemm_tc_launches
         loss, g, W1 = probe_grad(engine, W0, batch)
         launches = (engine.stats().gemm_tc_launches - before) / 2          # probe_grad takes two steps
-        res[mode] = (loss, _block_errors(g, g_ref, dims), launches, W1)
+        res[mode] = (loss, block_errors(g, g_ref, dims), launches, W1)
     engine.set_option("gemm_simt", 0)
     (loss_t, err_t, n_t, W1_t), (loss_s, err_s, n_s, _) = res["tc"], res["simt"]
     print(f"\n{label}: loss {loss_ref:.9g}, rel err tc {abs(loss_t / loss_ref - 1):.1e} simt {abs(loss_s / loss_ref - 1):.1e}; "
@@ -147,7 +83,7 @@ def test_training_gradient_c4(engine, nb):
     kernels, as a contiguous window and, at nb = 512, as an index batch over the same columns (the gather path).  Also:
     the window and the index batch give identical weights (same kernels: 784 * 4 bytes is 16-byte aligned), a repeated probe
     gives identical weights, and a step without the loss read back updates the weights identically."""
-    W0, X, Y = _problem(C4_DIMS, C4_ACTS, 4096, stable_seed("c4", nb))
+    W0, X, Y = problem(C4_DIMS, C4_ACTS, 4096, stable_seed("c4", nb))
     _setup(engine, C4_DIMS, C4_ACTS, X, Y)
     j0 = 1024 + 5
     W1_win = _check_step(engine, f"C4 nb={nb} window j0={j0}", C4_DIMS, C4_ACTS, W0, X, Y, (j0, nb), 8)
@@ -166,7 +102,7 @@ def test_training_gradient_ragged(engine, kind):
     accumulation chunk is one k-block, the tanh derivative after a two-chunk back-propagation, and SIMT layers (the ones that
     read X, whose row stride of 97 floats TMA cannot address) mixed into the same step."""
     N, nb = 3000, 1025
-    W0, X, Y = _problem(RAGGED_DIMS, RAGGED_ACTS, N, stable_seed("ragged", kind))
+    W0, X, Y = problem(RAGGED_DIMS, RAGGED_ACTS, N, stable_seed("ragged", kind))
     _setup(engine, RAGGED_DIMS, RAGGED_ACTS, X, Y)
     batch = np.random.default_rng(3).permutation(N)[:nb] if kind == "index" else (3, nb)
     # k_gemm_tc: hidden forward (K = 1300), hidden weight gradient (K = 1025), back-propagation into the tanh layer (K = 1100)
@@ -178,7 +114,7 @@ def test_adam_and_snapshots_teacher_forced(ssi):
     with the gradient A used (read by a Descent probe on engine B at the same weights and batch: the kernels are
     deterministic).  The optimiser's m and v live in FP32 on the device, so the allowed error is 1e-6 eta plus 2 ulp of W.
     A snapshot follows every step; the SWA mean and the deviation columns are checked against the Float64 recurrence."""
-    W0, X, Y = _problem(C4_DIMS, C4_ACTS, 4096, stable_seed("adam"))
+    W0, X, Y = problem(C4_DIMS, C4_ACTS, 4096, stable_seed("adam"))
     eta, beta, nb, steps = 1e-3, (0.9, 0.999), 512, 8
     n = orc.n_params(C4_DIMS)
     with ssi.Engine(0) as A, ssi.Engine(0) as B:
@@ -223,7 +159,7 @@ def test_gradient_long_contractions(engine, mask):
     forward (bias + sigmoid), weight-gradient and back-propagation (tanh derivative) epilogues, against the Float64 oracle
     and against the same call on SIMT, with the bars of test_gradient_wide_on_tensor_cores."""
     dims, acts, N, M, B = (96, 1300, 1100, 8), (2, 3, 0), 1500, 6, 3
-    W_swa, X, Y = _problem(dims, acts, N, stable_seed("grad", mask))
+    W_swa, X, Y = problem(dims, acts, N, stable_seed("grad", mask))
     rng = np.random.default_rng(stable_seed("grad-P", mask))
     prob = orc.Problem(dims, acts, X, Y, W_swa, orc.synthetic_subspace(rng, orc.n_params(dims), M, 0.5 ** np.arange(1, M + 1)))
     engine.set_model(dims, acts)
