@@ -91,8 +91,8 @@ struct ssi_ctx {
     // scratch
     ssi_buf_t bZ, bLp, bTerms, bPartials, bW, bH0, bH1, bGram, bEig, bMisc, bGradW, bGradP;
     ssi_buf_t bGemmAmax;      // per-batch operand magnitudes of the tensor-core GEMM in flight (ssi_gemm_tc.cu)
-    ssi_buf_t bSkinny;        // contraction-slice partials of the skinny weight-gradient kernel (ssi_grad.cu)
-    ssi_buf_t bRowsum;        // per-slice partials of the bias gradients (ssi_grad.cu)
+    ssi_buf_t bSkinny;        // contraction-slice partials of the skinny weight-gradient kernel (ssi_gemm.cu)
+    ssi_buf_t bRowsum;        // per-slice partials of the bias gradients (ssi_gemm.cu)
 
     // MH state
     ssi_buf_t bMhZ, bMhZp, bMhLp, bMhLpP, bMhCnt, bMhG;

@@ -3,7 +3,7 @@
 // C(o, j) = epi( sum_k A(o, k) B(k, j) ) for a batch of independent problems: the contraction every step of the reverse
 // pass (src/space_inference.jl:107 through the AD backends of src/libs.jl:23-34) and of the mini-batch training step
 // (src/subspace_construction.jl:39-43) is made of -- forward W H, weight gradient delta H', back-propagated delta W' delta --
-// with FP32 operands in whatever orientation the Julia column-major layout gives them.  The SIMT kernel in ssi_grad.cu
+// with FP32 operands in whatever orientation the Julia column-major layout gives them.  The SIMT kernel in ssi_gemm.cu
 // (64x64 tiles, ~17 TFLOP/s) made a gradient on the wide MLP cost 100x a density evaluation.  This one keeps the
 // operands FP32 in global memory and does the split on the fly, the way the Gram kernel does:
 //
@@ -438,8 +438,8 @@ int ssi_gemm_tc_try(ssi_ctx* ctx, const gemm_t& g, int batches, bool a_kfast, bo
     p.split_acc = g.epi == 1 ? 1 : 0;
     p.epi = g.epi; p.act = g.act; p.bias = g.bias; p.bias_sb = g.bias_sb; p.Hprev = g.Hprev; p.h_sb = g.h_sb;
     typedef void (*gx_kernel_t)(const CUtensorMap, const CUtensorMap, const gemm_tc_params);
-    static const gx_kernel_t kernels[4] = {k_gemm_tc<false, false>, k_gemm_tc<false, true>, k_gemm_tc<true, false>, k_gemm_tc<true, true>};
-    const gx_kernel_t kern = kernels[(p.a_kfast ? 2 : 0) + (p.b_kfast ? 1 : 0)];
+    // the three orientations ssi_launch_gemm accepts: A k-fast with B k-fast, A o-fast with B either way
+    const gx_kernel_t kern = p.a_kfast ? k_gemm_tc<true, true> : p.b_kfast ? k_gemm_tc<false, true> : k_gemm_tc<false, false>;
     SSI_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, GX_SMEM));
     const int grid = (int)std::min<long long>(ctx->sm_count, p.n_work);
     kern<<<grid, GX_THREADS, GX_SMEM, ctx->stream>>>(mapA, mapB, p);

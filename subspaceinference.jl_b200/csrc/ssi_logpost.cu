@@ -9,13 +9,15 @@
 //            datapoints through the whole chain with activations in shared memory
 //            (small networks: README 10-20-20-2, UCI 13-50-1).
 //   LAYERED  weights of a group of samples are materialised, then one batched FP32 SIMT
-//            GEMM per layer with fused bias/activation, the last one fused with the
-//            squared-error reduction (any shape; correctness scaffold for wide nets).
+//            GEMM per layer (ssi_launch_gemm_simt) with fused bias/activation, the last one
+//            fused with the squared-error reduction (any shape; the exact FP32 cross-check
+//            of the tensor path).
 //   TENSOR   ssi_tc.cu (tcgen05 / TMEM / TMA).
 //
 // Reductions are two-stage and fixed-order (per-CTA partials -> finalize), so a
 // sample's lp does not depend on how many other samples share the call.
 #include "ssi_common.cuh"
+#include "ssi_gemm.cuh"
 
 #include <algorithm>
 #include <cmath>
@@ -318,92 +320,10 @@ int ssi_project_device(ssi_ctx* ctx, const float* dZ, int64_t B, float* dW, int6
     return SSI_OK;
 }
 
-#define LT 64
-#define LK 16
-// C[o,j] = act( sum_i A[o + i*out] * Hin[i + j*in] + bias[o] ), one 64x64 tile per CTA, 4x4 per thread.
-// FINAL: instead of storing, reduce (C - Y)^2 over the tile into partials.
-template <bool FINAL>
-__global__ void __launch_bounds__(256)
-k_dense_simt(const float* __restrict__ A, long long a_bs, const float* __restrict__ bias, long long bias_bs,
-             const float* __restrict__ Hin, long long hin_bs, float* __restrict__ Hout, long long hout_bs,
-             const float* __restrict__ Y, double* __restrict__ partials,
-             int out, int in, long long N, int act, int ld_out) {
-    __shared__ __align__(16) float As[LK][LT];
-    __shared__ __align__(16) float Bs[LK][LT + 4];
-    __shared__ double red[32];
-    const int tid = threadIdx.x;
-    const int tx = tid & 15, ty = tid >> 4;
-    const int o0 = blockIdx.y * LT;
-    const long long j0 = (long long)blockIdx.x * LT;
-    const int g = blockIdx.z;
-    A += (long long)g * a_bs;
-    bias += (long long)g * bias_bs;
-    Hin += (long long)g * hin_bs;
-
-    float acc[4][4];
-#pragma unroll
-    for (int r = 0; r < 4; ++r)
-#pragma unroll
-        for (int c = 0; c < 4; ++c) acc[r][c] = 0.0f;
-
-    for (int k0 = 0; k0 < in; k0 += LK) {
-#pragma unroll
-        for (int s = 0; s < 4; ++s) {
-            const int idx = tid + s * 256;
-            const int o = idx & (LT - 1), k = idx >> 6;
-            As[k][o] = (o0 + o < out && k0 + k < in) ? A[(o0 + o) + (long long)(k0 + k) * out] : 0.0f;
-        }
-#pragma unroll
-        for (int s = 0; s < 4; ++s) {
-            const int idx = tid + s * 256;
-            const int k = idx & (LK - 1), j = idx >> 4;
-            Bs[k][j] = (j0 + j < N && k0 + k < in) ? Hin[(k0 + k) + (j0 + j) * in] : 0.0f;
-        }
-        __syncthreads();
-#pragma unroll
-        for (int k = 0; k < LK; ++k) {
-            const float4 a4 = *reinterpret_cast<const float4*>(&As[k][tx * 4]);
-            const float4 b4 = *reinterpret_cast<const float4*>(&Bs[k][ty * 4]);
-            const float a[4] = {a4.x, a4.y, a4.z, a4.w};
-            const float b[4] = {b4.x, b4.y, b4.z, b4.w};
-#pragma unroll
-            for (int r = 0; r < 4; ++r)
-#pragma unroll
-                for (int c = 0; c < 4; ++c) acc[r][c] = fmaf(a[r], b[c], acc[r][c]);
-        }
-        __syncthreads();
-    }
-
-    double sse = 0.0;
-#pragma unroll
-    for (int c = 0; c < 4; ++c) {
-        const long long j = j0 + ty * 4 + c;
-#pragma unroll
-        for (int r = 0; r < 4; ++r) {
-            const int o = o0 + tx * 4 + r;
-            if (o < out && j < N) {
-                const float v = ssi_act(acc[r][c] + bias[o], act);
-                if (FINAL) {
-                    const float df = v - Y[o + j * out];
-                    sse += (double)df * (double)df;
-                } else {
-                    Hout[(long long)g * hout_bs + o + j * ld_out] = v;
-                }
-            }
-        }
-    }
-    if (FINAL) {
-        const double tot = ssi_block_sum(sse, red);
-        if (tid == 0) {
-            const long long tiles = (long long)gridDim.x * gridDim.y;
-            partials[(long long)g * tiles + (long long)blockIdx.y * gridDim.x + blockIdx.x] = tot;
-        }
-    }
-}
-
 static int run_layered(ssi_ctx* ctx, const float* dZ, int64_t B, double* d_sse) {
     const ssi_model_t& m = ctx->model;
     const int64_t N = ctx->N, n = m.n;
+    if (N >= (1ll << 31)) return ssi_fail(ctx, SSI_ERR_UNSUPPORTED, "LAYERED path: N must fit 31 bits");
     // group size: bounded by scratch (two activation buffers of max hidden width)
     int hid = 1;
     for (int l = 1; l < m.L; ++l) hid = std::max(hid, m.dims[l]);
@@ -416,8 +336,7 @@ static int run_layered(ssi_ctx* ctx, const float* dZ, int64_t B, double* d_sse) 
         if (m.L > 2) SSI_TRY(ssi_reserve(ctx, ctx->bH1, sizeof(float) * (size_t)hid * N * G));
     }
     const int O = m.dims[m.L];
-    const int tiles_j = (int)((N + LT - 1) / LT), tiles_o = (O + LT - 1) / LT;
-    const int parts = tiles_j * tiles_o;
+    const int parts = (int)((N + GT_T - 1) / GT_T) * ((O + GT_T - 1) / GT_T);      // one per tile of the last layer
     SSI_TRY(ssi_reserve(ctx, ctx->bPartials, sizeof(double) * (size_t)B * parts));
     float* dW = (float*)ctx->bW.p;
     float* hbuf[2] = {(float*)ctx->bH0.p, (float*)ctx->bH1.p};
@@ -429,22 +348,17 @@ static int run_layered(ssi_ctx* ctx, const float* dZ, int64_t B, double* d_sse) 
         const float* hin = ctx->dX;
         long long hin_bs = 0;
         for (int l = 0; l < m.L; ++l) {
-            const int in = m.dims[l], out = m.dims[l + 1];
-            const bool last = (l == m.L - 1);
-            dim3 grid(tiles_j, (out + LT - 1) / LT, g);
-            if (last) {
-                k_dense_simt<true><<<grid, 256, 0, ctx->stream>>>(dW + m.w_off[l], n, dW + m.b_off[l], n, hin, hin_bs,
-                                                                 nullptr, 0, ctx->dY, partials + b0 * parts,
-                                                                 out, in, N, m.act[l], out);
+            const int out = m.dims[l + 1];
+            if (l == m.L - 1) {         // the squared error against Y instead of the output
+                SSI_TRY(ssi_launch_gemm_simt(ctx, ssi_dense_gemm(m, l, dW, n, hin, hin_bs, nullptr, out, 0, (int)N), g, false, false,
+                                             ctx->dY, partials + b0 * parts));
             } else {
                 float* hout = hbuf[l & 1];
-                k_dense_simt<false><<<grid, 256, 0, ctx->stream>>>(dW + m.w_off[l], n, dW + m.b_off[l], n, hin, hin_bs,
-                                                                  hout, (long long)out * N, nullptr, nullptr,
-                                                                  out, in, N, m.act[l], out);
+                SSI_TRY(ssi_launch_gemm_simt(ctx, ssi_dense_gemm(m, l, dW, n, hin, hin_bs, hout, out, (long long)out * N, (int)N), g,
+                                             false, false));
                 hin = hout;
                 hin_bs = (long long)out * N;
             }
-            SSI_LAUNCH_CHECK(ctx);
         }
     }
     return ssi_reduce_partials(ctx, partials, B, parts, d_sse);
@@ -491,6 +405,7 @@ __global__ void k_pred_std(const double* __restrict__ m2, long long ON, long lon
 // dZ (M x B), dXg (in0 x Ng) device; d_preds (O x Ng x B) optional; d_mean, d_std (O x Ng doubles); d_m2 scratch (O x Ng)
 int ssi_predict_device(ssi_ctx* ctx, const float* dZ, int64_t B, const float* dXg, int64_t Ng,
                        float* d_preds, double* d_mean, double* d_std, double* d_m2) {
+    if (Ng >= (1ll << 31)) return ssi_fail(ctx, SSI_ERR_UNSUPPORTED, "predictive sweep: Ng must fit 31 bits");
     if (ctx->dec_active) SSI_TRY(ssi_dec_project(ctx, dZ, B, &dZ));       // W = W_swa + decoder(z): continue with z' = h(z)
     const ssi_model_t& m = ctx->model;
     const int64_t n = m.n;
@@ -510,20 +425,16 @@ int ssi_predict_device(ssi_ctx* ctx, const float* dZ, int64_t B, const float* dX
     float* dW = (float*)ctx->bW.p;
     float* hbuf[2] = {(float*)ctx->bH0.p, (float*)ctx->bH1.p};
     float* pg = (float*)ctx->bPartials.p;
-    const int tiles_j = (int)((Ng + LT - 1) / LT);
     for (int64_t b0 = 0; b0 < B; b0 += G) {
         const int g = (int)std::min<int64_t>(G, B - b0);
         SSI_TRY(ssi_project_device(ctx, dZ + b0 * ctx->M, g, dW));
         const float* hin = dXg;
         long long hin_bs = 0;
         for (int l = 0; l < m.L; ++l) {
-            const int in = m.dims[l], out = m.dims[l + 1];
-            const bool last = (l == m.L - 1);
-            float* hout = last ? pg : hbuf[l & 1];
-            dim3 grid(tiles_j, (out + LT - 1) / LT, g);
-            k_dense_simt<false><<<grid, 256, 0, ctx->stream>>>(dW + m.w_off[l], n, dW + m.b_off[l], n, hin, hin_bs, hout,
-                                                              (long long)out * Ng, nullptr, nullptr, out, in, Ng, m.act[l], out);
-            SSI_LAUNCH_CHECK(ctx);
+            const int out = m.dims[l + 1];
+            float* hout = l == m.L - 1 ? pg : hbuf[l & 1];
+            SSI_TRY(ssi_launch_gemm_simt(ctx, ssi_dense_gemm(m, l, dW, n, hin, hin_bs, hout, out, (long long)out * Ng, (int)Ng), g,
+                                         false, false));
             hin = hout;
             hin_bs = (long long)out * Ng;
         }
@@ -543,15 +454,11 @@ int ssi_predict_device(ssi_ctx* ctx, const float* dZ, int64_t B, const float* dX
 // First-layer bases for the tensor path: B_m = (column m of [P | W_swa])_layer0 applied to X, m = 0..M,
 // as FP32 pre-activations [m][N][ld] (bias parts included).  Exact FP32 SIMT GEMM, run once per (data, subspace).
 int ssi_build_first_layer_bases(ssi_ctx* ctx, float* bases, int ld) {
-    const ssi_model_t& m = ctx->model;
-    const int in = m.dims[0], out = m.dims[1];
     const int64_t N = ctx->N;
-    dim3 grid((unsigned)((N + LT - 1) / LT), (out + LT - 1) / LT, ctx->M + 1);
-    k_dense_simt<false><<<grid, 256, 0, ctx->stream>>>(ctx->dP + m.w_off[0], m.n, ctx->dP + m.b_off[0], m.n, ctx->dX, 0,
-                                                      bases, (long long)N * ld, nullptr, nullptr, out, in, N,
-                                                      SSI_ACT_IDENTITY, ld);
-    SSI_LAUNCH_CHECK(ctx);
-    return SSI_OK;
+    if (N >= (1ll << 31)) return ssi_fail(ctx, SSI_ERR_UNSUPPORTED, "tensor path bases: N must fit 31 bits");
+    gemm_t q = ssi_dense_gemm(ctx->model, 0, ctx->dP, ctx->model.n, ctx->dX, 0, bases, ld, N * ld, (int)N);
+    q.act = SSI_ACT_IDENTITY;
+    return ssi_launch_gemm_simt(ctx, q, ctx->M + 1, false, false);
 }
 
 // SSE (+ the M-space prior terms) -> log-probabilities: the closed form of logpdf(MvNormal(vec(pred), sigma_m), vec(Y))

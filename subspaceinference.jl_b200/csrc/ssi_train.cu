@@ -13,9 +13,9 @@
 //     Descent: W -= eta g          ADAM (Flux 0.11): m = b1 m + (1-b1) g;  v = b2 v + (1-b2) g^2;
 //                                                    W -= eta m/(1-b1^t) / (sqrt(v/(1-b2^t)) + 1e-8)
 //
-// Contractions are the strided FP32 SIMT GEMM of the gradient path (ssi_gemm.cuh); the optimiser update is one
-// element-wise pass evaluated in FP64 like Julia's broadcast with Float64 hyper-parameters.  Correctness-first: this is a
-// "next" row, measured but not tuned.
+// The forward and backward passes are the gradient path's ssi_reverse_pass (ssi_gemm.cu) with one sample; the optimiser
+// update is one element-wise pass evaluated in FP64 like Julia's broadcast with Float64 hyper-parameters.
+// Correctness-first: this is a "next" row, measured but not tuned.
 #include "ssi_common.cuh"
 #include "ssi_gemm.cuh"
 
@@ -137,56 +137,19 @@ int ssi_train_step_impl(ssi_ctx* ctx, const int64_t* idx, int64_t j0, int64_t nb
         Yb = (const float*)t->bYb.p;
     }
 
-    long long act_elems = 0;
     int maxw = 0;
-    long long h_off[SSI_MAX_LAYERS + 1];
-    h_off[0] = 0;
-    for (int l = 1; l <= L; ++l) { h_off[l] = act_elems; act_elems += (long long)m.dims[l] * nb; maxw = std::max(maxw, m.dims[l]); }
+    const long long act_elems = ssi_act_offsets(m, nb, nullptr, &maxw);
     const int n_chunks = (int)((nb + 255) / 256);
     SSI_TRY(ssi_reserve(ctx, t->bAct, sizeof(float) * (size_t)act_elems));
     SSI_TRY(ssi_reserve(ctx, t->bDelta, sizeof(float) * (size_t)2 * maxw * nb));
     SSI_TRY(ssi_reserve(ctx, t->bPart, sizeof(double) * (size_t)n_chunks));
-    float* H = (float*)t->bAct.p;
     float* D[2] = {(float*)t->bDelta.p, (float*)t->bDelta.p + (size_t)maxw * nb};
-    const float* W = t->W;
-    float* gW = t->G;
-
-    for (int l = 0; l < L; ++l) {
-        const int in = m.dims[l], out = m.dims[l + 1];
-        gemm_t q{};
-        q.A = W + m.w_off[l]; q.a_so = 1; q.a_sk = out;
-        q.B = l == 0 ? Xb : H + h_off[l]; q.b_sk = 1; q.b_sj = in;
-        q.C = H + h_off[l + 1]; q.c_so = 1; q.c_sj = out;
-        q.O = out; q.J = (int)nb; q.K = in;
-        q.epi = 1; q.act = m.act[l]; q.bias = W + m.b_off[l];
-        SSI_TRY(ssi_launch_gemm(ctx, q, 1, false, false));
-    }
-    // delta_L = 2/(O nb) (pred - y) act'(pred): k_grad_delta_out computes -(pred - y) * coef * act'
+    // delta_L = 2/(O nb) (pred - y) act'(pred): the reverse pass computes -(pred - y) * coef * act'
     const double count = (double)O * (double)nb;
-    SSI_TRY(ssi_launch_delta_out(ctx, H + h_off[L], 0, Yb, D[L & 1], 0, nb, O, m.act[L - 1], (float)(-2.0 / count), n_chunks, 1,
-                                 (double*)t->bPart.p));
+    SSI_TRY(ssi_reverse_pass(ctx, 1, nb, t->W, t->G, m.n, Xb, Yb, (float*)t->bAct.p, act_elems, D, (long long)maxw * nb,
+                             (float)(-2.0 / count), (double*)t->bPart.p));
     k_train_loss<<<1, 32, 0, ctx->stream>>>((const double*)t->bPart.p, n_chunks, 1.0 / count, t->loss);
     SSI_LAUNCH_CHECK(ctx);
-    for (int l = L - 1; l >= 0; --l) {
-        const int in = m.dims[l], out = m.dims[l + 1];
-        const float* delta = D[(l + 1) & 1];
-        gemm_t q{};
-        q.A = delta; q.a_so = 1; q.a_sk = out;
-        q.B = l == 0 ? Xb : H + h_off[l]; q.b_sk = in; q.b_sj = 1;
-        q.C = gW + m.w_off[l]; q.c_so = 1; q.c_sj = out;
-        q.O = out; q.J = in; q.K = nb; q.epi = 0;
-        SSI_TRY(ssi_launch_gemm(ctx, q, 1, false, true));
-        SSI_TRY(ssi_launch_rowsum(ctx, delta, 0, out, nb, 1, gW + m.b_off[l], 0));
-        if (l > 0) {
-            gemm_t r{};
-            r.A = W + m.w_off[l]; r.a_so = out; r.a_sk = 1;
-            r.B = delta; r.b_sk = 1; r.b_sj = out;
-            r.C = D[l & 1]; r.c_so = 1; r.c_sj = in;
-            r.O = in; r.J = (int)nb; r.K = out;
-            r.epi = 2; r.act = m.act[l - 1]; r.Hprev = H + h_off[l];
-            SSI_TRY(ssi_launch_gemm(ctx, r, 1, true, false));
-        }
-    }
     k_train_update<<<(unsigned)((m.n + 255) / 256), 256, 0, ctx->stream>>>(t->W, t->G, t->m, t->v, m.n, t->kind, t->eta, t->b1, t->b2,
                                                                        t->bp1, t->bp2);
     SSI_LAUNCH_CHECK(ctx);

@@ -1,4 +1,4 @@
-"""Every kernel family ssi_launch_gemm (ssi_grad.cu) picks for the gradient and training paths, at the shapes where it
+"""Every kernel family ssi_launch_gemm (ssi_gemm.cu) picks for the gradient and training paths, at the shapes where it
 picks it, against the Float64 oracle: narrow heads and bottleneck layers on the skinny kernels, the tensor-core GEMM right
 after a bottleneck, and the thresholds between the families.
 
